@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Throughput benchmark of the MAPF reset()/step() hot path (BASELINE.json metric: agent-steps/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -12,6 +12,10 @@ reset()`, scripts/benchmark_multi_agent_env.py:89-95), actions uniform over the 
 A "step" is one pass of the hot path over the whole batch: ONE launch of the step kernel, which
 also draws the next step's masked-uniform actions (the benchmark sampler fused in).  Envs shard independently across GPUs (weak scaling, no data-path collective); the one
 NCCL all-reduce (episode/lock metric sums) runs once after the timed region.
+
+The timed region is exactly `--steps` launches after `--warmup` untimed ones.  `--dump-outputs DIR` then writes what
+the last timed step returned (rank 0's shard, a fixed sample of its envs) as float32 / float64 .npy files; the inputs
+depend on the arguments only, so two builds run with the same arguments can be compared output for output.
 
 Prints ONE JSON line (rank 0).  `value` = agent-steps/s with inputs resident in HBM; `e2e` = the
 same metric through the C ABI's host-buffer entry point (mapf_step_host: pinned host actions in,
@@ -34,6 +38,7 @@ import numpy as np
 
 REPO = Path(__file__).resolve().parent
 sys.path.insert(0, str(REPO))
+sys.dont_write_bytecode = True   # the tree may be read-only: no __pycache__ is written next to the sources
 
 METRIC = "agent_steps_per_sec"
 UNIT = "agent-steps/s"
@@ -314,6 +319,7 @@ class SteadyBatch:
         e = self.envs[self.i % len(self.envs)]
         self.i += 1
         e.step(e._next, auto_reset=True)
+        self.last = e
 
     def launches(self) -> int:
         return sum(e.launch_count for e in self.envs)
@@ -331,6 +337,43 @@ class SteadyBatch:
     def close(self):
         for e in self.envs:
             e.close()
+
+
+DUMP_BYTES = 48 << 20   # .npy payload --dump-outputs writes at most
+
+
+def dump_outputs(env, out_dir: str) -> None:
+    """What the env's last step handed its caller -- every output channel, the actions the fused sampler drew for the
+    next step, the agents' positions and goals -- as DIR/<name>.npy (info as float64, the rest float32), for a seeded
+    sample of the envs that fits DUMP_BYTES (all of them when they fit); env_ids.npy lists the sampled envs."""
+    import torch
+
+    from dl_reference_models_b200 import _native as nat
+
+    chans = {k: env.out[k] for k in nat.OUTPUT_FIELDS}
+    chans.update(next_actions=env._actions, positions=env.state["positions"], goals=env.state["goals"])
+    wide = {"info"}   # int32 counters: float64 keeps them exact
+    per_env = sum(t[0].numel() * (8 if k in wide else 4) for k, t in chans.items())
+    n = min(env.B, DUMP_BYTES // per_env)
+    ids = np.sort(np.random.default_rng(0).choice(env.B, n, replace=False))
+    idx = torch.from_numpy(ids).to(env.device)
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "env_ids.npy", ids.astype(np.float64))
+    for k, t in chans.items():
+        np.save(d / f"{k}.npy", t.index_select(0, idx).cpu().numpy().astype(np.float64 if k in wide else np.float32))
+
+
+def timed_steps(step, K: int, barrier, torch) -> float:
+    """Time exactly K steps (CUDA events on the launching stream, no host sync in between); returns the region's ms."""
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    barrier()
+    e0.record()
+    for _ in range(K):
+        step()
+    e1.record()
+    barrier()
+    return e0.elapsed_time(e1)
 
 
 def timed_blocks(step, K: int, min_seconds: float, barrier, torch, max_blocks: int = 20000):
@@ -460,18 +503,18 @@ def run_b200(args, rank: int, local_rank: int, world: int):
         sampler.wait_first_sample()
     launches0 = sb.launches()
     sampler.mark_begin()
-    blocks, region_ms, _ = timed_blocks(sb.step, K, args.min_seconds, barrier, torch)
+    region_ms = timed_steps(sb.step, K, barrier, torch)
     sampler.mark_end()
     clocks = sampler.stop() if rank == 0 else None
     launches = sb.launches() - launches0
-    nblocks = len(blocks)
-    # one step = ONE launch of the step kernel (checked below): a block's CUDA-event time / K is the kernel's average
+    # one step = ONE launch of the step kernel (checked below): the region's CUDA-event time / K is the kernel's average
     # launch duration, launch gaps included
-    assert launches == K * (nblocks + 1), (launches, K, nblocks)   # + the calibration block
+    assert launches == K, (launches, K)
     sb.check()
-    block_ms = float(np.median(blocks))
-    block_ms_max = reduce_max(block_ms)                      # slowest rank
-    kernel_ms = block_ms_max / K
+    if args.dump_outputs and rank == 0:
+        dump_outputs(sb.last, args.dump_outputs)
+    region_ms_max = reduce_max(region_ms)                    # slowest rank
+    kernel_ms = region_ms_max / K
     metrics, allreduce_check = reduced_metrics(sb)
 
     # ------------------------------------------------------------------ the same batches through mapf_step_many: K steps per launch
@@ -575,7 +618,7 @@ def run_b200(args, rank: int, local_rank: int, world: int):
         bytes_per_as = algorithmic_bytes_per_agent_step(N, V, True, 0)
         alg_bytes = bytes_per_as * B * N
         achieved = alg_bytes / (kernel_ms * 1e-3) / 1e9
-        value = world * B * N * K / (block_ms_max * 1e-3)
+        value = world * B * N * K / (region_ms_max * 1e-3)
         traffic, traffic_src = (args.traffic_bytes, "--traffic-bytes") if args.traffic_bytes is not None else \
             committed_traffic(args.shape, sb.kind)
         e2e_value = world * B * N * Ke / (e2e_ms * 1e-3)
@@ -588,13 +631,13 @@ def run_b200(args, rank: int, local_rank: int, world: int):
 
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-            "ms_per_step": block_ms_max / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "ms_per_step": region_ms_max / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "int16/u8", "data": "synthetic", "impl": "b200", "config": config_dict(args, world),
-            "timing": {"blocks": nblocks, "steps_per_block": K, "block_ms_median": block_ms_max,
-                       "block_ms_min_rank0": float(np.min(blocks)), "block_ms_max_rank0": float(np.max(blocks)),
-                       "region_ms_rank0": region_ms, "burn_in_steps_per_replica": sb.burn_steps,
-                       "note": "median block of exactly `steps` launches (slowest rank); steady state: episode phases "
-                               "staggered, 1/steps_per_episode of the envs reset inside every launch"},
+            "timing": {"timed_steps": K, "region_ms": region_ms_max, "region_ms_rank0": region_ms,
+                       "burn_in_steps_per_replica": sb.burn_steps,
+                       "note": "one region of exactly `steps` launches after `warmup` untimed ones (slowest rank); "
+                               "steady state: episode phases staggered, 1/steps_per_episode of the envs reset inside "
+                               "every launch"},
             "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                          "traffic": traffic, "traffic_source": traffic_src,
                          "kernel": kernel_name(sb.kind, N, args.sensor_range), "kernel_ms": kernel_ms,
@@ -889,7 +932,7 @@ def _python_reference_worker(root, cfg, grid, seconds, seed, q):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed step launches")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", choices=("b200", "reference"), default="b200")
     ap.add_argument("--shape", choices=tuple(SHAPES), default="c3",
@@ -902,10 +945,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-shapes", action="store_true", help="skip the C4 / C5 legs of the JSON line")
     ap.add_argument("--min-seconds", type=float, default=0.5,
-                    help="the timed region repeats blocks of --steps launches until it lasts this long (median block reported)")
+                    help="the step_many leg repeats blocks of launches until it lasts this long, at most 0.2 s "
+                         "(median block reported)")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per step-kernel launch from the committed ncu --set full capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (a seeded sample of rank 0's envs) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     apply_shape(args)
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
