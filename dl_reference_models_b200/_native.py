@@ -17,6 +17,7 @@ REPO = PKG.parent
 CSRC = PKG / "csrc"
 LIB_PATH = Path(os.environ.get("MAPF_B200_LIB", PKG / "libmapf_b200.so"))
 SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_kernel.cuh", CSRC / "mapf_pair_kernel.cuh", CSRC / "mapf_cte_kernel.cuh", CSRC / "mapf_policy_kernel.cuh",
+           CSRC / "mapf_policy_lstm_kernel.cuh",
            CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
@@ -103,6 +104,18 @@ class MapfPolicyArgs(C.Structure):
     ] + [(k, C.c_void_p) for k in (
         "local_obs", "goal_delta", "blocking_prev", "action_mask", "weights", "actions", "actions64", "logp", "value",
         "logits_out", "features_out", "action_mask_out")]
+
+
+class MapfLstmPolicyArgs(C.Structure):
+    """mapf_lstm_policy_args of include/mapf_b200.h (fused LSTM-64 policy + sampler)."""
+
+    _fields_ = [
+        ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("v2", C.c_int32), ("feature_dim", C.c_int32),
+        ("no_masking", C.c_int32), ("reserved", C.c_int32),
+        ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
+    ] + [(k, C.c_void_p) for k in (
+        "local_obs", "goal_delta", "blocking_prev", "action_mask", "prev_terminated", "prev_truncated", "prev_action",
+        "prev_reward", "h_in", "c_in", "h_out", "c_out", "weights", "actions", "actions64", "logp", "value", "logits_out")]
 
 
 class MapfError(RuntimeError):
@@ -200,11 +213,16 @@ def lib():
     L.mapf_policy_weights_nbytes.restype = i64
     L.mapf_policy_pack_weights.argtypes = [i32] + [vp] * 9
     L.mapf_policy_act.argtypes = [C.POINTER(MapfPolicyArgs), vp]
+    L.mapf_lstm_policy_weights_nbytes.argtypes = [i32]
+    L.mapf_lstm_policy_weights_nbytes.restype = i64
+    L.mapf_lstm_policy_pack_weights.argtypes = [i32] + [vp] * 13
+    L.mapf_lstm_policy_act.argtypes = [C.POINTER(MapfLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
-        if name not in ("mapf_version", "mapf_last_error", "mapf_launch_count", "mapf_policy_weights_nbytes"):
+        if name not in ("mapf_version", "mapf_last_error", "mapf_launch_count", "mapf_policy_weights_nbytes",
+                        "mapf_lstm_policy_weights_nbytes"):
             getattr(L, name).restype = C.c_int
     _lib = L
     return L
@@ -220,6 +238,7 @@ EXPORTS = (
     "mapf_sample_random_actions", "mapf_set_fused_sampler", "mapf_metrics_reduce", "mapf_poll_errors", "mapf_launch_count",
     "mapf_step_kernel_kind", "mapf_cte_step", "mapf_cte_reset", "mapf_occupancy_accumulate", "mapf_distance_table", "mapf_goal_path_lengths",
     "mapf_policy_weights_nbytes", "mapf_policy_pack_weights", "mapf_policy_act", "mapf_gae",
+    "mapf_lstm_policy_weights_nbytes", "mapf_lstm_policy_pack_weights", "mapf_lstm_policy_act",
 )
 
 

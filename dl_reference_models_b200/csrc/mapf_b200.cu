@@ -6,6 +6,7 @@
 #include "mapf_pair_kernel.cuh"
 #include "mapf_cte_kernel.cuh"
 #include "mapf_policy_kernel.cuh"
+#include "mapf_policy_lstm_kernel.cuh"
 #include "mapf_pack_kernel.cuh"
 #include "mapf_host_unpack.h"
 
@@ -1658,6 +1659,79 @@ int mapf_policy_act(const mapf_policy_args *a, void *stream) {
         CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_policy_act_kernel<4>),
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         mapf::mapf_policy_act_kernel<4><<<(unsigned)blocks, threads, smem, st>>>(*a);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int64_t mapf_lstm_policy_weights_nbytes(int32_t F) {
+    const int kc1 = policy_kc1(F);
+    if (!kc1) return fail(MAPF_ERR_UNSUPPORTED, "lstm policy: feature_dim %d outside 1..64", F);
+    return mapf::lstm_weight_bytes(kc1);
+}
+
+int mapf_lstm_policy_pack_weights(int32_t F, const float *w1, const float *b1, const float *w2, const float *b2,
+                                  const float *w_ih, const float *w_hh, const float *b_ih, const float *b_hh,
+                                  const float *wl, const float *bl, const float *wv, const float *bv, void *packed) {
+    const int kc1 = policy_kc1(F);
+    if (!kc1) return fail(MAPF_ERR_UNSUPPORTED, "lstm policy: feature_dim %d outside 1..64", F);
+    if (!w1 || !b1 || !w2 || !b2 || !w_ih || !w_hh || !b_ih || !b_hh || !wl || !bl || !wv || !bv || !packed)
+        return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    const int s1 = 16 * kc1 + 8, H = mapf::POL_H, S2 = mapf::POL_W2_STRIDE, SG = mapf::LSTM_SG, KI = H + 5 + 1;
+    memset(packed, 0, (size_t)mapf::lstm_weight_bytes(kc1));
+    __nv_bfloat16 *p1 = static_cast<__nv_bfloat16 *>(packed), *p2 = p1 + H * s1, *p3 = p2 + H * S2, *pg = p3 + 8 * S2;
+    float *pb = reinterpret_cast<float *>(pg + 4 * H * SG);
+    for (int o = 0; o < H; ++o) {
+        for (int i = 0; i < F; ++i) p1[o * s1 + i] = __float2bfloat16_rn(w1[o * F + i]);
+        for (int i = 0; i < H; ++i) p2[o * S2 + i] = __float2bfloat16_rn(w2[o * H + i]);
+        pb[o] = b1[o];
+        pb[H + o] = b2[o];
+    }
+    for (int o = 0; o < 5; ++o) {
+        for (int i = 0; i < H; ++i) p3[o * S2 + i] = __float2bfloat16_rn(wl[o * H + i]);
+        pb[2 * H + o] = bl[o];
+    }
+    for (int i = 0; i < H; ++i) p3[5 * S2 + i] = __float2bfloat16_rn(wv[i]);
+    pb[2 * H + 5] = bv[0];
+    for (int o = 0; o < 4 * H; ++o) {   // [W_ih (70 cols) | 10 zero cols | W_hh (64 cols)]
+        for (int i = 0; i < KI; ++i) pg[o * SG + i] = __float2bfloat16_rn(w_ih[o * KI + i]);
+        for (int i = 0; i < H; ++i) pg[o * SG + mapf::LSTM_KX + i] = __float2bfloat16_rn(w_hh[o * H + i]);
+        pb[2 * H + 8 + o] = b_ih[o] + b_hh[o];
+    }
+    return MAPF_OK;
+}
+
+int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    const int kc1 = policy_kc1(a->feature_dim);
+    if (!kc1 || a->v2 < 1 || a->feature_dim != a->v2 + 2 + (a->blocking_prev ? 1 : 0))
+        return fail(MAPF_ERR_UNSUPPORTED, "lstm policy: feature_dim %d does not match v2 %d (+2 goal delta, +1 pressure) or exceeds 64",
+                    a->feature_dim, a->v2);
+    if (a->num_envs < 1 || a->num_agents < 1 || !a->local_obs || !a->goal_delta || !a->weights)
+        return fail(MAPF_ERR_INVALID_ARG, "lstm policy: env outputs and weights are required");
+    if (!a->prev_action || !a->prev_reward || !a->h_in || !a->c_in)
+        return fail(MAPF_ERR_INVALID_ARG, "lstm policy: prev_action, prev_reward, h_in and c_in are required");
+    if (!a->h_out != !a->c_out)
+        return fail(MAPF_ERR_INVALID_ARG, "lstm policy: h_out and c_out are given together (both NULL = state not advanced)");
+    int ndev = 0, dev = 0, sms = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int threads = mapf::LSTM_THREADS, warps = threads / 32;
+    const size_t smem = (size_t)mapf::lstm_weight_bytes(kc1) + (size_t)warps * mapf::pol_warp_bytes(kc1, a->v2);
+    const long long tiles = ((long long)a->num_envs * a->num_agents + 31) / 32;
+    long long blocks = (tiles + warps - 1) / warps;
+    if (blocks > sms) blocks = sms;   // one resident block per SM loads the weights once and loops over the tiles
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (kc1 == 2) {
+        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_lstm_policy_act_kernel<2>),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        mapf::mapf_lstm_policy_act_kernel<2><<<(unsigned)blocks, threads, smem, st>>>(*a);
+    } else {
+        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_lstm_policy_act_kernel<4>),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        mapf::mapf_lstm_policy_act_kernel<4><<<(unsigned)blocks, threads, smem, st>>>(*a);
     }
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;

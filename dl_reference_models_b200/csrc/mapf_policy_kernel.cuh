@@ -44,6 +44,151 @@ __host__ __device__ constexpr int pol_warp_bytes(int kc1, int v2) {
     return 32 * (16 * kc1 + 8) * 2 /* bf16 feature tile */ + pol_raw_bytes(v2) + 160 /* masks */ + 32 * 8 * 4 /* head outputs */;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Pieces shared by mapf_policy_act_kernel and mapf_lstm_policy_act_kernel (mapf_policy_lstm_kernel.cuh).  All of them
+// work on one warp's tile of 32 agents; `g` / `t` are the lane's mma.sync group / thread-in-group indices.
+
+// raw channels of the tile, coalesced: window bytes -> raw, mask bytes -> rawm (+ an optional copy of the masks)
+__device__ __forceinline__ void pol_load_tile(const uint8_t *local_obs, const int8_t *action_mask, int8_t *action_mask_out,
+                                              int V2, long long ag0, int na, uint32_t *raw, uint32_t *rawm, int lane) {
+    const uint32_t *ob32 = reinterpret_cast<const uint32_t *>(local_obs + ag0 * V2);   // 32 * V2 bytes: 4-byte aligned
+    const int nwords = (na * V2 + 3) >> 2;
+    for (int i = lane; i < (32 * V2 + 3) / 4 + 2; i += 32) raw[i] = i < nwords ? ob32[i] : 0u;
+    if (action_mask) {
+        const uint32_t *mk32 = reinterpret_cast<const uint32_t *>(action_mask + ag0 * 5);
+        const int mwords = (na * 5 + 3) >> 2;
+        for (int i = lane; i < 40; i += 32) rawm[i] = i < mwords ? mk32[i] : 0u;
+        if (action_mask_out) {   // the rollout buffer's copy of the masks (saves a separate copy launch per step)
+            uint32_t *mo32 = reinterpret_cast<uint32_t *>(action_mask_out + ag0 * 5);
+            // word copies when the destination row is 4-byte aligned (a [T,B,N,5] row may start anywhere)
+            const int full_words = (reinterpret_cast<uintptr_t>(action_mask_out) & 3) == 0 ? (na * 5) >> 2 : 0;
+            for (int i = lane; i < full_words; i += 32) mo32[i] = mk32[i];
+            for (int i = full_words * 4 + lane; i < na * 5; i += 32) action_mask_out[ag0 * 5 + i] = action_mask[ag0 * 5 + i];
+        }
+    }
+}
+
+// bf16 feature row of agent `lane` (ENV:306-328 order: window, goal delta, pressure) into xs[lane][0 .. 16 KC1)
+template <int KC1>
+__device__ __forceinline__ void pol_feature_row(__nv_bfloat16 *xs, const uint32_t *raw, const float *goal_delta,
+                                                const uint8_t *blocking_prev, int V2, long long ag0, int na, int lane) {
+    constexpr int S1 = 16 * KC1 + 8;
+    const int NW = (V2 + 3) >> 2;   // words of one agent's window
+    uint2 *row = reinterpret_cast<uint2 *>(xs + lane * S1);
+    const int off = lane * V2;
+    for (int j = 0; j < 4 * KC1; ++j) {   // 4 cells -> 4 bf16 per trip; columns beyond the window are zero
+        uint32_t w = 0;
+        if (j < NW) {
+            const int b = off + 4 * j;
+            w = __funnelshift_r(raw[b >> 2], raw[(b >> 2) + 1], (b & 3) * 8);
+            if (4 * j + 4 > V2) w &= (1u << (8 * (V2 - 4 * j))) - 1u;
+        }
+        const __nv_bfloat162 lo = __floats2bfloat162_rn((float)(w & 0xFFu), (float)((w >> 8) & 0xFFu));
+        const __nv_bfloat162 hi = __floats2bfloat162_rn((float)((w >> 16) & 0xFFu), (float)(w >> 24));
+        row[j] = make_uint2(*reinterpret_cast<const uint32_t *>(&lo), *reinterpret_cast<const uint32_t *>(&hi));
+    }
+    if (lane < na) {
+        const float2 gd = reinterpret_cast<const float2 *>(goal_delta)[ag0 + lane];
+        xs[lane * S1 + V2] = __float2bfloat16(gd.x);
+        xs[lane * S1 + V2 + 1] = __float2bfloat16(gd.y);
+        if (blocking_prev) xs[lane * S1 + V2 + 2] = __float2bfloat16((float)blocking_prev[ag0 + lane]);
+    }
+}
+
+// the two ReLU layers of the 16-row m-tile whose rows are row0 and row0 + 8: features xs -> A fragments of the next
+// GEMM (bias = b1[64] b2[64])
+template <int KC1>
+__device__ __forceinline__ void pol_trunk(const __nv_bfloat16 *xs, const __nv_bfloat16 *w1, const __nv_bfloat16 *w2,
+                                          const float *bias, int row0, int g, int t, uint32_t (&h2)[POL_H / 16][4]) {
+    constexpr int S1 = 16 * KC1 + 8;
+    // ------------------------------------------------------------ layer 1
+    uint32_t af[KC1][4];
+#pragma unroll
+    for (int kk = 0; kk < KC1; ++kk) {
+        const uint32_t *p0 = reinterpret_cast<const uint32_t *>(xs + row0 * S1 + 16 * kk + 2 * t);
+        const uint32_t *p1 = reinterpret_cast<const uint32_t *>(xs + (row0 + 8) * S1 + 16 * kk + 2 * t);
+        af[kk][0] = p0[0]; af[kk][1] = p1[0]; af[kk][2] = p0[4]; af[kk][3] = p1[4];
+    }
+    uint32_t h1[POL_H / 16][4];   // A fragments of layer 2
+#pragma unroll
+    for (int j = 0; j < POL_H / 8; ++j) {
+        const float2 bb = *reinterpret_cast<const float2 *>(bias + 8 * j + 2 * t);
+        float d[4] = {bb.x, bb.y, bb.x, bb.y};
+#pragma unroll
+        for (int kk = 0; kk < KC1; ++kk) {
+            const uint32_t *wb = reinterpret_cast<const uint32_t *>(w1 + (8 * j + g) * S1 + 16 * kk + 2 * t);
+            mma_bf16_16816(d, af[kk], wb[0], wb[4]);
+        }
+        h1[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);   // row g,   cols 8j + 2t, +1
+        h1[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);   // row g+8
+    }
+    // ------------------------------------------------------------ layer 2
+#pragma unroll
+    for (int j = 0; j < POL_H / 8; ++j) {
+        const float2 bb = *reinterpret_cast<const float2 *>(bias + POL_H + 8 * j + 2 * t);
+        float d[4] = {bb.x, bb.y, bb.x, bb.y};
+#pragma unroll
+        for (int kk = 0; kk < POL_H / 16; ++kk) {
+            const uint32_t *wb = reinterpret_cast<const uint32_t *>(w2 + (8 * j + g) * POL_W2_STRIDE + 16 * kk + 2 * t);
+            mma_bf16_16816(d, h1[kk], wb[0], wb[4]);
+        }
+        h2[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);
+        h2[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);
+    }
+}
+
+// heads: columns 0..4 logits, 5 value (w3 [8][72], b3[8]) of the m-tile -> os[32][8]
+__device__ __forceinline__ void pol_heads(const uint32_t (&hf)[POL_H / 16][4], const __nv_bfloat16 *w3, const float *b3,
+                                          float *os, int row0, int g, int t) {
+    const float2 bb = *reinterpret_cast<const float2 *>(b3 + 2 * t);
+    float d[4] = {bb.x, bb.y, bb.x, bb.y};
+#pragma unroll
+    for (int kk = 0; kk < POL_H / 16; ++kk) {
+        const uint32_t *wb = reinterpret_cast<const uint32_t *>(w3 + g * POL_W2_STRIDE + 16 * kk + 2 * t);
+        mma_bf16_16816(d, hf[kk], wb[0], wb[4]);
+    }
+    *reinterpret_cast<float2 *>(os + row0 * 8 + 2 * t) = make_float2(d[0], d[1]);
+    *reinterpret_cast<float2 *>(os + (row0 + 8) * 8 + 2 * t) = make_float2(d[2], d[3]);
+}
+
+// one agent per lane (call for lane < na): mask, stable softmax, inverse-CDF draw from one Philox word keyed by
+// (seed ^ tag, env_id_base + env), counter (counter, agent); writes the outputs of `a` that are not NULL
+template <class Args>
+__device__ __forceinline__ void pol_sample(const Args &a, const float *os, const uint32_t *rawm, int lane, long long ag, int N,
+                                           unsigned long long tag) {
+    const float4 o03 = *reinterpret_cast<const float4 *>(os + lane * 8);
+    const float2 o45 = *reinterpret_cast<const float2 *>(os + lane * 8 + 4);
+    float l[5] = {o03.x, o03.y, o03.z, o03.w, o45.x};
+    if (!a.no_masking && a.action_mask) {   // logits + clamp(log(mask + 1e-6), FLOAT_MIN), action_mask_model.py:57-61
+        const uint8_t *mk = reinterpret_cast<const uint8_t *>(rawm) + lane * 5;
+#pragma unroll
+        for (int k = 0; k < 5; ++k) l[k] += mk[k] ? 9.99999e-07f : -13.815511f;
+    }
+    float mx = l[0];
+#pragma unroll
+    for (int k = 1; k < 5; ++k) mx = fmaxf(mx, l[k]);
+    float pr[5], sum = 0.f;
+#pragma unroll
+    for (int k = 0; k < 5; ++k) { pr[k] = __expf(l[k] - mx); sum += pr[k]; }
+    const unsigned env = (unsigned)((unsigned long long)ag / (unsigned)N);   // B * N < 2^32 in any batch that fits a GPU
+    const int agent = (int)(ag - (long long)env * N);
+    Philox ph(a.seed ^ tag, a.env_id_base + env);
+    const uint4 x = ph((uint32_t)a.counter, (uint32_t)(a.counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
+    const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
+    int act = 0;
+    float cum = pr[0];
+#pragma unroll
+    for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
+    if (a.actions) a.actions[ag] = (int8_t)act;
+    if (a.actions64) a.actions64[ag] = (long long)act;
+    if (a.logp) a.logp[ag] = l[act] - mx - __logf(sum);
+    if (a.value) a.value[ag] = o45.y;
+    if (a.logits_out) {
+#pragma unroll
+        for (int k = 0; k < 5; ++k) a.logits_out[ag * 5 + k] = l[k];
+    }
+}
+
 // KC1 = k16 chunks of the first layer (F <= 16 * KC1), W1 row stride = 16 * KC1 + 8
 template <int KC1>
 __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_args a) {
@@ -71,150 +216,35 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
     const int g = lane >> 2, t = lane & 3;
     const long long BN = (long long)a.num_envs * N;
     const long long ntiles = (BN + 31) >> 5;
-    const int NW = (V2 + 3) >> 2;   // words of one agent's window
     for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
         const long long ag0 = tile << 5;
         const long long left = BN - ag0;
         const int na = left < 32 ? (int)left : 32;
-        // ---------------------------------------------------------------- raw channels of the tile, coalesced
-        {
-            const uint32_t *ob32 = reinterpret_cast<const uint32_t *>(a.local_obs + ag0 * V2);   // 32 * V2 bytes: 4-byte aligned
-            const int nwords = (na * V2 + 3) >> 2;
-            for (int i = lane; i < (32 * V2 + 3) / 4 + 2; i += 32) raw[i] = i < nwords ? ob32[i] : 0u;
-            if (a.action_mask) {
-                const uint32_t *mk32 = reinterpret_cast<const uint32_t *>(a.action_mask + ag0 * 5);
-                const int mwords = (na * 5 + 3) >> 2;
-                for (int i = lane; i < 40; i += 32) rawm[i] = i < mwords ? mk32[i] : 0u;
-                if (a.action_mask_out) {   // the rollout buffer's copy of the masks (saves a separate copy launch per step)
-                    uint32_t *mo32 = reinterpret_cast<uint32_t *>(a.action_mask_out + ag0 * 5);
-                    // word copies when the destination row is 4-byte aligned (a [T,B,N,5] row may start anywhere)
-                    const int full_words = (reinterpret_cast<uintptr_t>(a.action_mask_out) & 3) == 0 ? (na * 5) >> 2 : 0;
-                    for (int i = lane; i < full_words; i += 32) mo32[i] = mk32[i];
-                    for (int i = full_words * 4 + lane; i < na * 5; i += 32) a.action_mask_out[ag0 * 5 + i] = a.action_mask[ag0 * 5 + i];
-                }
-            }
-        }
+        pol_load_tile(a.local_obs, a.action_mask, a.action_mask_out, V2, ag0, na, raw, rawm, lane);
         __syncwarp();
-        // ---------------------------------------------------------------- feature row of agent `lane` (ENV:306-328 order: window, goal delta, pressure)
-        {
-            uint2 *row = reinterpret_cast<uint2 *>(xs + lane * S1);
-            const int off = lane * V2;
-            for (int j = 0; j < 4 * KC1; ++j) {   // 4 cells -> 4 bf16 per trip; columns beyond the window are zero
-                uint32_t w = 0;
-                if (j < NW) {
-                    const int b = off + 4 * j;
-                    w = __funnelshift_r(raw[b >> 2], raw[(b >> 2) + 1], (b & 3) * 8);
-                    if (4 * j + 4 > V2) w &= (1u << (8 * (V2 - 4 * j))) - 1u;
-                }
-                const __nv_bfloat162 lo = __floats2bfloat162_rn((float)(w & 0xFFu), (float)((w >> 8) & 0xFFu));
-                const __nv_bfloat162 hi = __floats2bfloat162_rn((float)((w >> 16) & 0xFFu), (float)(w >> 24));
-                row[j] = make_uint2(*reinterpret_cast<const uint32_t *>(&lo), *reinterpret_cast<const uint32_t *>(&hi));
-            }
-            if (lane < na) {
-                const float2 gd = reinterpret_cast<const float2 *>(a.goal_delta)[ag0 + lane];
-                xs[lane * S1 + V2] = __float2bfloat16(gd.x);
-                xs[lane * S1 + V2 + 1] = __float2bfloat16(gd.y);
-                if (a.blocking_prev) xs[lane * S1 + V2 + 2] = __float2bfloat16((float)a.blocking_prev[ag0 + lane]);
-            }
-            if (a.features_out) {   // float32 feature block for the learner (optional)
-                float *fo = a.features_out + ag0 * F;
-                const uint8_t *rb = reinterpret_cast<const uint8_t *>(raw);
-                for (int i = lane; i < na * F; i += 32) {
-                    const int r = i / F, c = i - r * F;
-                    float v;
-                    if (c < V2) v = (float)rb[r * V2 + c];
-                    else if (c < V2 + 2) v = a.goal_delta[(ag0 + r) * 2 + (c - V2)];
-                    else v = (float)a.blocking_prev[ag0 + r];
-                    fo[i] = v;
-                }
+        pol_feature_row<KC1>(xs, raw, a.goal_delta, a.blocking_prev, V2, ag0, na, lane);
+        if (a.features_out) {   // float32 feature block for the learner (optional)
+            float *fo = a.features_out + ag0 * F;
+            const uint8_t *rb = reinterpret_cast<const uint8_t *>(raw);
+            for (int i = lane; i < na * F; i += 32) {
+                const int r = i / F, c = i - r * F;
+                float v;
+                if (c < V2) v = (float)rb[r * V2 + c];
+                else if (c < V2 + 2) v = a.goal_delta[(ag0 + r) * 2 + (c - V2)];
+                else v = (float)a.blocking_prev[ag0 + r];
+                fo[i] = v;
             }
         }
         __syncwarp();
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt) {
             const int row0 = 16 * mt + g;   // this lane's rows: row0 and row0 + 8
-            // ------------------------------------------------------------ layer 1
-            uint32_t af[KC1][4];
-#pragma unroll
-            for (int kk = 0; kk < KC1; ++kk) {
-                const uint32_t *p0 = reinterpret_cast<const uint32_t *>(xs + row0 * S1 + 16 * kk + 2 * t);
-                const uint32_t *p1 = reinterpret_cast<const uint32_t *>(xs + (row0 + 8) * S1 + 16 * kk + 2 * t);
-                af[kk][0] = p0[0]; af[kk][1] = p1[0]; af[kk][2] = p0[4]; af[kk][3] = p1[4];
-            }
-            uint32_t h1[POL_H / 16][4];   // A fragments of layer 2
-#pragma unroll
-            for (int j = 0; j < POL_H / 8; ++j) {
-                const float2 bb = *reinterpret_cast<const float2 *>(bias + 8 * j + 2 * t);
-                float d[4] = {bb.x, bb.y, bb.x, bb.y};
-#pragma unroll
-                for (int kk = 0; kk < KC1; ++kk) {
-                    const uint32_t *wb = reinterpret_cast<const uint32_t *>(w1 + (8 * j + g) * S1 + 16 * kk + 2 * t);
-                    mma_bf16_16816(d, af[kk], wb[0], wb[4]);
-                }
-                h1[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);   // row g,   cols 8j + 2t, +1
-                h1[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);   // row g+8
-            }
-            // ------------------------------------------------------------ layer 2
             uint32_t h2[POL_H / 16][4];
-#pragma unroll
-            for (int j = 0; j < POL_H / 8; ++j) {
-                const float2 bb = *reinterpret_cast<const float2 *>(bias + POL_H + 8 * j + 2 * t);
-                float d[4] = {bb.x, bb.y, bb.x, bb.y};
-#pragma unroll
-                for (int kk = 0; kk < POL_H / 16; ++kk) {
-                    const uint32_t *wb = reinterpret_cast<const uint32_t *>(w2 + (8 * j + g) * POL_W2_STRIDE + 16 * kk + 2 * t);
-                    mma_bf16_16816(d, h1[kk], wb[0], wb[4]);
-                }
-                h2[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);
-                h2[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);
-            }
-            // ------------------------------------------------------------ heads: columns 0..4 logits, 5 value
-            const float2 bb = *reinterpret_cast<const float2 *>(bias + 2 * POL_H + 2 * t);
-            float d[4] = {bb.x, bb.y, bb.x, bb.y};
-#pragma unroll
-            for (int kk = 0; kk < POL_H / 16; ++kk) {
-                const uint32_t *wb = reinterpret_cast<const uint32_t *>(w3 + g * POL_W2_STRIDE + 16 * kk + 2 * t);
-                mma_bf16_16816(d, h2[kk], wb[0], wb[4]);
-            }
-            *reinterpret_cast<float2 *>(os + row0 * 8 + 2 * t) = make_float2(d[0], d[1]);
-            *reinterpret_cast<float2 *>(os + (row0 + 8) * 8 + 2 * t) = make_float2(d[2], d[3]);
+            pol_trunk<KC1>(xs, w1, w2, bias, row0, g, t, h2);
+            pol_heads(h2, w3, bias + 2 * POL_H, os, row0, g, t);
         }
         __syncwarp();
-        // ---------------------------------------------------------------- one agent per lane: mask, softmax, draw
-        if (lane < na) {
-            const long long ag = ag0 + lane;
-            const float4 o03 = *reinterpret_cast<const float4 *>(os + lane * 8);
-            const float2 o45 = *reinterpret_cast<const float2 *>(os + lane * 8 + 4);
-            float l[5] = {o03.x, o03.y, o03.z, o03.w, o45.x};
-            if (!a.no_masking && a.action_mask) {   // logits + clamp(log(mask + 1e-6), FLOAT_MIN), action_mask_model.py:57-61
-                const uint8_t *mk = reinterpret_cast<const uint8_t *>(rawm) + lane * 5;
-#pragma unroll
-                for (int k = 0; k < 5; ++k) l[k] += mk[k] ? 9.99999e-07f : -13.815511f;
-            }
-            float mx = l[0];
-#pragma unroll
-            for (int k = 1; k < 5; ++k) mx = fmaxf(mx, l[k]);
-            float pr[5], sum = 0.f;
-#pragma unroll
-            for (int k = 0; k < 5; ++k) { pr[k] = __expf(l[k] - mx); sum += pr[k]; }
-            const unsigned env = (unsigned)((unsigned long long)ag / (unsigned)N);   // B * N < 2^32 in any batch that fits a GPU
-            const int agent = (int)(ag - (long long)env * N);
-            Philox ph(a.seed ^ 0x504F4C49ull /* "POLI" */, a.env_id_base + env);
-            const uint4 x = ph((uint32_t)a.counter, (uint32_t)(a.counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
-            const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
-            int act = 0;
-            float cum = pr[0];
-#pragma unroll
-            for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
-            if (a.actions) a.actions[ag] = (int8_t)act;
-            if (a.actions64) a.actions64[ag] = (long long)act;
-            if (a.logp) a.logp[ag] = l[act] - mx - __logf(sum);
-            if (a.value) a.value[ag] = o45.y;
-            if (a.logits_out) {
-#pragma unroll
-                for (int k = 0; k < 5; ++k) a.logits_out[ag * 5 + k] = l[k];
-            }
-        }
+        if (lane < na) pol_sample(a, os, rawm, lane, ag0 + lane, N, 0x504F4C49ull /* "POLI" */);
         __syncwarp();
     }
 }

@@ -1,6 +1,6 @@
 """Rollout-loop CUDA kernels around the env step (BASELINE config 5): the action-mask MLP evaluated straight from the
-env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tensor-core MLP with f32 accumulation), and
-GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
+env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tensor-core MLP with f32 accumulation), the
+same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), and GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
 
@@ -70,6 +70,99 @@ class FusedPolicy:
             weights=p(self._dev), actions=p(self.actions), actions64=p(actions64), logp=p(logp), value=p(value),
             logits_out=p(logits_out), features_out=p(features_out), action_mask_out=p(mask_out))
         nat.check(self._lib.mapf_policy_act(C.byref(args), env._stream()))
+        return self.actions, logp, value
+
+
+class FusedRecurrentPolicy:
+    """Inference view of a :class:`recurrent.RecurrentActionMaskPolicy` of the reference's shape (trunk 64-64, LSTM
+    cell 64 fed with the previous action and reward): features -> trunk -> LSTM cell -> masked draw in ONE launch
+    (``mapf_lstm_policy_act``).  The module stays the learner's model: call :meth:`refresh` after every optimizer
+    step.  Other shapes are refused (``ValueError``); run those through the module itself."""
+
+    def __init__(self, policy, env, seed: int | None = None):
+        lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
+        F = int(env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0))
+        shape_ok = (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64
+                    and lin[1].in_features == 64 and lin[1].out_features == 64 and policy.cell == 64
+                    and policy.num_actions == 5 and policy.use_prev_action and policy.use_prev_reward
+                    and policy.lstm.input_size == 64 + 5 + 1 and policy.lstm.hidden_size == 64)
+        if not shape_ok:
+            raise ValueError("the fused LSTM kernel implements the reference's policy only: trunk (64, 64) over "
+                             f"F = V*V + 2 (+1) = {F} features, LSTM cell 64 with previous action and previous reward, "
+                             "5 actions")
+        self.policy, self.env, self.F, self._lin = policy, env, F, lin
+        self.with_bp = bool(env.include_blocking_pressure)
+        self._lib = nat.lib()
+        n = int(self._lib.mapf_lstm_policy_weights_nbytes(self.F))
+        if n < 0:
+            raise nat.MapfError(n, self._lib.mapf_last_error().decode())
+        self._host = np.zeros(n, np.uint8)
+        self._dev = torch.zeros(n, dtype=torch.uint8, device=env.device)
+        B, N, dev = env.B, env.N, env.device
+        self.actions = torch.zeros((B, N), dtype=torch.int8, device=dev)
+        self.actions64 = torch.zeros((B, N), dtype=torch.int64, device=dev)
+        self.logp = torch.zeros((B, N), dtype=torch.float32, device=dev)
+        self.value = torch.zeros((B, N), dtype=torch.float32, device=dev)
+        self.seed = int(env.cfg.seed if seed is None else seed) & (2 ** 64 - 1)
+        self.counter = 0
+        self.refresh()
+
+    def refresh(self):
+        """Re-pack the module's current float32 parameters (bf16, padded; b_ih + b_hh summed) and upload them."""
+        f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
+        p, lstm = self.policy, self.policy.lstm
+        arrs = [f(self._lin[0].weight), f(self._lin[0].bias), f(self._lin[1].weight), f(self._lin[1].bias),
+                f(lstm.weight_ih), f(lstm.weight_hh), f(lstm.bias_ih), f(lstm.bias_hh),
+                f(p.logits.weight), f(p.logits.bias), f(p.value.weight), f(p.value.bias)]
+        nat.check(self._lib.mapf_lstm_policy_pack_weights(self.F, *[a.ctypes.data_as(C.c_void_p) for a in arrs],
+                                                          self._host.ctypes.data_as(C.c_void_p)))
+        self._dev.copy_(torch.from_numpy(self._host))
+
+    def args(self, out_channels: dict, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *,
+             state_out=None, actions=None, actions64=None, logp=None, value=None, logits_out=None) -> nat.MapfLstmPolicyArgs:
+        """The argument block of one launch (counter 0; set ``.counter`` before launching).  ``out_channels`` maps
+        local_obs / goal_delta / blocking_prev / action_mask to device tensors; every other tensor argument may be None
+        (``state_out=None``: the state is not advanced)."""
+        env = self.env
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+        h, c = state
+        ho, co = (None, None) if state_out is None else state_out
+        return nat.MapfLstmPolicyArgs(
+            num_envs=env.B, num_agents=env.N, v2=env.V * env.V, feature_dim=self.F,
+            no_masking=0, reserved=0, seed=self.seed, counter=0, env_id_base=int(env.cfg.env_id_base),
+            local_obs=p(out_channels["local_obs"]), goal_delta=p(out_channels["goal_delta"]),
+            blocking_prev=p(out_channels["blocking_prev"]) if self.with_bp else None,
+            action_mask=p(out_channels["action_mask"]), prev_terminated=p(prev_terminated),
+            prev_truncated=p(prev_truncated), prev_action=p(prev_action), prev_reward=p(prev_reward),
+            h_in=p(h), c_in=p(c), h_out=p(ho), c_out=p(co), weights=p(self._dev), actions=p(actions),
+            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out))
+
+    def act(self, out, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *, advance: bool = True,
+            state_out=None, logits_out: torch.Tensor | None = None, logp: torch.Tensor | None = None,
+            value: torch.Tensor | None = None, actions64: torch.Tensor | None = None):
+        """One launch for the env's StepOutput ``out``.  ``state`` = (h, c) float32 [B*N, 64]; ``prev_action`` int8
+        [B,N] (may be :attr:`actions` itself), ``prev_reward`` float32 [B,N]; ``prev_terminated`` / ``prev_truncated``
+        uint8 [B] flag the envs whose episode starts at this step (their state, previous action and reward count as
+        zero).  With ``advance`` the new state goes to ``state_out`` (default: ``state``, in place) and the draw to
+        :attr:`actions`; without it (a bootstrap value) the state and :attr:`actions` -- the next step's previous
+        actions -- are left as they are and the draw goes to ``actions64`` only.  Returns (actions int8 [B,N], logp,
+        value); ``logits_out`` [B,N,5] receives the masked logits."""
+        for name, t, dt in (("h", state[0], torch.float32), ("c", state[1], torch.float32),
+                            ("prev_action", prev_action, torch.int8), ("prev_reward", prev_reward, torch.float32)):
+            if t.dtype != dt or not t.is_contiguous() or t.device != self.env.device:
+                raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.env.device}")
+        logp = self.logp if logp is None else logp
+        value = self.value if value is None else value
+        actions64 = self.actions64 if actions64 is None else actions64
+        ch = {"local_obs": out.local_obs, "goal_delta": out.goal_delta, "blocking_prev": out.blocking_prev,
+              "action_mask": out.action_mask}
+        a = self.args(ch, state, prev_action, prev_reward, prev_terminated, prev_truncated,
+                      state_out=(state if state_out is None else state_out) if advance else None,
+                      actions=self.actions if advance else None,
+                      actions64=actions64, logp=logp, value=value, logits_out=logits_out)
+        self.counter += 1
+        a.counter = self.counter
+        nat.check(self._lib.mapf_lstm_policy_act(C.byref(a), self.env._stream()))
         return self.actions, logp, value
 
 

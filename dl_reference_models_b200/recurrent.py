@@ -1,6 +1,6 @@
 """The recurrent policy of the reference's PPO configuration and a multi-GPU learner step around the batched env
-(SURVEY 8f N1; plain PyTorch by design -- the policy is the user's model, the env transition inside the loop is the
-CUDA kernel).
+(SURVEY 8f N1).  The module is plain PyTorch -- it is the user's model and the learner's; the rollout forward has a
+fused CUDA path for the reference's shape (:class:`FusedRecurrentCollector`, ``mapf_lstm_policy_act``).
 
 Reference: ``src/agents/ppo.py:67-75`` (``fcnet_hiddens [64, 64]``, ``use_lstm``, ``lstm_cell_size 64``,
 ``lstm_use_prev_action``, ``lstm_use_prev_reward``, ``max_seq_len 32``, ``vf_share_layers``) and ``:104-117``
@@ -12,6 +12,8 @@ Reference: ``src/agents/ppo.py:67-75`` (``fcnet_hiddens [64, 64]``, ``use_lstm``
   *channels* (uint8 window 25 B + float32 goal delta 8 B + pressure flag 1 B = 34 B per agent-step at sensor range 2)
   instead of float32 feature rows (112 B), and expands them per minibatch (:func:`features_from_channels`), plus the
   LSTM state at the start of every ``max_seq_len`` chunk (truncated back-propagation through time, as RLlib does).
+* :class:`FusedRecurrentCollector` -- the same :class:`CompactRollout` in two launches per step (fused LSTM policy +
+  draw, env step); ``python -m dl_reference_models_b200.recurrent`` times it against :class:`RecurrentCollector`.
 * :func:`ppo_update_recurrent` -- PPO on sequence minibatches; with ``world_size > 1`` every rank holds its own env
   shard and the gradients are all-reduced (mean) before each optimizer step: an N-GPU data-parallel learner whose
   only traffic is the ~50 k parameters' gradients (NCCL on GPUs, gloo in the CPU tests).
@@ -23,7 +25,7 @@ from dataclasses import dataclass
 import torch
 from torch import nn
 
-from .rollout import FLOAT_MIN, gae, sample_categorical
+from .rollout import FLOAT_MIN, gae, observation_rows, sample_categorical
 
 
 def features_from_channels(local_obs: torch.Tensor, goal_delta: torch.Tensor, blocking_prev: torch.Tensor | None) -> torch.Tensor:
@@ -163,6 +165,118 @@ class RecurrentCollector:
         return r
 
 
+class FusedRecurrentCollector:
+    """:class:`RecurrentCollector` with the forward pass and the draw in one CUDA launch
+    (:class:`policy_kernels.FusedRecurrentPolicy`): a step is exactly two launches, ``mapf_lstm_policy_act`` then
+    ``mapf_step``, with argument blocks built once here.  The layout is ``FusedCollector(compact=True)``'s: env step t
+    writes the observation channels into row t + 1 of [T + 1, ...] buffers and reward / terminated / truncated into row
+    t; the policy launch of step t reads channel row t, the reward and episode ends of step t - 1 (the carried ones at
+    t = 0), writes actions[t] / logp[t] / values[t] and advances the LSTM state in place.  The previous actions /
+    rewards, reset flags and chunk-start states of the :class:`CompactRollout` are filled with a few vectorised ops per
+    collect (one state snapshot per ``max_seq_len`` steps).  The returned batch's buffers are reused by the next
+    :meth:`collect`."""
+
+    def __init__(self, env, fused, steps: int, max_seq_len: int = 32):
+        import ctypes as C
+
+        from . import _native as nat
+
+        T, L = int(steps), int(max_seq_len)
+        if T % L:
+            raise ValueError(f"steps ({T}) must be a multiple of max_seq_len ({L})")
+        self.env, self.fused, self.T, self.L = env, fused, T, L
+        B, N, dev, cell = env.B, env.N, env.device, 64
+        o = env.out
+        self.obs_rows = observation_rows(env, T + 1)
+        z = lambda shape, dt=torch.float32: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
+        self.actions, self.prev_actions = z((T, B, N), torch.int64), z((T, B, N), torch.int64)
+        self.logp, self.values, self.rewards = z((T, B, N)), z((T, B, N)), z((T, B, N))
+        self.prev_rewards = z((T, B, N))
+        self.term, self.trunc = z((T, B), torch.uint8), z((T, B), torch.uint8)
+        self.last_value = z((B, N))
+        self.chunk_h, self.chunk_c = z((T // L, B * N, cell)), z((T // L, B * N, cell))
+        # carried across collects, as RecurrentCollector does: state, previous action / reward, episode-start flags
+        self.state = (z((B * N, cell)), z((B * N, cell)))
+        self.act8 = z((B, N), torch.int8)   # this step's actions (to mapf_step) = the next step's previous actions
+        self.prev_reward = z((B, N))
+        self.prev_term, self.prev_trunc = torch.ones((B,), dtype=torch.uint8, device=dev), z((B,), torch.uint8)
+        self._C, self._nat, self._lib = C, nat, nat.lib()
+        rows = self.obs_rows
+
+        def policy_args(t):
+            last = t == T
+            ch = {k: r[t] for k, r in rows.items()}
+            pr, pt, ptr = (self.prev_reward, self.prev_term, self.prev_trunc) if t == 0 else \
+                (self.rewards[t - 1], self.term[t - 1], self.trunc[t - 1])
+            return fused.args(ch, self.state, self.act8, pr, pt, ptr, state_out=None if last else self.state,
+                              actions=None if last else self.act8, actions64=None if last else self.actions[t],
+                              logp=None if last else self.logp[t], value=self.last_value if last else self.values[t])
+
+        self._pargs = [policy_args(t) for t in range(T + 1)]   # the last one: bootstrap value, state not advanced
+
+        def dst(k, t):   # where the env step t writes channel k
+            if k == "reward":
+                return self.rewards[t]
+            if k == "terminated":
+                return self.term[t]
+            if k == "truncated":
+                return self.trunc[t]
+            if k in rows:
+                return rows[k][t + 1]
+            return o[k]
+
+        self._couts = [nat.MapfOutputs(**{k: dst(k, t).data_ptr() for k in nat.OUTPUT_FIELDS}) for t in range(T)]
+        self._actions_ptr = C.c_void_p(self.act8.data_ptr())
+
+    @torch.no_grad()
+    def collect(self) -> CompactRollout:
+        """Roll T steps from the env's current observation (its output buffers, i.e. the last reset / step)."""
+        C, lib, env, fused, T, L = self._C, self._lib, self.env, self.fused, self.T, self.L
+        if getattr(env, "_fused", 0):
+            raise RuntimeError("turn the env's fused uniform sampler off (fuse_sampler(None)) before a policy rollout")
+        B, N = env.B, env.N
+        stream, hnd, check = env._stream(), env._h, self._nat.check
+        h, c = self.state
+        for k, r in self.obs_rows.items():   # row 0 = the env's current observation
+            r[0].copy_(env.out[k])
+        # step 0's previous action / reward / episode start are the carried ones (read before step 0 overwrites them)
+        resets = torch.empty((T, B), dtype=torch.bool, device=env.device)
+        resets[0] = (self.prev_term | self.prev_trunc).bool()
+        self.prev_actions[0].copy_(self.act8)
+        self.prev_rewards[0].copy_(self.prev_reward)
+        for t in range(T):
+            if t % L == 0:   # the chunk's start state after the episode-start cut (RecurrentCollector's h * keep)
+                keep = (~(resets[0] if t == 0 else (self.term[t - 1] | self.trunc[t - 1]).bool())).to(h.dtype).view(B, 1, 1)
+                torch.mul(h.view(B, N, -1), keep, out=self.chunk_h[t // L].view(B, N, -1))
+                torch.mul(c.view(B, N, -1), keep, out=self.chunk_c[t // L].view(B, N, -1))
+            fused.counter += 1
+            a = self._pargs[t]
+            a.counter = fused.counter
+            check(lib.mapf_lstm_policy_act(C.byref(a), stream))
+            check(lib.mapf_step(hnd, self._actions_ptr, None, None, C.byref(self._couts[t]), 1, stream))
+        fused.counter += 1
+        a = self._pargs[T]
+        a.counter = fused.counter
+        check(lib.mapf_lstm_policy_act(C.byref(a), stream))
+        dones = (self.term | self.trunc).bool()
+        resets[1:] = dones[:-1]
+        self.prev_actions[1:] = self.actions[:-1]
+        self.prev_rewards[1:] = self.rewards[:-1]
+        keep = (~resets).unsqueeze(-1)
+        self.prev_actions.mul_(keep)
+        self.prev_rewards.mul_(keep)
+        # carried into the next collect; act8 already holds the last step's actions
+        self.prev_reward.copy_(self.rewards[T - 1])
+        self.prev_term.copy_(self.term[T - 1])
+        self.prev_trunc.copy_(self.trunc[T - 1])
+        for k, r in self.obs_rows.items():   # the env's own buffers show the latest observation again
+            env.out[k].copy_(r[T])
+        rows = self.obs_rows
+        return CompactRollout(rows["local_obs"][:T], rows["goal_delta"][:T], rows["blocking_prev"][:T],
+                              rows["action_mask"][:T], self.actions, self.prev_actions, self.prev_rewards, resets,
+                              self.logp, self.values, self.rewards, dones, self.last_value, self.chunk_h, self.chunk_c)
+
+
 def collect_recurrent(env, policy, steps: int, max_seq_len: int = 32) -> CompactRollout:
     return RecurrentCollector(env, policy, max_seq_len).collect(steps)
 
@@ -234,3 +348,63 @@ def ppo_update_recurrent(policy: RecurrentActionMaskPolicy, optimizer, batch: Co
             if max_minibatches is not None and done_mb >= max_minibatches:
                 return stats
     return stats
+
+
+def benchmark(num_envs: int = 65536, steps: int = 64, max_seq_len: int = 32, rounds: int = 3, device: str = "cuda:0") -> dict:
+    """C3 (num_envs x 16 agents, 32x32 map, lifelong): agent-steps/s of the env alone, of :class:`RecurrentCollector`
+    (the PyTorch module's forward every step) and of :class:`FusedRecurrentCollector` (one policy launch + one env
+    launch per step), the two collectors alternated in the same process after a warm-up collect each.  Rates are the
+    best of ``rounds`` timed collects (host clock around work that ends in a device synchronise)."""
+    import subprocess
+    import time
+
+    from . import maps
+    from .batched_env import BatchedMapfEnv
+    from .policy_kernels import FusedRecurrentPolicy
+
+    cfg = {"num_agents": 16, "sensor_range": 2, "steps_per_episode": 256, "lifelong_mapf": True, "seed": 999,
+           "grid": maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32)}
+    env = BatchedMapfEnv(cfg, num_envs, device)
+    env.reset()
+    n = num_envs * env.N * steps
+
+    def timed(fn):
+        torch.cuda.synchronize(env.device)
+        t0 = time.perf_counter()
+        fn()
+        torch.cuda.synchronize(env.device)
+        return time.perf_counter() - t0
+
+    a = env.sample_actions(masked=True)
+    env.fuse_sampler("masked")
+    for _ in range(8):
+        env.step(a, auto_reset=True)
+    env_s = min(timed(lambda: [env.step(a, auto_reset=True) for _ in range(steps)]) for _ in range(rounds))
+    env.fuse_sampler(None)
+    torch.manual_seed(0)
+    pol = RecurrentActionMaskPolicy(env.flat_obs_dim(include_action_mask=False)).to(env.device)
+    torch_col = RecurrentCollector(env, pol, max_seq_len)
+    fused_col = FusedRecurrentCollector(env, FusedRecurrentPolicy(pol, env), steps, max_seq_len)
+    torch_col.collect(steps)   # warm-up: allocator, cuBLAS / kernel selection, module load
+    fused_col.collect()
+    ts, fs = [], []
+    for _ in range(rounds):
+        ts.append(timed(lambda: torch_col.collect(steps)))
+        fs.append(timed(fused_col.collect))
+    try:
+        gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i",
+                              str(env.device.index)], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        gpu = f"nvidia-smi not readable: {exc}"
+    assert env.poll_errors() == 0
+    return {"gpu": gpu or torch.cuda.get_device_name(env.device), "envs": num_envs, "agents": env.N, "steps": steps,
+            "max_seq_len": max_seq_len, "env_only_agent_steps_per_s": n / env_s,
+            "torch_recurrent_collector_agent_steps_per_s": n / min(ts),
+            "fused_recurrent_collector_agent_steps_per_s": n / min(fs),
+            "torch_collect_s": ts, "fused_collect_s": fs}
+
+
+if __name__ == "__main__":
+    import json
+
+    print(json.dumps(benchmark()))

@@ -105,6 +105,18 @@ def sample_categorical(logits: torch.Tensor):
     return a, torch.gather(logp_all, -1, a.unsqueeze(-1)).squeeze(-1)
 
 
+def observation_rows(env, rows: int) -> dict:
+    """[rows, *shape] buffers of the env's observation channels (local_obs, goal_delta, blocking_prev, action_mask) with
+    every row 256-byte aligned (the kernels store 128-bit words): a compact rollout's per-step rows."""
+    def rows_of(t):
+        n, es = t.numel(), t.element_size()
+        stride = -(-(n * es) // 256) * 256 // es
+        buf = torch.empty((rows, stride), dtype=t.dtype, device=env.device)
+        return buf[:, :n].view((rows,) + tuple(t.shape))
+
+    return {k: rows_of(env.out[k]) for k in ("local_obs", "goal_delta", "blocking_prev", "action_mask")}
+
+
 class FusedCollector:
     """T-step rollouts with two kernel launches per env step and nothing else: the policy kernel
     (:class:`policy_kernels.FusedPolicy`: bf16 tensor-core MLP straight from the env's output channels + masked draw)
@@ -124,15 +136,7 @@ class FusedCollector:
         if self.compact:
             # compact rollout: the env step writes the observation channels of step t straight into row t + 1 of
             # [T + 1, ...] buffers, the policy kernel reads row t and stores no feature block at all
-            o = env.out
-
-            def rows_of(t):   # [T + 1, *t.shape] with every row 256-byte aligned (the kernels store 128-bit words)
-                n, es = t.numel(), t.element_size()
-                stride = -(-(n * es) // 256) * 256 // es
-                buf = torch.empty((T + 1, stride), dtype=t.dtype, device=dev)
-                return buf[:, :n].view((T + 1,) + tuple(t.shape))
-
-            self.obs_rows = {k: rows_of(o[k]) for k in ("local_obs", "goal_delta", "blocking_prev", "action_mask")}
+            self.obs_rows = observation_rows(env, T + 1)
             self.feats = None
             self.masks = self.obs_rows["action_mask"][:T]
         else:

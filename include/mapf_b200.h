@@ -441,6 +441,50 @@ int mapf_policy_pack_weights(int32_t feature_dim, const float *w1, const float *
                              const float *w_logits, const float *b_logits, const float *w_value, const float *b_value,
                              void *packed_host);
 int mapf_policy_act(const mapf_policy_args *args, void *stream);
+
+/* The recurrent policy of the reference's PPO configuration (src/agents/ppo.py:67-75): the same 64-64 ReLU trunk,
+ * then an LSTM cell of 64 fed with [trunk output | one_hot(previous action, 5) | previous reward] (torch LSTMCell
+ * layout, gate rows [i; f; g; o]), then logits (masked as above) and value, both reading the new h.  One launch per
+ * step: features from the env's output channels, bf16 tensor-core GEMMs with f32 accumulation, the cell update in f32
+ * (c stays f32), the masked inverse-CDF draw from Philox (a stream of its own, distinct from mapf_policy_act's). */
+typedef struct mapf_lstm_policy_args {
+    int32_t num_envs, num_agents;
+    int32_t v2;           /* window cells, V * V */
+    int32_t feature_dim;  /* F = v2 + 2 + (blocking_prev ? 1 : 0), <= 64: order of ENV:306-328 without the mask */
+    int32_t no_masking;   /* action_mask_model.py:33 */
+    int32_t reserved;
+    uint64_t seed;        /* Philox key (with env_id_base + env), counter = (counter, agent) */
+    uint64_t counter;
+    int64_t env_id_base;
+    const uint8_t *local_obs;       /* [B,N,V,V]   device, the env's outputs */
+    const float *goal_delta;        /* [B,N,2] */
+    const uint8_t *blocking_prev;   /* [B,N] or NULL */
+    const int8_t *action_mask;      /* [B,N,5] or NULL (no masking) */
+    const uint8_t *prev_terminated; /* [B] or NULL: nonzero = this step starts an episode (h, c, previous action and */
+    const uint8_t *prev_truncated;  /* [B] or NULL     previous reward count as zero for every agent of the env)     */
+    const int8_t *prev_action;      /* [B,N] in 0..4, may alias `actions` (each agent's is read before it is written) */
+    const float *prev_reward;       /* [B,N] */
+    const float *h_in;              /* [B*N,64] LSTM state, float32 */
+    const float *c_in;              /* [B*N,64] */
+    float *h_out;                   /* [B*N,64] new state, may equal h_in / c_in; both NULL = do not advance the */
+    float *c_out;                   /* [B*N,64]   state (h_in, c_in untouched); one NULL without the other is an error */
+    const void *weights;            /* device copy of the block written by mapf_lstm_policy_pack_weights */
+    int8_t *actions;                /* [B,N] sampled action (feeds mapf_step), may be NULL */
+    int64_t *actions64;             /* [B,N] the same as int64, may be NULL */
+    float *logp;                    /* [B,N] log-probability of the sampled action, may be NULL */
+    float *value;                   /* [B,N] value head, may be NULL */
+    float *logits_out;              /* [B,N,5] masked logits, may be NULL */
+} mapf_lstm_policy_args;
+
+/* Bytes of the packed LSTM policy weight block for feature_dim F (negative = unsupported F). */
+int64_t mapf_lstm_policy_weights_nbytes(int32_t feature_dim);
+/* HOST float32 weights in torch's layouts (Linear [out, in]; LSTMCell weight_ih [256, 70], weight_hh [256, 64],
+ * b_ih / b_hh [256]) -> HOST packed block (bf16 weights, padded; b_ih + b_hh summed in f32). */
+int mapf_lstm_policy_pack_weights(int32_t feature_dim, const float *w1, const float *b1, const float *w2, const float *b2,
+                                  const float *w_ih, const float *w_hh, const float *b_ih, const float *b_hh,
+                                  const float *w_logits, const float *b_logits, const float *w_value, const float *b_value,
+                                  void *packed_host);
+int mapf_lstm_policy_act(const mapf_lstm_policy_args *args, void *stream);
 /* rewards / values / adv / ret: device float32 [T,B,N]; dones uint8 [T,B]; last_value float32 [B,N]. */
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
              float *ret, int32_t T, int64_t B, int32_t N, float gamma, float lam, void *stream);

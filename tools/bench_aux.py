@@ -1,5 +1,5 @@
 """Timings of the kernels next to the hot path (CUDA events, warm-up, L2-sized working sets): the fused policy
-kernel, the GAE scan, the single-agent (CTE) step.  Prints one JSON object.  `python tools/bench_aux.py`"""
+kernels (MLP and LSTM-64), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.  `python tools/bench_aux.py`"""
 import json
 import sys
 from pathlib import Path
@@ -10,6 +10,7 @@ sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 
 from dl_reference_models_b200 import maps, policy_kernels  # noqa: E402
 from dl_reference_models_b200.batched_env import BatchedMapfEnv  # noqa: E402
+from dl_reference_models_b200.recurrent import RecurrentActionMaskPolicy  # noqa: E402
 from dl_reference_models_b200.rollout import ActionMaskPolicy  # noqa: E402
 from dl_reference_models_b200.single_agent import BatchedCteEnv  # noqa: E402
 
@@ -61,6 +62,30 @@ def main():
     except Exception as exc:   # no peaks file on this box
         res["policy_act"]["bf16_peak_TFLOPs"] = None
         res["policy_act"]["frac_note"] = f"MEASURED_PEAKS.json not readable: {exc}"
+    # fused LSTM-64 policy (mapf_lstm_policy_act), same 4-env rotation; state advanced in place, episode starts off
+    lstm = RecurrentActionMaskPolicy(envs[0].flat_obs_dim(include_action_mask=False)).cuda()
+    lfused = [policy_kernels.FusedRecurrentPolicy(lstm, e) for e in envs]
+    lstate = [(torch.randn(B * N, 64, device="cuda") * 0.1, torch.randn(B * N, 64, device="cuda") * 0.1) for _ in envs]
+    lprev = [(torch.randint(0, 5, (B, N), dtype=torch.int8, device="cuda"), torch.zeros(B, N, device="cuda")) for _ in envs]
+
+    def lstm_act():
+        k = i[0] % 4
+        lfused[k].act(outs[k], lstate[k], *lprev[k])
+        i[0] += 1
+
+    s = timed(lstm_act, 200)
+    # byte / FLOP model per agent: channels 25 + 8 + 1 + 5, prev action 1, prev reward 4, h 256, c 256 in;
+    # h 256, c 256, actions 1 + 8, logp 4, value 4 out.  GEMMs without padding: F x 64, 64 x 64, (70 + 64) x 256, 64 x 6
+    lstm_bytes = (25 + 8 + 1 + 5 + 1 + 4 + 256 + 256) + (256 + 256 + 1 + 8 + 4 + 4)
+    lstm_flops = 2 * (28 * 64 + 64 * 64 + (70 + 64) * 256 + 64 * 6)
+    hbm_tbs, bf16_tflops = 6.45, 2250.0   # SURVEY 8d measured copy bandwidth; dense bf16 data-sheet rate (tcgen05)
+    gbps, tflops = lstm_bytes * B * N / s / 1e9, lstm_flops * B * N / s / 1e12
+    res["lstm_policy_act"] = {"us_per_launch": s * 1e6, "agents": B * N, "bytes_per_agent": lstm_bytes,
+                              "flops_per_agent": lstm_flops, "GBps": gbps, "TFLOPs": tflops,
+                              "agent_steps_per_s": B * N / s, "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3),
+                              "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops,
+                              "hbm_floor_us": lstm_bytes * B * N / (hbm_tbs * 1e12) * 1e6}
+    del lstate, lprev
     T = 64
     rewards, values = torch.randn(T, B, N, device="cuda"), torch.randn(T, B, N, device="cuda")
     dones = torch.rand(T, B, device="cuda") < 0.01
