@@ -17,7 +17,7 @@ REPO = PKG.parent
 CSRC = PKG / "csrc"
 LIB_PATH = Path(os.environ.get("MAPF_B200_LIB", PKG / "libmapf_b200.so"))
 SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_kernel.cuh", CSRC / "mapf_pair_kernel.cuh", CSRC / "mapf_cte_kernel.cuh", CSRC / "mapf_policy_kernel.cuh",
-           CSRC / "mapf_policy_lstm_kernel.cuh",
+           CSRC / "mapf_policy_lstm_kernel.cuh", CSRC / "mapf_eval_kernel.cuh",
            CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
@@ -99,7 +99,7 @@ class MapfPolicyArgs(C.Structure):
 
     _fields_ = [
         ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("v2", C.c_int32), ("feature_dim", C.c_int32),
-        ("no_masking", C.c_int32), ("reserved", C.c_int32),
+        ("no_masking", C.c_int32), ("greedy", C.c_int32),
         ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
     ] + [(k, C.c_void_p) for k in (
         "local_obs", "goal_delta", "blocking_prev", "action_mask", "weights", "actions", "actions64", "logp", "value",
@@ -111,11 +111,19 @@ class MapfLstmPolicyArgs(C.Structure):
 
     _fields_ = [
         ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("v2", C.c_int32), ("feature_dim", C.c_int32),
-        ("no_masking", C.c_int32), ("reserved", C.c_int32),
+        ("no_masking", C.c_int32), ("greedy", C.c_int32),
         ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
     ] + [(k, C.c_void_p) for k in (
         "local_obs", "goal_delta", "blocking_prev", "action_mask", "prev_terminated", "prev_truncated", "prev_action",
         "prev_reward", "h_in", "c_in", "h_out", "c_out", "weights", "actions", "actions64", "logp", "value", "logits_out")]
+
+
+class MapfEvalArgs(C.Structure):
+    """mapf_eval_args of include/mapf_b200.h (the evaluator's per-step bookkeeping)."""
+
+    _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("step", C.c_int64)] + [(k, C.c_void_p) for k in (
+        "reward", "terminated", "truncated", "info", "active", "episode_reward", "agent_reward", "timesteps", "success",
+        "last_info", "active_count")]
 
 
 class MapfError(RuntimeError):
@@ -218,6 +226,7 @@ def lib():
     L.mapf_lstm_policy_pack_weights.argtypes = [i32] + [vp] * 13
     L.mapf_lstm_policy_act.argtypes = [C.POINTER(MapfLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
+    L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
@@ -238,7 +247,7 @@ EXPORTS = (
     "mapf_sample_random_actions", "mapf_set_fused_sampler", "mapf_metrics_reduce", "mapf_poll_errors", "mapf_launch_count",
     "mapf_step_kernel_kind", "mapf_cte_step", "mapf_cte_reset", "mapf_occupancy_accumulate", "mapf_distance_table", "mapf_goal_path_lengths",
     "mapf_policy_weights_nbytes", "mapf_policy_pack_weights", "mapf_policy_act", "mapf_gae",
-    "mapf_lstm_policy_weights_nbytes", "mapf_lstm_policy_pack_weights", "mapf_lstm_policy_act",
+    "mapf_lstm_policy_weights_nbytes", "mapf_lstm_policy_pack_weights", "mapf_lstm_policy_act", "mapf_eval_accumulate",
 )
 
 

@@ -7,6 +7,7 @@
 #include "mapf_cte_kernel.cuh"
 #include "mapf_policy_kernel.cuh"
 #include "mapf_policy_lstm_kernel.cuh"
+#include "mapf_eval_kernel.cuh"
 #include "mapf_pack_kernel.cuh"
 #include "mapf_host_unpack.h"
 
@@ -1642,6 +1643,7 @@ int mapf_policy_act(const mapf_policy_args *a, void *stream) {
                     a->feature_dim, a->v2);
     if (a->num_envs < 1 || a->num_agents < 1 || !a->local_obs || !a->goal_delta || !a->weights)
         return fail(MAPF_ERR_INVALID_ARG, "policy: env outputs and weights are required");
+    if (a->greedy != 0 && a->greedy != 1) return fail(MAPF_ERR_INVALID_ARG, "policy: greedy %d is neither 0 nor 1", a->greedy);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
@@ -1651,15 +1653,12 @@ int mapf_policy_act(const mapf_policy_args *a, void *stream) {
     long long blocks = (tiles + warps - 1) / warps;
     if (blocks > 148 * 8) blocks = 148 * 8;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (kc1 == 2) {
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_policy_act_kernel<2>),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mapf::mapf_policy_act_kernel<2><<<(unsigned)blocks, threads, smem, st>>>(*a);
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_policy_act_kernel<4>),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mapf::mapf_policy_act_kernel<4><<<(unsigned)blocks, threads, smem, st>>>(*a);
-    }
+    void (*const kernels[2][2])(const mapf_policy_args) = {
+        {mapf::mapf_policy_act_kernel<2, false>, mapf::mapf_policy_act_kernel<2, true>},
+        {mapf::mapf_policy_act_kernel<4, false>, mapf::mapf_policy_act_kernel<4, true>}};
+    const auto kernel = kernels[kc1 == 4][a->greedy];
+    CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<(unsigned)blocks, threads, smem, st>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }
@@ -1713,6 +1712,8 @@ int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
         return fail(MAPF_ERR_INVALID_ARG, "lstm policy: prev_action, prev_reward, h_in and c_in are required");
     if (!a->h_out != !a->c_out)
         return fail(MAPF_ERR_INVALID_ARG, "lstm policy: h_out and c_out are given together (both NULL = state not advanced)");
+    if (a->greedy != 0 && a->greedy != 1)
+        return fail(MAPF_ERR_INVALID_ARG, "lstm policy: greedy %d is neither 0 nor 1", a->greedy);
     int ndev = 0, dev = 0, sms = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
@@ -1724,15 +1725,12 @@ int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
     long long blocks = (tiles + warps - 1) / warps;
     if (blocks > sms) blocks = sms;   // one resident block per SM loads the weights once and loops over the tiles
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (kc1 == 2) {
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_lstm_policy_act_kernel<2>),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mapf::mapf_lstm_policy_act_kernel<2><<<(unsigned)blocks, threads, smem, st>>>(*a);
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(mapf::mapf_lstm_policy_act_kernel<4>),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mapf::mapf_lstm_policy_act_kernel<4><<<(unsigned)blocks, threads, smem, st>>>(*a);
-    }
+    void (*const kernels[2][2])(const mapf_lstm_policy_args) = {
+        {mapf::mapf_lstm_policy_act_kernel<2, false>, mapf::mapf_lstm_policy_act_kernel<2, true>},
+        {mapf::mapf_lstm_policy_act_kernel<4, false>, mapf::mapf_lstm_policy_act_kernel<4, true>}};
+    const auto kernel = kernels[kc1 == 4][a->greedy];
+    CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<(unsigned)blocks, threads, smem, st>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }
@@ -1744,6 +1742,26 @@ int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, co
     const long long BN = (long long)B * N;
     mapf::mapf_gae_kernel<<<(unsigned)((BN + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         rewards, values, dones, last_value, adv, ret, T, BN, N, gamma, lam);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_eval_accumulate(const mapf_eval_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    if (a->num_envs < 1 || a->num_agents < 1 || !a->reward || !a->terminated || !a->truncated || !a->info || !a->active ||
+        !a->episode_reward || !a->agent_reward || !a->timesteps || !a->success || !a->last_info || !a->active_count)
+        return fail(MAPF_ERR_INVALID_ARG, "eval: null or empty argument");
+    if (a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "eval: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    int P = 1;   // lanes per env: N rounded up to a power of two
+    while (P < a->num_agents) P <<= 1;
+    const int envs_per_block = mapf::EVAL_THREADS / 32 * (32 / P);
+    long long blocks = ((long long)a->num_envs + envs_per_block - 1) / envs_per_block;
+    if (blocks > 148 * 8) blocks = 148 * 8;   // one resident wave; the count then costs one atomic per block
+    mapf::mapf_eval_accumulate_kernel<<<(unsigned)blocks, mapf::EVAL_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a, P);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }

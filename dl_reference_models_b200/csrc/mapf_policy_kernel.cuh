@@ -151,9 +151,12 @@ __device__ __forceinline__ void pol_heads(const uint32_t (&hf)[POL_H / 16][4], c
     *reinterpret_cast<float2 *>(os + (row0 + 8) * 8 + 2 * t) = make_float2(d[2], d[3]);
 }
 
-// one agent per lane (call for lane < na): mask, stable softmax, inverse-CDF draw from one Philox word keyed by
-// (seed ^ tag, env_id_base + env), counter (counter, agent); writes the outputs of `a` that are not NULL
-template <class Args>
+// one agent per lane (call for lane < na): mask, stable softmax, then the action: with GREEDY the first index of the
+// largest masked logit (torch.argmax's tie rule), otherwise an inverse-CDF draw from one Philox word keyed by
+// (seed ^ tag, env_id_base + env), counter (counter, agent); writes the outputs of `a` that are not NULL.  GREEDY is a
+// template parameter, not a runtime branch: the draw instantiation then compiles to the same code as a draw-only kernel
+// (the LSTM kernel has no register to spare).
+template <bool GREEDY, class Args>
 __device__ __forceinline__ void pol_sample(const Args &a, const float *os, const uint32_t *rawm, int lane, long long ag, int N,
                                            unsigned long long tag) {
     const float4 o03 = *reinterpret_cast<const float4 *>(os + lane * 8);
@@ -170,15 +173,21 @@ __device__ __forceinline__ void pol_sample(const Args &a, const float *os, const
     float pr[5], sum = 0.f;
 #pragma unroll
     for (int k = 0; k < 5; ++k) { pr[k] = __expf(l[k] - mx); sum += pr[k]; }
-    const unsigned env = (unsigned)((unsigned long long)ag / (unsigned)N);   // B * N < 2^32 in any batch that fits a GPU
-    const int agent = (int)(ag - (long long)env * N);
-    Philox ph(a.seed ^ tag, a.env_id_base + env);
-    const uint4 x = ph((uint32_t)a.counter, (uint32_t)(a.counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
-    const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
     int act = 0;
-    float cum = pr[0];
+    if constexpr (GREEDY) {
+        float best = l[0];
 #pragma unroll
-    for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
+        for (int k = 1; k < 5; ++k) { if (l[k] > best) { best = l[k]; act = k; } }
+    } else {
+        const unsigned env = (unsigned)((unsigned long long)ag / (unsigned)N);   // B * N < 2^32 in any batch that fits a GPU
+        const int agent = (int)(ag - (long long)env * N);
+        Philox ph(a.seed ^ tag, a.env_id_base + env);
+        const uint4 x = ph((uint32_t)a.counter, (uint32_t)(a.counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
+        const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
+        float cum = pr[0];
+#pragma unroll
+        for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
+    }
     if (a.actions) a.actions[ag] = (int8_t)act;
     if (a.actions64) a.actions64[ag] = (long long)act;
     if (a.logp) a.logp[ag] = l[act] - mx - __logf(sum);
@@ -189,8 +198,8 @@ __device__ __forceinline__ void pol_sample(const Args &a, const float *os, const
     }
 }
 
-// KC1 = k16 chunks of the first layer (F <= 16 * KC1), W1 row stride = 16 * KC1 + 8
-template <int KC1>
+// KC1 = k16 chunks of the first layer (F <= 16 * KC1), W1 row stride = 16 * KC1 + 8; GREEDY = a.greedy (argmax, no draw)
+template <int KC1, bool GREEDY>
 __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_args a) {
     constexpr int S1 = 16 * KC1 + 8;   // bf16 row stride of the feature tile and of W1
     extern __shared__ __align__(16) unsigned char psm[];
@@ -244,7 +253,7 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
             pol_heads(h2, w3, bias + 2 * POL_H, os, row0, g, t);
         }
         __syncwarp();
-        if (lane < na) pol_sample(a, os, rawm, lane, ag0 + lane, N, 0x504F4C49ull /* "POLI" */);
+        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, ag0 + lane, N, 0x504F4C49ull /* "POLI" */);
         __syncwarp();
     }
 }

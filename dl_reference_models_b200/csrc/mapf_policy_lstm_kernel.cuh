@@ -51,7 +51,9 @@ __device__ __forceinline__ void lstm_gate_chunk(float (&d)[4][4], const uint32_t
     }
 }
 
-template <int KC1>
+// GREEDY = a.greedy: argmax instead of the draw, in the epilogue only, where the gate fragments are dead (see
+// pol_sample for why it is a template parameter)
+template <int KC1, bool GREEDY>
 __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(const mapf_lstm_policy_args a) {
     constexpr int S1 = 16 * KC1 + 8;
     extern __shared__ __align__(16) unsigned char psm[];
@@ -173,7 +175,7 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
             pol_heads(hn, w3, bias + 2 * POL_H, os, row0, g, t);
         }
         __syncwarp();
-        if (lane < na) pol_sample(a, os, rawm, lane, ag0 + lane, N, 0x4C53544Dull /* "LSTM" */);
+        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, ag0 + lane, N, 0x4C53544Dull /* "LSTM" */);
         __syncwarp();
     }
 }

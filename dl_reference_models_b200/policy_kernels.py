@@ -1,6 +1,6 @@
 """Rollout-loop CUDA kernels around the env step (BASELINE config 5): the action-mask MLP evaluated straight from the
 env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tensor-core MLP with f32 accumulation), the
-same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), and GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
+same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a greedy (argmax) mode for evaluation, and GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
 
@@ -22,10 +22,8 @@ class FusedPolicy:
         self.F = int(env.flat_obs_dim(include_action_mask=False))
         self.with_bp = bool(env.include_blocking_pressure)
         assert self.F == env.V * env.V + 2 + (1 if self.with_bp else 0)
-        lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
-        assert len(lin) == 2 and lin[0].out_features == 64 and lin[1].out_features == 64 and lin[0].in_features == self.F, \
-            "the fused kernel implements the reference's 64-64 action-mask MLP"
-        self._lin = lin
+        assert FusedPolicy.matches(policy, env), "the fused kernel implements the reference's 64-64 action-mask MLP"
+        self._lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
         n = int(self._lib.mapf_policy_weights_nbytes(self.F))
         if n < 0:
             raise nat.MapfError(n, self._lib.mapf_last_error().decode())
@@ -41,6 +39,15 @@ class FusedPolicy:
         self.counter = 0
         self.refresh()
 
+    @staticmethod
+    def matches(policy, env) -> bool:
+        """Whether the fused kernel implements ``policy`` (an :class:`rollout.ActionMaskPolicy`) at ``env``'s feature
+        width: trunk Linear(F, 64)-ReLU-Linear(64, 64)-ReLU over F = V*V + 2 (+1 pressure) features, 5 logits."""
+        F = env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0)
+        lin = [m for m in policy.trunk.modules() if isinstance(m, torch.nn.Linear)]
+        return (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64 and lin[1].in_features == 64
+                and lin[1].out_features == 64 and policy.logits.out_features == 5)
+
     def refresh(self):
         """Re-pack the module's current float32 parameters (bf16, padded) and upload them."""
         f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
@@ -52,8 +59,9 @@ class FusedPolicy:
 
     def act(self, out, logits_out: torch.Tensor | None = None, features_out: torch.Tensor | None = None,
             logp: torch.Tensor | None = None, value: torch.Tensor | None = None, actions64: torch.Tensor | None = None,
-            mask_out: torch.Tensor | None = None):
-        """One launch: features from ``out`` (the env's StepOutput) -> MLP -> masked categorical draw.
+            mask_out: torch.Tensor | None = None, greedy: bool = False):
+        """One launch: features from ``out`` (the env's StepOutput) -> MLP -> masked categorical draw (``greedy``: the
+        first argmax of the masked logits instead, as RLlib's ``forward_inference``).
         Returns (actions int8 [B,N], logp, value); optional tensors receive the masked logits / the float feature
         block / a copy of the action masks (the rollout buffer's rows, so the loop needs no copy launches)."""
         env = self.env
@@ -64,7 +72,7 @@ class FusedPolicy:
         self.counter += 1
         args = nat.MapfPolicyArgs(
             num_envs=env.B, num_agents=env.N, v2=env.V * env.V, feature_dim=self.F,
-            no_masking=int(bool(self.policy.no_masking)), reserved=0, seed=self.seed, counter=self.counter,
+            no_masking=int(bool(self.policy.no_masking)), greedy=int(bool(greedy)), seed=self.seed, counter=self.counter,
             env_id_base=int(env.cfg.env_id_base), local_obs=p(out.local_obs), goal_delta=p(out.goal_delta),
             blocking_prev=p(out.blocking_prev) if self.with_bp else None, action_mask=p(out.action_mask),
             weights=p(self._dev), actions=p(self.actions), actions64=p(actions64), logp=p(logp), value=p(value),
@@ -82,11 +90,7 @@ class FusedRecurrentPolicy:
     def __init__(self, policy, env, seed: int | None = None):
         lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
         F = int(env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0))
-        shape_ok = (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64
-                    and lin[1].in_features == 64 and lin[1].out_features == 64 and policy.cell == 64
-                    and policy.num_actions == 5 and policy.use_prev_action and policy.use_prev_reward
-                    and policy.lstm.input_size == 64 + 5 + 1 and policy.lstm.hidden_size == 64)
-        if not shape_ok:
+        if not FusedRecurrentPolicy.matches(policy, env):
             raise ValueError("the fused LSTM kernel implements the reference's policy only: trunk (64, 64) over "
                              f"F = V*V + 2 (+1) = {F} features, LSTM cell 64 with previous action and previous reward, "
                              "5 actions")
@@ -107,6 +111,18 @@ class FusedRecurrentPolicy:
         self.counter = 0
         self.refresh()
 
+    @staticmethod
+    def matches(policy, env) -> bool:
+        """Whether the fused kernel implements ``policy`` (a :class:`recurrent.RecurrentActionMaskPolicy`) at ``env``'s
+        feature width: trunk (64, 64) over F = V*V + 2 (+1 pressure) features, LSTM cell 64 fed with the previous
+        action and reward, 5 actions."""
+        F = env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0)
+        lin = [m for m in policy.trunk.modules() if isinstance(m, torch.nn.Linear)]
+        return (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64
+                and lin[1].in_features == 64 and lin[1].out_features == 64 and policy.cell == 64
+                and policy.num_actions == 5 and policy.use_prev_action and policy.use_prev_reward
+                and policy.lstm.input_size == 64 + 5 + 1 and policy.lstm.hidden_size == 64)
+
     def refresh(self):
         """Re-pack the module's current float32 parameters (bf16, padded; b_ih + b_hh summed) and upload them."""
         f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
@@ -119,17 +135,18 @@ class FusedRecurrentPolicy:
         self._dev.copy_(torch.from_numpy(self._host))
 
     def args(self, out_channels: dict, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *,
-             state_out=None, actions=None, actions64=None, logp=None, value=None, logits_out=None) -> nat.MapfLstmPolicyArgs:
+             state_out=None, actions=None, actions64=None, logp=None, value=None, logits_out=None,
+             greedy: bool = False) -> nat.MapfLstmPolicyArgs:
         """The argument block of one launch (counter 0; set ``.counter`` before launching).  ``out_channels`` maps
         local_obs / goal_delta / blocking_prev / action_mask to device tensors; every other tensor argument may be None
-        (``state_out=None``: the state is not advanced)."""
+        (``state_out=None``: the state is not advanced).  ``greedy``: first argmax of the masked logits, no draw."""
         env = self.env
         p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
         h, c = state
         ho, co = (None, None) if state_out is None else state_out
         return nat.MapfLstmPolicyArgs(
             num_envs=env.B, num_agents=env.N, v2=env.V * env.V, feature_dim=self.F,
-            no_masking=0, reserved=0, seed=self.seed, counter=0, env_id_base=int(env.cfg.env_id_base),
+            no_masking=0, greedy=int(bool(greedy)), seed=self.seed, counter=0, env_id_base=int(env.cfg.env_id_base),
             local_obs=p(out_channels["local_obs"]), goal_delta=p(out_channels["goal_delta"]),
             blocking_prev=p(out_channels["blocking_prev"]) if self.with_bp else None,
             action_mask=p(out_channels["action_mask"]), prev_terminated=p(prev_terminated),
@@ -139,14 +156,15 @@ class FusedRecurrentPolicy:
 
     def act(self, out, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *, advance: bool = True,
             state_out=None, logits_out: torch.Tensor | None = None, logp: torch.Tensor | None = None,
-            value: torch.Tensor | None = None, actions64: torch.Tensor | None = None):
+            value: torch.Tensor | None = None, actions64: torch.Tensor | None = None, greedy: bool = False):
         """One launch for the env's StepOutput ``out``.  ``state`` = (h, c) float32 [B*N, 64]; ``prev_action`` int8
         [B,N] (may be :attr:`actions` itself), ``prev_reward`` float32 [B,N]; ``prev_terminated`` / ``prev_truncated``
         uint8 [B] flag the envs whose episode starts at this step (their state, previous action and reward count as
         zero).  With ``advance`` the new state goes to ``state_out`` (default: ``state``, in place) and the draw to
         :attr:`actions`; without it (a bootstrap value) the state and :attr:`actions` -- the next step's previous
         actions -- are left as they are and the draw goes to ``actions64`` only.  Returns (actions int8 [B,N], logp,
-        value); ``logits_out`` [B,N,5] receives the masked logits."""
+        value); ``logits_out`` [B,N,5] receives the masked logits.  ``greedy``: the action is the first argmax of the
+        masked logits (RLlib's ``forward_inference``), every other output is what the draw mode writes."""
         for name, t, dt in (("h", state[0], torch.float32), ("c", state[1], torch.float32),
                             ("prev_action", prev_action, torch.int8), ("prev_reward", prev_reward, torch.float32)):
             if t.dtype != dt or not t.is_contiguous() or t.device != self.env.device:
@@ -159,7 +177,7 @@ class FusedRecurrentPolicy:
         a = self.args(ch, state, prev_action, prev_reward, prev_terminated, prev_truncated,
                       state_out=(state if state_out is None else state_out) if advance else None,
                       actions=self.actions if advance else None,
-                      actions64=actions64, logp=logp, value=value, logits_out=logits_out)
+                      actions64=actions64, logp=logp, value=value, logits_out=logits_out, greedy=greedy)
         self.counter += 1
         a.counter = self.counter
         nat.check(self._lib.mapf_lstm_policy_act(C.byref(a), self.env._stream()))

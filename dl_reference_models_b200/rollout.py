@@ -162,7 +162,7 @@ class FusedCollector:
             last = t == T
             return nat.MapfPolicyArgs(
                 num_envs=B, num_agents=N, v2=env.V * env.V, feature_dim=fused.F,
-                no_masking=int(bool(fused.policy.no_masking)), reserved=0, seed=fused.seed, counter=0,
+                no_masking=int(bool(fused.policy.no_masking)), greedy=0, seed=fused.seed, counter=0,
                 env_id_base=int(env.cfg.env_id_base), local_obs=src("local_obs", t), goal_delta=src("goal_delta", t),
                 blocking_prev=src("blocking_prev", t) if fused.with_bp else None, action_mask=src("action_mask", t),
                 weights=vp(fused._dev), actions=vp(fused.actions),

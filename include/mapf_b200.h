@@ -416,7 +416,9 @@ typedef struct mapf_policy_args {
     int32_t v2;           /* window cells, V * V */
     int32_t feature_dim;  /* F = v2 + 2 + (blocking_prev ? 1 : 0), <= 64: order of ENV:306-328 without the mask */
     int32_t no_masking;   /* action_mask_model.py:33 */
-    int32_t reserved;
+    int32_t greedy;       /* 0 = draw from softmax(masked logits) by inverse CDF (Philox); 1 = first index of the
+                             largest masked logit (torch.argmax, RLlib forward_inference), no Philox call.  Every other
+                             output is the same in both modes.  Other values: MAPF_ERR_INVALID_ARG */
     uint64_t seed;        /* Philox key (with env_id_base + env), counter = (counter, agent) */
     uint64_t counter;
     int64_t env_id_base;
@@ -425,9 +427,9 @@ typedef struct mapf_policy_args {
     const uint8_t *blocking_prev; /* [B,N] or NULL */
     const int8_t *action_mask;    /* [B,N,5] */
     const void *weights;          /* device copy of the block written by mapf_policy_pack_weights */
-    int8_t *actions;              /* [B,N] sampled action (feeds mapf_step), may be NULL */
+    int8_t *actions;              /* [B,N] chosen action (feeds mapf_step), may be NULL */
     int64_t *actions64;           /* [B,N] the same as int64 (torch indexing dtype), may be NULL */
-    float *logp;                  /* [B,N] log-probability of the sampled action */
+    float *logp;                  /* [B,N] log-probability of the chosen action */
     float *value;                 /* [B,N] value head */
     float *logits_out;            /* [B,N,5] masked logits, may be NULL */
     float *features_out;          /* [B,N,F] float32 feature block for the learner, may be NULL */
@@ -452,7 +454,9 @@ typedef struct mapf_lstm_policy_args {
     int32_t v2;           /* window cells, V * V */
     int32_t feature_dim;  /* F = v2 + 2 + (blocking_prev ? 1 : 0), <= 64: order of ENV:306-328 without the mask */
     int32_t no_masking;   /* action_mask_model.py:33 */
-    int32_t reserved;
+    int32_t greedy;       /* 0 = masked inverse-CDF draw (Philox); 1 = first index of the largest masked logit, no Philox
+                             call (h_out, c_out, value, logp and logits_out as in draw mode).  Other values:
+                             MAPF_ERR_INVALID_ARG */
     uint64_t seed;        /* Philox key (with env_id_base + env), counter = (counter, agent) */
     uint64_t counter;
     int64_t env_id_base;
@@ -469,9 +473,9 @@ typedef struct mapf_lstm_policy_args {
     float *h_out;                   /* [B*N,64] new state, may equal h_in / c_in; both NULL = do not advance the */
     float *c_out;                   /* [B*N,64]   state (h_in, c_in untouched); one NULL without the other is an error */
     const void *weights;            /* device copy of the block written by mapf_lstm_policy_pack_weights */
-    int8_t *actions;                /* [B,N] sampled action (feeds mapf_step), may be NULL */
+    int8_t *actions;                /* [B,N] chosen action (feeds mapf_step), may be NULL */
     int64_t *actions64;             /* [B,N] the same as int64, may be NULL */
-    float *logp;                    /* [B,N] log-probability of the sampled action, may be NULL */
+    float *logp;                    /* [B,N] log-probability of the chosen action, may be NULL */
     float *value;                   /* [B,N] value head, may be NULL */
     float *logits_out;              /* [B,N,5] masked logits, may be NULL */
 } mapf_lstm_policy_args;
@@ -485,6 +489,33 @@ int mapf_lstm_policy_pack_weights(int32_t feature_dim, const float *w1, const fl
                                   const float *w_logits, const float *b_logits, const float *w_value, const float *b_value,
                                   void *packed_host);
 int mapf_lstm_policy_act(const mapf_lstm_policy_args *args, void *stream);
+/* Per-step bookkeeping of the batched evaluator (main.py:test_trained_model, one episode per env, no auto-reset), in
+ * one launch after mapf_step (and after mapf_occupancy_accumulate, which reads `active` before this call clears it).
+ * For every env with active[b] != 0: episode_reward[b] += sum of the agents' rewards (main.py:251), agent_reward[b,n]
+ * += reward[b,n] (main.py:262), timesteps[b] += 1, last_info[b,:] = info[b,:]; if terminated[b] | truncated[b] the
+ * episode ends: success[b] = terminated[b] && !truncated[b] (main.py:294) and active[b] = 0.  Inactive envs are not
+ * touched.  The envs still active after the call are counted into active_count[step & 1], which must be zero on entry;
+ * the call zeroes active_count[(step & 1) ^ 1] for the next call, so a loop that passes step = 0, 1, 2, ... starting
+ * from two zero words needs no memset between steps and reads one word per step.  Every pointer is a device pointer
+ * and is required. */
+typedef struct mapf_eval_args {
+    int32_t num_envs, num_agents;
+    int64_t step;               /* selects the counter word, see above */
+    const float *reward;        /* [B,N] this step's rewards */
+    const uint8_t *terminated;  /* [B] */
+    const uint8_t *truncated;   /* [B] */
+    const int32_t *info;        /* [B,16] */
+    uint8_t *active;            /* [B] 1 while the env's first episode runs; cleared by this call at its end */
+    double *episode_reward;     /* [B] */
+    double *agent_reward;       /* [B,N] */
+    int64_t *timesteps;         /* [B] */
+    uint8_t *success;           /* [B] */
+    int32_t *last_info;         /* [B,16] info of the env's last active step */
+    uint32_t *active_count;     /* [2] envs still active after this step, in word step & 1 */
+} mapf_eval_args;
+
+int mapf_eval_accumulate(const mapf_eval_args *args, void *stream);
+
 /* rewards / values / adv / ret: device float32 [T,B,N]; dones uint8 [T,B]; last_value float32 [B,N]. */
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
              float *ret, int32_t T, int64_t B, int32_t N, float gamma, float lam, void *stream);
