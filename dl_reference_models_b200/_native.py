@@ -225,6 +225,8 @@ def lib():
     L.mapf_lstm_policy_weights_nbytes.restype = i64
     L.mapf_lstm_policy_pack_weights.argtypes = [i32] + [vp] * 13
     L.mapf_lstm_policy_act.argtypes = [C.POINTER(MapfLstmPolicyArgs), vp]
+    L.mapf_policy_act_per_agent.argtypes = [C.POINTER(MapfPolicyArgs), vp]
+    L.mapf_lstm_policy_act_per_agent.argtypes = [C.POINTER(MapfLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
     L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
@@ -248,6 +250,7 @@ EXPORTS = (
     "mapf_step_kernel_kind", "mapf_cte_step", "mapf_cte_reset", "mapf_occupancy_accumulate", "mapf_distance_table", "mapf_goal_path_lengths",
     "mapf_policy_weights_nbytes", "mapf_policy_pack_weights", "mapf_policy_act", "mapf_gae",
     "mapf_lstm_policy_weights_nbytes", "mapf_lstm_policy_pack_weights", "mapf_lstm_policy_act", "mapf_eval_accumulate",
+    "mapf_policy_act_per_agent", "mapf_lstm_policy_act_per_agent",
 )
 
 

@@ -1635,7 +1635,7 @@ int mapf_policy_pack_weights(int32_t F, const float *w1, const float *b1, const 
     return MAPF_OK;
 }
 
-int mapf_policy_act(const mapf_policy_args *a, void *stream) {
+static int policy_launch(const mapf_policy_args *a, bool per_agent, void *stream) {
     if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
     const int kc1 = policy_kc1(a->feature_dim);
     if (!kc1 || a->v2 < 1 || a->feature_dim != a->v2 + 2 + (a->blocking_prev ? 1 : 0))
@@ -1644,24 +1644,33 @@ int mapf_policy_act(const mapf_policy_args *a, void *stream) {
     if (a->num_envs < 1 || a->num_agents < 1 || !a->local_obs || !a->goal_delta || !a->weights)
         return fail(MAPF_ERR_INVALID_ARG, "policy: env outputs and weights are required");
     if (a->greedy != 0 && a->greedy != 1) return fail(MAPF_ERR_INVALID_ARG, "policy: greedy %d is neither 0 nor 1", a->greedy);
+    if (per_agent && a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "policy: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
     const int threads = 256, warps = threads / 32;
     const size_t smem = (size_t)mapf_policy_weights_nbytes(a->feature_dim) + (size_t)warps * mapf::pol_warp_bytes(kc1, a->v2);
-    const long long tiles = ((long long)a->num_envs * a->num_agents + 31) / 32;
+    // a per-agent tile holds one agent's rows: ceil(B / 32) tiles per agent
+    const long long tiles = per_agent ? ((long long)a->num_envs + 31) / 32 * a->num_agents
+                                      : ((long long)a->num_envs * a->num_agents + 31) / 32;
     long long blocks = (tiles + warps - 1) / warps;
     if (blocks > 148 * 8) blocks = 148 * 8;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    void (*const kernels[2][2])(const mapf_policy_args) = {
-        {mapf::mapf_policy_act_kernel<2, false>, mapf::mapf_policy_act_kernel<2, true>},
-        {mapf::mapf_policy_act_kernel<4, false>, mapf::mapf_policy_act_kernel<4, true>}};
-    const auto kernel = kernels[kc1 == 4][a->greedy];
+    void (*const kernels[2][2][2])(const mapf_policy_args) = {
+        {{mapf::mapf_policy_act_kernel<2, false>, mapf::mapf_policy_act_kernel<2, true>},
+         {mapf::mapf_policy_act_kernel<4, false>, mapf::mapf_policy_act_kernel<4, true>}},
+        {{mapf::mapf_policy_act_kernel<2, false, true>, mapf::mapf_policy_act_kernel<2, true, true>},
+         {mapf::mapf_policy_act_kernel<4, false, true>, mapf::mapf_policy_act_kernel<4, true, true>}}};
+    const auto kernel = kernels[per_agent][kc1 == 4][a->greedy];
     CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kernel<<<(unsigned)blocks, threads, smem, st>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }
+
+int mapf_policy_act(const mapf_policy_args *a, void *stream) { return policy_launch(a, false, stream); }
+int mapf_policy_act_per_agent(const mapf_policy_args *a, void *stream) { return policy_launch(a, true, stream); }
 
 int64_t mapf_lstm_policy_weights_nbytes(int32_t F) {
     const int kc1 = policy_kc1(F);
@@ -1700,7 +1709,7 @@ int mapf_lstm_policy_pack_weights(int32_t F, const float *w1, const float *b1, c
     return MAPF_OK;
 }
 
-int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
+static int lstm_policy_launch(const mapf_lstm_policy_args *a, bool per_agent, void *stream) {
     if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
     const int kc1 = policy_kc1(a->feature_dim);
     if (!kc1 || a->v2 < 1 || a->feature_dim != a->v2 + 2 + (a->blocking_prev ? 1 : 0))
@@ -1714,6 +1723,8 @@ int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
         return fail(MAPF_ERR_INVALID_ARG, "lstm policy: h_out and c_out are given together (both NULL = state not advanced)");
     if (a->greedy != 0 && a->greedy != 1)
         return fail(MAPF_ERR_INVALID_ARG, "lstm policy: greedy %d is neither 0 nor 1", a->greedy);
+    if (per_agent && a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "lstm policy: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
     int ndev = 0, dev = 0, sms = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
@@ -1721,19 +1732,27 @@ int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) {
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int threads = mapf::LSTM_THREADS, warps = threads / 32;
     const size_t smem = (size_t)mapf::lstm_weight_bytes(kc1) + (size_t)warps * mapf::pol_warp_bytes(kc1, a->v2);
-    const long long tiles = ((long long)a->num_envs * a->num_agents + 31) / 32;
+    const long long tiles = per_agent ? ((long long)a->num_envs + 31) / 32 * a->num_agents
+                                      : ((long long)a->num_envs * a->num_agents + 31) / 32;
     long long blocks = (tiles + warps - 1) / warps;
-    if (blocks > sms) blocks = sms;   // one resident block per SM loads the weights once and loops over the tiles
+    // one resident block per SM loads the weights once (per agent: once per agent of its tile range) and loops over
+    // the tiles
+    if (blocks > sms) blocks = sms;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    void (*const kernels[2][2])(const mapf_lstm_policy_args) = {
-        {mapf::mapf_lstm_policy_act_kernel<2, false>, mapf::mapf_lstm_policy_act_kernel<2, true>},
-        {mapf::mapf_lstm_policy_act_kernel<4, false>, mapf::mapf_lstm_policy_act_kernel<4, true>}};
-    const auto kernel = kernels[kc1 == 4][a->greedy];
+    void (*const kernels[2][2][2])(const mapf_lstm_policy_args) = {
+        {{mapf::mapf_lstm_policy_act_kernel<2, false>, mapf::mapf_lstm_policy_act_kernel<2, true>},
+         {mapf::mapf_lstm_policy_act_kernel<4, false>, mapf::mapf_lstm_policy_act_kernel<4, true>}},
+        {{mapf::mapf_lstm_policy_act_kernel<2, false, true>, mapf::mapf_lstm_policy_act_kernel<2, true, true>},
+         {mapf::mapf_lstm_policy_act_kernel<4, false, true>, mapf::mapf_lstm_policy_act_kernel<4, true, true>}}};
+    const auto kernel = kernels[per_agent][kc1 == 4][a->greedy];
     CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kernel<<<(unsigned)blocks, threads, smem, st>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }
+
+int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) { return lstm_policy_launch(a, false, stream); }
+int mapf_lstm_policy_act_per_agent(const mapf_lstm_policy_args *a, void *stream) { return lstm_policy_launch(a, true, stream); }
 
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
              float *ret, int32_t T, int64_t B, int32_t N, float gamma, float lam, void *stream) {

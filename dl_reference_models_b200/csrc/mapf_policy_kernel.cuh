@@ -13,6 +13,8 @@
 //     does a stable softmax and draws by inverse CDF from one Philox word (keyed by the global env id).
 // The op is tiny-tile GEMM work bounded by its ~50 B of HBM traffic per agent, not by tensor throughput, which
 // is why the legacy mma.sync path is enough here (no TMA / TMEM pipeline to amortise at K <= 64).
+// With PER_AGENT (mapf_policy_act_per_agent) every agent has its own weight block: a tile is 32 envs of one agent
+// (rows N apart, pol_row), and a CTA reloads the block in shared memory when its agent changes (pol_per_agent_tiles).
 //
 // mapf_gae_kernel: generalised advantage estimation as a backwards scan, one thread per (env, agent) series.
 #pragma once
@@ -68,10 +70,70 @@ __device__ __forceinline__ void pol_load_tile(const uint8_t *local_obs, const in
     }
 }
 
+// Per-agent policies (mapf_policy_act_per_agent, mapf_lstm_policy_act_per_agent): a tile is (agent j, envs e0 ..
+// e0 + 31) and its row r is the flat row (e0 + r) N + j, i.e. ag0 + r N with ag0 = e0 N + j; a shared-policy tile is
+// 32 consecutive rows ag0 + r.  Every per-row access of the kernels goes through pol_row.
+template <bool PER_AGENT>
+__device__ __forceinline__ long long pol_row(long long ag0, int r, int N) {
+    if constexpr (PER_AGENT) return ag0 + (long long)r * N;
+    else return ag0 + r;
+}
+
+// pol_load_tile for a per-agent tile: the window rows are N * V2 bytes apart, gathered into the same raw layout (row r
+// at r * V2, zero beyond the tile's na rows and in the slack words), the mask rows into rawm (+ the optional copy)
+__device__ __forceinline__ void pol_gather_tile(const uint8_t *local_obs, const int8_t *action_mask, int8_t *action_mask_out,
+                                                int V2, long long ag0, int N, int na, uint32_t *raw, uint32_t *rawm, int lane) {
+    uint8_t *rb = reinterpret_cast<uint8_t *>(raw);
+    for (int i = lane; i < ((32 * V2 + 3) / 4 + 2) * 4; i += 32) {
+        const int r = i / V2;
+        rb[i] = r < na ? local_obs[pol_row<true>(ag0, r, N) * V2 + (i - r * V2)] : 0;
+    }
+    if (action_mask) {
+        uint8_t *mb = reinterpret_cast<uint8_t *>(rawm);
+        for (int i = lane; i < 160; i += 32) {
+            const int r = i / 5;
+            int8_t v = 0;
+            if (r < na) {
+                const long long m = pol_row<true>(ag0, r, N) * 5 + (i - r * 5);
+                v = action_mask[m];
+                if (action_mask_out) action_mask_out[m] = v;
+            }
+            mb[i] = (uint8_t)v;
+        }
+    }
+}
+
+// The tile loop of the per-agent kernels.  Tiles are ordered agent-major (tile k: agent k / tpa, envs 32 (k % tpa) ..,
+// tpa = ceil(B / 32)) and each CTA takes one contiguous range of that order (the ranges of the G CTAs differ in length
+// by at most one tile), so it meets only a few agent changes.  The range is walked in rounds of at most one tile per warp that never cross an agent boundary; at each
+// change of agent the CTA reloads that agent's weight block into shared memory between two barriers (load(j)), so all
+// warps use one block between two barriers.  body(ag0, na) runs one tile: rows pol_row<true>(ag0, r, N), r < na.
+template <class Load, class Body>
+__device__ __forceinline__ void pol_per_agent_tiles(int B, int N, int warp, int warps, Load load, Body body) {
+    const int tpa = (B + 31) >> 5, ntiles = tpa * N;   // B * N < 2^31, as in pol_sample
+    const int G = gridDim.x, b = blockIdx.x, q = ntiles / G, rm = ntiles % G;
+    int k = b * q + (b < rm ? b : rm);
+    const int k1 = k + q + (b < rm ? 1 : 0);
+    for (int j = k / tpa; k < k1; ++j) {
+        __syncthreads();   // every warp is done with the previous agent's block
+        load(j);
+        __syncthreads();
+        const int kend = k1 < (j + 1) * tpa ? k1 : (j + 1) * tpa;
+        for (; k < kend; k += warps) {
+            if (k + warp < kend) {
+                const int e0 = (k + warp - j * tpa) << 5;
+                body((long long)e0 * N + j, B - e0 < 32 ? B - e0 : 32);
+            }
+        }
+        k = kend;
+    }
+}
+
 // bf16 feature row of agent `lane` (ENV:306-328 order: window, goal delta, pressure) into xs[lane][0 .. 16 KC1)
-template <int KC1>
+template <int KC1, bool PER_AGENT = false>
 __device__ __forceinline__ void pol_feature_row(__nv_bfloat16 *xs, const uint32_t *raw, const float *goal_delta,
-                                                const uint8_t *blocking_prev, int V2, long long ag0, int na, int lane) {
+                                                const uint8_t *blocking_prev, int V2, long long ag0, int na, int lane,
+                                                int N = 1) {
     constexpr int S1 = 16 * KC1 + 8;
     const int NW = (V2 + 3) >> 2;   // words of one agent's window
     uint2 *row = reinterpret_cast<uint2 *>(xs + lane * S1);
@@ -88,10 +150,10 @@ __device__ __forceinline__ void pol_feature_row(__nv_bfloat16 *xs, const uint32_
         row[j] = make_uint2(*reinterpret_cast<const uint32_t *>(&lo), *reinterpret_cast<const uint32_t *>(&hi));
     }
     if (lane < na) {
-        const float2 gd = reinterpret_cast<const float2 *>(goal_delta)[ag0 + lane];
+        const float2 gd = reinterpret_cast<const float2 *>(goal_delta)[pol_row<PER_AGENT>(ag0, lane, N)];
         xs[lane * S1 + V2] = __float2bfloat16(gd.x);
         xs[lane * S1 + V2 + 1] = __float2bfloat16(gd.y);
-        if (blocking_prev) xs[lane * S1 + V2 + 2] = __float2bfloat16((float)blocking_prev[ag0 + lane]);
+        if (blocking_prev) xs[lane * S1 + V2 + 2] = __float2bfloat16((float)blocking_prev[pol_row<PER_AGENT>(ag0, lane, N)]);
     }
 }
 
@@ -198,8 +260,9 @@ __device__ __forceinline__ void pol_sample(const Args &a, const float *os, const
     }
 }
 
-// KC1 = k16 chunks of the first layer (F <= 16 * KC1), W1 row stride = 16 * KC1 + 8; GREEDY = a.greedy (argmax, no draw)
-template <int KC1, bool GREEDY>
+// KC1 = k16 chunks of the first layer (F <= 16 * KC1), W1 row stride = 16 * KC1 + 8; GREEDY = a.greedy (argmax, no draw);
+// PER_AGENT: a.weights holds num_agents consecutive blocks and tile rows are one agent's (pol_per_agent_tiles)
+template <int KC1, bool GREEDY, bool PER_AGENT = false>
 __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_args a) {
     constexpr int S1 = 16 * KC1 + 8;   // bf16 row stride of the feature tile and of W1
     extern __shared__ __align__(16) unsigned char psm[];
@@ -209,13 +272,13 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
     float *bias = reinterpret_cast<float *>(w3 + 8 * POL_W2_STRIDE);            // b1[64] b2[64] b3[8]
     unsigned char *wsm0 = reinterpret_cast<unsigned char *>(bias + 2 * POL_H + 8);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, warps = blockDim.x >> 5;
-    {   // weights: already bf16 and padded on the host side (mapf_policy_pack_weights)
+    if constexpr (!PER_AGENT) {   // weights: already bf16 and padded on the host side (mapf_policy_pack_weights)
         const uint4 *src = reinterpret_cast<const uint4 *>(a.weights);
         uint4 *dst = reinterpret_cast<uint4 *>(psm);
         const int n16 = (int)((wsm0 - psm) >> 4);
         for (int i = tid; i < n16; i += blockDim.x) dst[i] = src[i];
+        __syncthreads();
     }
-    __syncthreads();
     const int V2 = a.v2, F = a.feature_dim, N = a.num_agents;
     unsigned char *wsm = wsm0 + warp * pol_warp_bytes(KC1, V2);
     __nv_bfloat16 *xs = reinterpret_cast<__nv_bfloat16 *>(wsm);                 // [32][S1] bf16 features
@@ -223,15 +286,11 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
     uint32_t *rawm = reinterpret_cast<uint32_t *>(wsm + 32 * S1 * 2 + pol_raw_bytes(V2));   // 32 x 5 mask bytes
     float *os = reinterpret_cast<float *>(wsm + 32 * S1 * 2 + pol_raw_bytes(V2) + 160);     // [32][8] head outputs
     const int g = lane >> 2, t = lane & 3;
-    const long long BN = (long long)a.num_envs * N;
-    const long long ntiles = (BN + 31) >> 5;
-    for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
-        const long long ag0 = tile << 5;
-        const long long left = BN - ag0;
-        const int na = left < 32 ? (int)left : 32;
-        pol_load_tile(a.local_obs, a.action_mask, a.action_mask_out, V2, ag0, na, raw, rawm, lane);
+    auto tile_body = [&](const long long ag0, const int na) {
+        if constexpr (PER_AGENT) pol_gather_tile(a.local_obs, a.action_mask, a.action_mask_out, V2, ag0, N, na, raw, rawm, lane);
+        else pol_load_tile(a.local_obs, a.action_mask, a.action_mask_out, V2, ag0, na, raw, rawm, lane);
         __syncwarp();
-        pol_feature_row<KC1>(xs, raw, a.goal_delta, a.blocking_prev, V2, ag0, na, lane);
+        pol_feature_row<KC1, PER_AGENT>(xs, raw, a.goal_delta, a.blocking_prev, V2, ag0, na, lane, N);
         if (a.features_out) {   // float32 feature block for the learner (optional)
             float *fo = a.features_out + ag0 * F;
             const uint8_t *rb = reinterpret_cast<const uint8_t *>(raw);
@@ -239,9 +298,10 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
                 const int r = i / F, c = i - r * F;
                 float v;
                 if (c < V2) v = (float)rb[r * V2 + c];
-                else if (c < V2 + 2) v = a.goal_delta[(ag0 + r) * 2 + (c - V2)];
-                else v = (float)a.blocking_prev[ag0 + r];
-                fo[i] = v;
+                else if (c < V2 + 2) v = a.goal_delta[pol_row<PER_AGENT>(ag0, r, N) * 2 + (c - V2)];
+                else v = (float)a.blocking_prev[pol_row<PER_AGENT>(ag0, r, N)];
+                if constexpr (PER_AGENT) a.features_out[pol_row<true>(ag0, r, N) * F + c] = v;
+                else fo[i] = v;
             }
         }
         __syncwarp();
@@ -253,8 +313,24 @@ __global__ void __launch_bounds__(256) mapf_policy_act_kernel(const mapf_policy_
             pol_heads(h2, w3, bias + 2 * POL_H, os, row0, g, t);
         }
         __syncwarp();
-        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, ag0 + lane, N, 0x504F4C49ull /* "POLI" */);
+        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, pol_row<PER_AGENT>(ag0, lane, N), N, 0x504F4C49ull /* "POLI" */);
         __syncwarp();
+    };
+    if constexpr (PER_AGENT) {
+        const int n16 = (int)((wsm0 - psm) >> 4);   // 16-byte words of one agent's block
+        pol_per_agent_tiles(a.num_envs, N, warp, warps, [&](int j) {
+            const uint4 *src = reinterpret_cast<const uint4 *>(a.weights) + (long long)j * n16;
+            uint4 *dst = reinterpret_cast<uint4 *>(psm);
+            for (int i = tid; i < n16; i += blockDim.x) dst[i] = src[i];
+        }, tile_body);
+    } else {
+        const long long BN = (long long)a.num_envs * N;
+        const long long ntiles = (BN + 31) >> 5;
+        for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
+            const long long ag0 = tile << 5;
+            const long long left = BN - ag0;
+            tile_body(ag0, left < 32 ? (int)left : 32);
+        }
     }
 }
 

@@ -52,8 +52,9 @@ __device__ __forceinline__ void lstm_gate_chunk(float (&d)[4][4], const uint32_t
 }
 
 // GREEDY = a.greedy: argmax instead of the draw, in the epilogue only, where the gate fragments are dead (see
-// pol_sample for why it is a template parameter)
-template <int KC1, bool GREEDY>
+// pol_sample for why it is a template parameter); PER_AGENT: a.weights holds num_agents consecutive blocks and tile
+// rows are one agent's (pol_per_agent_tiles)
+template <int KC1, bool GREEDY, bool PER_AGENT = false>
 __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(const mapf_lstm_policy_args a) {
     constexpr int S1 = 16 * KC1 + 8;
     extern __shared__ __align__(16) unsigned char psm[];
@@ -65,12 +66,12 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
     const float *bg = bias + 2 * POL_H + 8;
     unsigned char *wsm0 = psm + lstm_weight_bytes(KC1);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, warps = blockDim.x >> 5;
-    {   // weights: already bf16 and padded on the host side (mapf_lstm_policy_pack_weights)
+    if constexpr (!PER_AGENT) {   // weights: already bf16 and padded on the host side (mapf_lstm_policy_pack_weights)
         const uint4 *src = reinterpret_cast<const uint4 *>(a.weights);
         uint4 *dst = reinterpret_cast<uint4 *>(psm);
         for (int i = tid; i < lstm_weight_bytes(KC1) / 16; i += blockDim.x) dst[i] = src[i];
+        __syncthreads();
     }
-    __syncthreads();
     const int V2 = a.v2, N = a.num_agents;
     unsigned char *wsm = wsm0 + warp * pol_warp_bytes(KC1, V2);
     __nv_bfloat16 *xs = reinterpret_cast<__nv_bfloat16 *>(wsm);                 // [32][S1] bf16 features
@@ -78,15 +79,11 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
     uint32_t *rawm = reinterpret_cast<uint32_t *>(wsm + 32 * S1 * 2 + pol_raw_bytes(V2));
     float *os = reinterpret_cast<float *>(wsm + 32 * S1 * 2 + pol_raw_bytes(V2) + 160);     // [32][8] head outputs
     const int g = lane >> 2, t = lane & 3;
-    const long long BN = (long long)a.num_envs * N;
-    const long long ntiles = (BN + 31) >> 5;
-    for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
-        const long long ag0 = tile << 5;
-        const long long left = BN - ag0;
-        const int na = left < 32 ? (int)left : 32;
-        pol_load_tile(a.local_obs, a.action_mask, nullptr, V2, ag0, na, raw, rawm, lane);
+    auto tile_body = [&](const long long ag0, const int na) {
+        if constexpr (PER_AGENT) pol_gather_tile(a.local_obs, a.action_mask, nullptr, V2, ag0, N, na, raw, rawm, lane);
+        else pol_load_tile(a.local_obs, a.action_mask, nullptr, V2, ag0, na, raw, rawm, lane);
         __syncwarp();
-        pol_feature_row<KC1>(xs, raw, a.goal_delta, a.blocking_prev, V2, ag0, na, lane);
+        pol_feature_row<KC1, PER_AGENT>(xs, raw, a.goal_delta, a.blocking_prev, V2, ag0, na, lane, N);
         __syncwarp();
 #pragma unroll 1
         for (int mt = 0; mt < 2; ++mt) {
@@ -101,7 +98,7 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
 #pragma unroll
             for (int r = 0; r < 2; ++r) {
                 const int row = row0 + 8 * r;
-                agr[r] = ag0 + row;
+                agr[r] = pol_row<PER_AGENT>(ag0, row, N);
                 const bool valid = row < na;
                 bool start = false;
                 int pa = 0;
@@ -163,7 +160,7 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
                 if (a.h_out) {   // h_out and c_out are given together
 #pragma unroll
                     for (int r = 0; r < 2; ++r) {
-                        if (agr[r] - ag0 < na) {
+                        if (PER_AGENT ? row0 + 8 * r < na : agr[r] - ag0 < na) {
                             *reinterpret_cast<float2 *>(a.c_out + agr[r] * POL_H + col) = make_float2(cn[2 * r], cn[2 * r + 1]);
                             *reinterpret_cast<float2 *>(a.h_out + agr[r] * POL_H + col) = make_float2(hv[2 * r], hv[2 * r + 1]);
                         }
@@ -175,8 +172,24 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) mapf_lstm_policy_act_kernel(c
             pol_heads(hn, w3, bias + 2 * POL_H, os, row0, g, t);
         }
         __syncwarp();
-        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, ag0 + lane, N, 0x4C53544Dull /* "LSTM" */);
+        if (lane < na) pol_sample<GREEDY>(a, os, rawm, lane, pol_row<PER_AGENT>(ag0, lane, N), N, 0x4C53544Dull /* "LSTM" */);
         __syncwarp();
+    };
+    if constexpr (PER_AGENT) {
+        pol_per_agent_tiles(a.num_envs, N, warp, warps, [&](int j) {
+            const uint4 *src = reinterpret_cast<const uint4 *>(static_cast<const unsigned char *>(a.weights) +
+                                                               (long long)j * lstm_weight_bytes(KC1));
+            uint4 *dst = reinterpret_cast<uint4 *>(psm);
+            for (int i = tid; i < lstm_weight_bytes(KC1) / 16; i += blockDim.x) dst[i] = src[i];
+        }, tile_body);
+    } else {
+        const long long BN = (long long)a.num_envs * N;
+        const long long ntiles = (BN + 31) >> 5;
+        for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
+            const long long ag0 = tile << 5;
+            const long long left = BN - ag0;
+            tile_body(ag0, left < 32 ? (int)left : 32);
+        }
     }
 }
 

@@ -11,7 +11,8 @@ reference's ``ALGO_NAME == "RANDOM"`` branch: uniform actions, main.py:212-214),
 mask), any callable ``policy(env, out) -> int8 [B,N]``, or a trained :class:`rollout.ActionMaskPolicy` /
 :class:`recurrent.RecurrentActionMaskPolicy` played like ``rl_module.forward_inference`` (main.py:209-223): argmax of the
 masked logits, the LSTM state, previous action and previous reward carried from step to step.  Modules of the
-reference's shape run as one fused kernel launch per step (``mapf_policy_act`` / ``mapf_lstm_policy_act`` in greedy
+reference's shape (and the per-agent variants :class:`rollout.PerAgentActionMaskPolicy` /
+:class:`recurrent.PerAgentRecurrentPolicy`, one module per agent, of that shape) run as one fused kernel launch per step (``mapf_policy_act`` / ``mapf_lstm_policy_act`` in greedy
 mode), any other shape through its PyTorch forward.
 
 ``python -m dl_reference_models_b200.evaluate`` times the evaluator (:func:`benchmark`).
@@ -28,7 +29,10 @@ from . import _native as nat
 from . import rollout
 from .batched_env import BatchedMapfEnv
 from .policy_kernels import FusedPolicy, FusedRecurrentPolicy
-from .recurrent import RecurrentActionMaskPolicy
+from .recurrent import PerAgentRecurrentPolicy, RecurrentActionMaskPolicy
+
+MODULE_TYPES = (rollout.ActionMaskPolicy, RecurrentActionMaskPolicy, rollout.PerAgentActionMaskPolicy, PerAgentRecurrentPolicy)
+RECURRENT_TYPES = (RecurrentActionMaskPolicy, PerAgentRecurrentPolicy)
 
 
 @dataclass
@@ -51,6 +55,8 @@ class EvalResult:
 
 
 def _module_in_features(policy) -> int:
+    if isinstance(policy, (rollout.PerAgentActionMaskPolicy, PerAgentRecurrentPolicy)):
+        return int(policy.feature_dim)
     lin = [m for m in policy.trunk.modules() if isinstance(m, torch.nn.Linear)]
     if lin:
         return int(lin[0].in_features)
@@ -71,8 +77,11 @@ def _module_actor(env, policy, explore: bool):
     wrong = {str(p.device) for p in policy.parameters() if p.device != env.device}
     if wrong:
         raise ValueError(f"the policy's parameters are on {sorted(wrong)}, the evaluation runs on {env.device}")
+    if isinstance(policy, (rollout.PerAgentActionMaskPolicy, PerAgentRecurrentPolicy)) and policy.num_agents != env.N:
+        raise ValueError(f"the per-agent policy has num_agents = {policy.num_agents} modules, the env has "
+                         f"num_agents = {env.N} agents")
     B, N, dev = env.B, env.N, env.device
-    recurrent = isinstance(policy, RecurrentActionMaskPolicy)
+    recurrent = isinstance(policy, RECURRENT_TYPES)
     if recurrent and FusedRecurrentPolicy.matches(policy, env):
         fused = FusedRecurrentPolicy(policy, env)
         state = (torch.zeros((B * N, 64), device=dev), torch.zeros((B * N, 64), device=dev))
@@ -93,7 +102,7 @@ def _torch_actor(env, policy, explore: bool):
     """The module's own forward (any shape), with the same carry as the fused path."""
     B, N, dev = env.B, env.N, env.device
     M = B * N
-    recurrent = isinstance(policy, RecurrentActionMaskPolicy)
+    recurrent = isinstance(policy, RECURRENT_TYPES)
     carry = {}
     if recurrent:
         carry.update(state=policy.initial_state(M, dev), prev_action=torch.zeros(M, dtype=torch.int64, device=dev),
@@ -123,7 +132,7 @@ def _play(env, policy="random", max_steps: int | None = None, explore: bool = Fa
     B, N = env.B, env.N
     dev = env.device
     out = env.reset()
-    if isinstance(policy, (rollout.ActionMaskPolicy, RecurrentActionMaskPolicy)):
+    if isinstance(policy, MODULE_TYPES):
         module_act = _module_actor(env, policy, explore)
         policy = lambda env, out: module_act(out)  # noqa: E731
     z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
@@ -164,7 +173,8 @@ def evaluate(env_config: dict, num_episodes: int, policy="random", device="cuda:
              explore: bool = False) -> EvalResult:
     """Play ``num_episodes`` episodes, one per env of a batch.  ``policy``: ``"random"``, ``"masked"``, a callable
     ``policy(env, out) -> int8 [B,N]``, or a trained :class:`rollout.ActionMaskPolicy` /
-    :class:`recurrent.RecurrentActionMaskPolicy` on ``device``, played as the reference's ``forward_inference`` (argmax
+    :class:`recurrent.RecurrentActionMaskPolicy` / :class:`rollout.PerAgentActionMaskPolicy` /
+    :class:`recurrent.PerAgentRecurrentPolicy` (``num_agents`` = the env's) on ``device``, played as the reference's ``forward_inference`` (argmax
     of the masked logits; ``explore=True``: a draw from them)."""
     env = BatchedMapfEnv(env_config, num_episodes, device)
     acc = _play(env, policy, max_steps, explore)

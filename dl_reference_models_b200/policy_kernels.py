@@ -1,6 +1,7 @@
 """Rollout-loop CUDA kernels around the env step (BASELINE config 5): the action-mask MLP evaluated straight from the
 env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tensor-core MLP with f32 accumulation), the
-same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a greedy (argmax) mode for evaluation, and GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
+same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a greedy (argmax) mode for evaluation and a
+per-agent variant (one weight set per agent: ``mapf_policy_act_per_agent`` / ``mapf_lstm_policy_act_per_agent``), and GAE as a backwards scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
 
@@ -12,9 +13,28 @@ import torch
 from . import _native as nat
 
 
+def _per_agent_kind(policy) -> str | None:
+    """"mlp" for a :class:`rollout.PerAgentActionMaskPolicy`, "lstm" for a :class:`recurrent.PerAgentRecurrentPolicy`,
+    None for any other module."""
+    from .recurrent import PerAgentRecurrentPolicy
+    from .rollout import PerAgentActionMaskPolicy
+
+    return "mlp" if isinstance(policy, PerAgentActionMaskPolicy) else "lstm" if isinstance(policy, PerAgentRecurrentPolicy) else None
+
+
+def _per_agent_arrays(policy, names):
+    """float32 numpy copies of a per-agent module's stacked parameters ``names``, then per agent j the list of their
+    [j] slices (the pack function's arguments for agent j)."""
+    f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
+    stacked = [f(getattr(policy, n)) if isinstance(n, str) else f(n) for n in names]
+    return [[np.ascontiguousarray(a[j]) for a in stacked] for j in range(policy.num_agents)]
+
+
 class FusedPolicy:
-    """Inference view of an :class:`rollout.ActionMaskPolicy` (two 64-wide ReLU layers, 5 logits + value): call
-    :meth:`refresh` after every optimizer step, :meth:`act` once per env step."""
+    """Inference view of an :class:`rollout.ActionMaskPolicy` (two 64-wide ReLU layers, 5 logits + value), or of a
+    :class:`rollout.PerAgentActionMaskPolicy` of that shape with one module per env agent (launched through
+    ``mapf_policy_act_per_agent``, :attr:`entry`): call :meth:`refresh` after every optimizer step, :meth:`act` once
+    per env step."""
 
     def __init__(self, policy, env, seed: int | None = None):
         self.policy, self.env = policy, env
@@ -22,11 +42,23 @@ class FusedPolicy:
         self.F = int(env.flat_obs_dim(include_action_mask=False))
         self.with_bp = bool(env.include_blocking_pressure)
         assert self.F == env.V * env.V + 2 + (1 if self.with_bp else 0)
-        assert FusedPolicy.matches(policy, env), "the fused kernel implements the reference's 64-64 action-mask MLP"
-        self._lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
+        self.per_agent = _per_agent_kind(policy) is not None
+        if self.per_agent:
+            if not FusedPolicy.matches(policy, env):
+                raise ValueError("the fused kernel implements the reference's 64-64 action-mask MLP only, one module per "
+                                 f"env agent: the policy has {policy.num_agents} agents of feature_dim "
+                                 f"{policy.feature_dim}, hiddens {policy.hiddens}, {policy.num_actions} actions; the env "
+                                 f"has {env.N} agents and {self.F} features")
+        else:
+            assert FusedPolicy.matches(policy, env), "the fused kernel implements the reference's 64-64 action-mask MLP"
+            self._lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
+        self.entry = "mapf_policy_act_per_agent" if self.per_agent else "mapf_policy_act"
+        self._act = getattr(self._lib, self.entry)
         n = int(self._lib.mapf_policy_weights_nbytes(self.F))
         if n < 0:
             raise nat.MapfError(n, self._lib.mapf_last_error().decode())
+        self._block = n
+        n *= policy.num_agents if self.per_agent else 1   # per agent: block j at j * n
         self._host = np.zeros(n, np.uint8)
         self._dev = torch.zeros(n, dtype=torch.uint8, device=env.device)
         B, N = env.B, env.N
@@ -44,17 +76,29 @@ class FusedPolicy:
         """Whether the fused kernel implements ``policy`` (an :class:`rollout.ActionMaskPolicy`) at ``env``'s feature
         width: trunk Linear(F, 64)-ReLU-Linear(64, 64)-ReLU over F = V*V + 2 (+1 pressure) features, 5 logits."""
         F = env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0)
+        kind = _per_agent_kind(policy)
+        if kind is not None:   # a rollout.PerAgentActionMaskPolicy: every agent's module has the reference's shape
+            return (kind == "mlp" and policy.num_agents == env.N and policy.feature_dim == F and tuple(policy.hiddens) == (64, 64)
+                    and policy.num_actions == 5)
         lin = [m for m in policy.trunk.modules() if isinstance(m, torch.nn.Linear)]
         return (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64 and lin[1].in_features == 64
                 and lin[1].out_features == 64 and policy.logits.out_features == 5)
 
     def refresh(self):
-        """Re-pack the module's current float32 parameters (bf16, padded) and upload them."""
+        """Re-pack the module's current float32 parameters (bf16, padded; per agent: one block per agent) and upload
+        them."""
         f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
-        arrs = [f(self._lin[0].weight), f(self._lin[0].bias), f(self._lin[1].weight), f(self._lin[1].bias),
-                f(self.policy.logits.weight), f(self.policy.logits.bias), f(self.policy.value.weight), f(self.policy.value.bias)]
-        nat.check(self._lib.mapf_policy_pack_weights(self.F, *[a.ctypes.data_as(C.c_void_p) for a in arrs],
-                                                     self._host.ctypes.data_as(C.c_void_p)))
+        if self.per_agent:
+            p = self.policy
+            per = _per_agent_arrays(p, [p.trunk_w[0], p.trunk_b[0], p.trunk_w[1], p.trunk_b[1], "logits_w", "logits_b",
+                                        "value_w", "value_b"])
+        else:
+            per = [[f(self._lin[0].weight), f(self._lin[0].bias), f(self._lin[1].weight), f(self._lin[1].bias),
+                    f(self.policy.logits.weight), f(self.policy.logits.bias), f(self.policy.value.weight),
+                    f(self.policy.value.bias)]]
+        for j, arrs in enumerate(per):
+            nat.check(self._lib.mapf_policy_pack_weights(self.F, *[a.ctypes.data_as(C.c_void_p) for a in arrs],
+                                                         C.c_void_p(self._host.ctypes.data + j * self._block)))
         self._dev.copy_(torch.from_numpy(self._host))
 
     def act(self, out, logits_out: torch.Tensor | None = None, features_out: torch.Tensor | None = None,
@@ -77,29 +121,37 @@ class FusedPolicy:
             blocking_prev=p(out.blocking_prev) if self.with_bp else None, action_mask=p(out.action_mask),
             weights=p(self._dev), actions=p(self.actions), actions64=p(actions64), logp=p(logp), value=p(value),
             logits_out=p(logits_out), features_out=p(features_out), action_mask_out=p(mask_out))
-        nat.check(self._lib.mapf_policy_act(C.byref(args), env._stream()))
+        nat.check(self._act(C.byref(args), env._stream()))
         return self.actions, logp, value
 
 
 class FusedRecurrentPolicy:
     """Inference view of a :class:`recurrent.RecurrentActionMaskPolicy` of the reference's shape (trunk 64-64, LSTM
     cell 64 fed with the previous action and reward): features -> trunk -> LSTM cell -> masked draw in ONE launch
-    (``mapf_lstm_policy_act``).  The module stays the learner's model: call :meth:`refresh` after every optimizer
-    step.  Other shapes are refused (``ValueError``); run those through the module itself."""
+    (``mapf_lstm_policy_act``); or of a :class:`recurrent.PerAgentRecurrentPolicy` of that shape with one module per
+    env agent (``mapf_lstm_policy_act_per_agent``, :attr:`entry`).  The module stays the learner's model: call
+    :meth:`refresh` after every optimizer step.  Other shapes are refused (``ValueError``); run those through the
+    module itself."""
 
     def __init__(self, policy, env, seed: int | None = None):
-        lin = [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
         F = int(env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0))
+        self.per_agent = _per_agent_kind(policy) is not None
         if not FusedRecurrentPolicy.matches(policy, env):
             raise ValueError("the fused LSTM kernel implements the reference's policy only: trunk (64, 64) over "
                              f"F = V*V + 2 (+1) = {F} features, LSTM cell 64 with previous action and previous reward, "
-                             "5 actions")
+                             "5 actions" + (f"; per agent, one module per env agent: the policy has {policy.num_agents} "
+                                            f"agents, the env {env.N}" if self.per_agent else ""))
+        lin = None if self.per_agent else [m for m in policy.trunk if isinstance(m, torch.nn.Linear)]
         self.policy, self.env, self.F, self._lin = policy, env, F, lin
         self.with_bp = bool(env.include_blocking_pressure)
         self._lib = nat.lib()
+        self.entry = "mapf_lstm_policy_act_per_agent" if self.per_agent else "mapf_lstm_policy_act"
+        self._act = getattr(self._lib, self.entry)
         n = int(self._lib.mapf_lstm_policy_weights_nbytes(self.F))
         if n < 0:
             raise nat.MapfError(n, self._lib.mapf_last_error().decode())
+        self._block = n
+        n *= policy.num_agents if self.per_agent else 1   # per agent: block j at j * n
         self._host = np.zeros(n, np.uint8)
         self._dev = torch.zeros(n, dtype=torch.uint8, device=env.device)
         B, N, dev = env.B, env.N, env.device
@@ -117,6 +169,11 @@ class FusedRecurrentPolicy:
         feature width: trunk (64, 64) over F = V*V + 2 (+1 pressure) features, LSTM cell 64 fed with the previous
         action and reward, 5 actions."""
         F = env.V * env.V + 2 + (1 if env.include_blocking_pressure else 0)
+        kind = _per_agent_kind(policy)
+        if kind is not None:   # a recurrent.PerAgentRecurrentPolicy: every agent's module has the reference's shape
+            return (kind == "lstm" and policy.num_agents == env.N and policy.feature_dim == F and tuple(policy.hiddens) == (64, 64)
+                    and policy.cell == 64 and policy.num_actions == 5 and policy.use_prev_action
+                    and policy.use_prev_reward)
         lin = [m for m in policy.trunk.modules() if isinstance(m, torch.nn.Linear)]
         return (len(lin) == 2 and lin[0].in_features == F and lin[0].out_features == 64
                 and lin[1].in_features == 64 and lin[1].out_features == 64 and policy.cell == 64
@@ -124,14 +181,21 @@ class FusedRecurrentPolicy:
                 and policy.lstm.input_size == 64 + 5 + 1 and policy.lstm.hidden_size == 64)
 
     def refresh(self):
-        """Re-pack the module's current float32 parameters (bf16, padded; b_ih + b_hh summed) and upload them."""
+        """Re-pack the module's current float32 parameters (bf16, padded; b_ih + b_hh summed; per agent: one block per
+        agent) and upload them."""
         f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
-        p, lstm = self.policy, self.policy.lstm
-        arrs = [f(self._lin[0].weight), f(self._lin[0].bias), f(self._lin[1].weight), f(self._lin[1].bias),
-                f(lstm.weight_ih), f(lstm.weight_hh), f(lstm.bias_ih), f(lstm.bias_hh),
-                f(p.logits.weight), f(p.logits.bias), f(p.value.weight), f(p.value.bias)]
-        nat.check(self._lib.mapf_lstm_policy_pack_weights(self.F, *[a.ctypes.data_as(C.c_void_p) for a in arrs],
-                                                          self._host.ctypes.data_as(C.c_void_p)))
+        p = self.policy
+        if self.per_agent:
+            per = _per_agent_arrays(p, [p.trunk_w[0], p.trunk_b[0], p.trunk_w[1], p.trunk_b[1], "w_ih", "w_hh", "b_ih",
+                                        "b_hh", "logits_w", "logits_b", "value_w", "value_b"])
+        else:
+            lstm = p.lstm
+            per = [[f(self._lin[0].weight), f(self._lin[0].bias), f(self._lin[1].weight), f(self._lin[1].bias),
+                    f(lstm.weight_ih), f(lstm.weight_hh), f(lstm.bias_ih), f(lstm.bias_hh),
+                    f(p.logits.weight), f(p.logits.bias), f(p.value.weight), f(p.value.bias)]]
+        for j, arrs in enumerate(per):
+            nat.check(self._lib.mapf_lstm_policy_pack_weights(self.F, *[a.ctypes.data_as(C.c_void_p) for a in arrs],
+                                                              C.c_void_p(self._host.ctypes.data + j * self._block)))
         self._dev.copy_(torch.from_numpy(self._host))
 
     def args(self, out_channels: dict, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *,
@@ -180,7 +244,7 @@ class FusedRecurrentPolicy:
                       actions64=actions64, logp=logp, value=value, logits_out=logits_out, greedy=greedy)
         self.counter += 1
         a.counter = self.counter
-        nat.check(self._lib.mapf_lstm_policy_act(C.byref(a), self.env._stream()))
+        nat.check(self._act(C.byref(a), self.env._stream()))
         return self.actions, logp, value
 
 

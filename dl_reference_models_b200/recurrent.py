@@ -25,7 +25,8 @@ from dataclasses import dataclass
 import torch
 from torch import nn
 
-from .rollout import FLOAT_MIN, gae, observation_rows, sample_categorical
+from .rollout import (FLOAT_MIN, agent_linear, draw_permutation, gae, normalize_advantages, observation_rows,
+                      per_agent_minibatches, ppo_loss, sample_categorical, stack_parameters)
 
 
 def features_from_channels(local_obs: torch.Tensor, goal_delta: torch.Tensor, blocking_prev: torch.Tensor | None) -> torch.Tensor:
@@ -81,6 +82,92 @@ class RecurrentActionMaskPolicy(nn.Module):
             lg.append(l)
             vs.append(v)
         return torch.stack(lg), torch.stack(vs), (h, c)
+
+
+class PerAgentRecurrentPolicy(nn.Module):
+    """One :class:`RecurrentActionMaskPolicy` per agent (the reference's DTE mode), parameters stacked along a leading
+    agent dimension (``trunk_w[k]`` / ``trunk_b[k]``, ``w_ih`` [N, 4 cell, in], ``w_hh``, ``b_ih``, ``b_hh``,
+    ``logits_w`` / ``logits_b``, ``value_w`` / ``value_b``; torch LSTMCell's gate order [i; f; g; o]).  Inputs follow
+    :class:`rollout.PerAgentActionMaskPolicy`'s convention: flat rows whose count is a multiple of ``num_agents``, row
+    r of agent ``r % num_agents`` (the [B*N, ...] rows of :class:`RecurrentCollector`, the state's [B*N, cell] layout).
+    :meth:`from_modules` / :meth:`module` convert from / to ordinary modules; the default initialisation is N
+    independently initialised ones."""
+
+    def __init__(self, num_agents: int, feature_dim: int, num_actions: int = 5, hiddens=(64, 64), cell: int = 64,
+                 use_prev_action: bool = True, use_prev_reward: bool = True):
+        super().__init__()
+        self._stack([RecurrentActionMaskPolicy(feature_dim, num_actions, hiddens, cell, use_prev_action, use_prev_reward)
+                     for _ in range(int(num_agents))])
+
+    @classmethod
+    def from_modules(cls, modules) -> "PerAgentRecurrentPolicy":
+        """Agent j's parameters are copies of ``modules[j]``'s (N :class:`RecurrentActionMaskPolicy` of one shape)."""
+        self = cls.__new__(cls)
+        nn.Module.__init__(self)
+        self._stack(list(modules))
+        return self
+
+    @staticmethod
+    def _shape(m) -> tuple:
+        lin = [x for x in m.trunk.modules() if isinstance(x, nn.Linear)]
+        feature_dim = lin[0].in_features if lin else m.lstm.input_size - m.num_actions * m.use_prev_action - m.use_prev_reward
+        return (int(feature_dim), tuple(x.out_features for x in lin), m.num_actions, m.cell, m.use_prev_action,
+                m.use_prev_reward)
+
+    def _stack(self, mods):
+        if not mods or any(self._shape(m) != self._shape(mods[0]) for m in mods):
+            raise ValueError(f"from_modules needs one or more modules of one shape, got {[self._shape(m) for m in mods]}")
+        self.num_agents = len(mods)
+        (self.feature_dim, self.hiddens, self.num_actions, self.cell, self.use_prev_action,
+         self.use_prev_reward) = self._shape(mods[0])
+        lins = [[x for x in m.trunk.modules() if isinstance(x, nn.Linear)] for m in mods]
+        self.trunk_w = nn.ParameterList([stack_parameters(ls[k].weight for ls in lins) for k in range(len(self.hiddens))])
+        self.trunk_b = nn.ParameterList([stack_parameters(ls[k].bias for ls in lins) for k in range(len(self.hiddens))])
+        for name, get in (("w_ih", lambda m: m.lstm.weight_ih), ("w_hh", lambda m: m.lstm.weight_hh),
+                          ("b_ih", lambda m: m.lstm.bias_ih), ("b_hh", lambda m: m.lstm.bias_hh),
+                          ("logits_w", lambda m: m.logits.weight), ("logits_b", lambda m: m.logits.bias),
+                          ("value_w", lambda m: m.value.weight), ("value_b", lambda m: m.value.bias)):
+            setattr(self, name, stack_parameters(get(m) for m in mods))
+
+    def module(self, j: int) -> RecurrentActionMaskPolicy:
+        """Agent j's policy as an ordinary :class:`RecurrentActionMaskPolicy` (a copy, on this module's device)."""
+        with torch.random.fork_rng(devices=[]):   # the throw-away default init must not move the caller's RNG
+            m = RecurrentActionMaskPolicy(self.feature_dim, self.num_actions, self.hiddens, self.cell,
+                                          self.use_prev_action, self.use_prev_reward)
+        m = m.to(self.w_ih.device)
+        with torch.no_grad():
+            for lin, w, b in zip([x for x in m.trunk.modules() if isinstance(x, nn.Linear)], self.trunk_w, self.trunk_b):
+                lin.weight.copy_(w[j])
+                lin.bias.copy_(b[j])
+            for t, name in ((m.lstm.weight_ih, "w_ih"), (m.lstm.weight_hh, "w_hh"), (m.lstm.bias_ih, "b_ih"),
+                            (m.lstm.bias_hh, "b_hh"), (m.logits.weight, "logits_w"), (m.logits.bias, "logits_b"),
+                            (m.value.weight, "value_w"), (m.value.bias, "value_b")):
+                t.copy_(getattr(self, name)[j])
+        return m
+
+    initial_state = RecurrentActionMaskPolicy.initial_state
+    sequence = RecurrentActionMaskPolicy.sequence   # steps through :meth:`step`
+
+    def step(self, features, action_mask, prev_action, prev_reward, state):
+        """One time step for flat rows [M, ...] (row r of agent r % N): (masked logits [M, A], value [M], new state)."""
+        N = self.num_agents
+        per = lambda x: x.reshape(-1, N, *x.shape[1:]).transpose(0, 1)   # noqa: E731  [M, ...] -> [N, M / N, ...]
+        flat = lambda x: x.transpose(0, 1).reshape(-1, *x.shape[2:])    # noqa: E731  and back
+        z = per(features.float())
+        for w, b in zip(self.trunk_w, self.trunk_b):
+            z = torch.relu(agent_linear(z, w, b))
+        x = [z]
+        if self.use_prev_action:
+            x.append(torch.nn.functional.one_hot(per(prev_action).long(), self.num_actions).to(z.dtype))
+        if self.use_prev_reward:
+            x.append(per(prev_reward).to(z.dtype).unsqueeze(-1))
+        gates = agent_linear(torch.cat(x, dim=-1), self.w_ih, self.b_ih) + agent_linear(per(state[0]), self.w_hh, self.b_hh)
+        i, f, g, o = gates.chunk(4, dim=-1)
+        c = torch.sigmoid(f) * per(state[1]) + torch.sigmoid(i) * torch.tanh(g)
+        h = torch.sigmoid(o) * torch.tanh(c)
+        logits = flat(agent_linear(h, self.logits_w, self.logits_b))
+        logits = logits + torch.clamp(torch.log(action_mask.to(h.dtype) + 1e-6), min=FLOAT_MIN)
+        return logits, flat(agent_linear(h, self.value_w, self.value_b)).squeeze(-1), (flat(h), flat(c))
 
 
 @dataclass
@@ -227,6 +314,7 @@ class FusedRecurrentCollector:
 
         self._couts = [nat.MapfOutputs(**{k: dst(k, t).data_ptr() for k in nat.OUTPUT_FIELDS}) for t in range(T)]
         self._actions_ptr = C.c_void_p(self.act8.data_ptr())
+        self._act = getattr(self._lib, fused.entry)   # mapf_lstm_policy_act, or its per-agent variant
 
     @torch.no_grad()
     def collect(self) -> CompactRollout:
@@ -252,12 +340,12 @@ class FusedRecurrentCollector:
             fused.counter += 1
             a = self._pargs[t]
             a.counter = fused.counter
-            check(lib.mapf_lstm_policy_act(C.byref(a), stream))
+            check(self._act(C.byref(a), stream))
             check(lib.mapf_step(hnd, self._actions_ptr, None, None, C.byref(self._couts[t]), 1, stream))
         fused.counter += 1
         a = self._pargs[T]
         a.counter = fused.counter
-        check(lib.mapf_lstm_policy_act(C.byref(a), stream))
+        check(self._act(C.byref(a), stream))
         dones = (self.term | self.trunc).bool()
         resets[1:] = dones[:-1]
         self.prev_actions[1:] = self.actions[:-1]
@@ -304,11 +392,17 @@ def ppo_update_recurrent(policy: RecurrentActionMaskPolicy, optimizer, batch: Co
                          max_minibatches: int | None = None, generator: torch.Generator | None = None) -> dict:
     """PPO over sequence minibatches: ``minibatch`` time steps = ``minibatch / max_seq_len`` sequences of one agent,
     each re-run through the LSTM from its stored start state (truncated BPTT).  Every rank draws its own minibatches
-    from its own shard; gradients are averaged over the ranks before each optimizer step."""
+    from its own shard; gradients are averaged over the ranks before each optimizer step.  A
+    :class:`PerAgentRecurrentPolicy` is trained as N independent learners in lockstep (see :func:`rollout.ppo_update`):
+    advantages normalised per agent, ``minibatch / max_seq_len`` of agent j's own sequences for every j per step
+    (agent-fastest), the loss summed over the agents' mean losses."""
     L = int(max_seq_len)
     T, B, N = batch.actions.shape
+    per_agent = isinstance(policy, PerAgentRecurrentPolicy)
+    if per_agent and policy.num_agents != N:
+        raise ValueError(f"the policy has {policy.num_agents} agents, the batch {N}")
     adv, ret = gae(batch.rewards, batch.values, batch.dones, batch.last_value, gamma, lam)
-    adv = (adv - adv.mean()) / (adv.std() + 1e-8)
+    adv = normalize_advantages(adv, per_agent)
     nchunks, M = T // L, B * N
     per_mb = max(1, minibatch // L)
 
@@ -321,29 +415,29 @@ def ppo_update_recurrent(policy: RecurrentActionMaskPolicy, optimizer, batch: Co
     rs = batch.resets.unsqueeze(-1).expand(T, B, N).reshape(nchunks, L, M)
     stats, done_mb = {}, 0
     total = nchunks * M
+
+    def minibatches():   # sequence numbers idx: chunk idx // M, row idx % M
+        if per_agent:   # sequence s of agent j: chunk s // B, row (s % B) * N + j
+            cols = torch.arange(N, device=ac.device)
+            for s in per_agent_minibatches(nchunks * B, N, per_mb, ac.device, generator):
+                yield ((s // B) * M + (s % B) * N + cols).reshape(-1)
+        else:
+            perm = draw_permutation(total, ac.device, generator)
+            for i in range(0, total, per_mb):
+                yield perm[i:i + per_mb]
+
     for _ in range(epochs):
-        perm = torch.randperm(total, device=ac.device, generator=generator) if generator is None or generator.device == ac.device \
-            else torch.randperm(total, generator=generator).to(ac.device)
-        for i in range(0, total, per_mb):
-            idx = perm[i:i + per_mb]
+        for idx in minibatches():
             ck, m = idx // M, idx % M
             g = lambda x: x[ck, :, m].transpose(0, 1)   # noqa: E731  -> [L, S, ...]
             feats = features_from_channels(g(lo), g(gd), g(bp))   # expanded here, per minibatch: 34 B -> 112 B per row
             lg, v, _ = policy.sequence(feats, g(mk), g(pa), g(pr), g(rs), (batch.chunk_h[ck, m], batch.chunk_c[ck, m]))
-            dist_ = torch.distributions.Categorical(logits=lg)
-            lp = dist_.log_prob(g(ac))
-            ratio = torch.exp(lp - g(olp))
-            a_ = g(av)
-            surr = torch.min(ratio * a_, torch.clamp(ratio, 1 - clip, 1 + clip) * a_)
-            vf = (v - g(rt)).pow(2).mean()
-            ent = dist_.entropy().mean()
-            loss = -surr.mean() + vf_coeff * vf - entropy_coeff * ent
+            loss, stats = ppo_loss(lg, v, g(ac), g(olp), g(av), g(rt), clip=clip, vf_coeff=vf_coeff,
+                                   entropy_coeff=entropy_coeff, num_agents=N if per_agent else None)
             optimizer.zero_grad(set_to_none=True)
             loss.backward()
             allreduce_gradients(policy, world_size, group)
             optimizer.step()
-            stats = {"loss": float(loss.detach()), "vf_loss": float(vf.detach()), "entropy": float(ent.detach()),
-                     "policy_loss": float(-surr.mean().detach())}
             done_mb += 1
             if max_minibatches is not None and done_mb >= max_minibatches:
                 return stats
@@ -353,7 +447,9 @@ def ppo_update_recurrent(policy: RecurrentActionMaskPolicy, optimizer, batch: Co
 def benchmark(num_envs: int = 65536, steps: int = 64, max_seq_len: int = 32, rounds: int = 3, device: str = "cuda:0") -> dict:
     """C3 (num_envs x 16 agents, 32x32 map, lifelong): agent-steps/s of the env alone, of :class:`RecurrentCollector`
     (the PyTorch module's forward every step) and of :class:`FusedRecurrentCollector` (one policy launch + one env
-    launch per step), the two collectors alternated in the same process after a warm-up collect each.  Rates are the
+    launch per step) with a shared policy and with a :class:`PerAgentRecurrentPolicy` (one LSTM per agent,
+    ``mapf_lstm_policy_act_per_agent``), the three collectors alternated in the same process after a warm-up collect
+    each.  Rates are the
     best of ``rounds`` timed collects (host clock around work that ends in a device synchronise)."""
     import subprocess
     import time
@@ -361,6 +457,7 @@ def benchmark(num_envs: int = 65536, steps: int = 64, max_seq_len: int = 32, rou
     from . import maps
     from .batched_env import BatchedMapfEnv
     from .policy_kernels import FusedRecurrentPolicy
+    from .recurrent import PerAgentRecurrentPolicy   # the package's class (this file may run as __main__)
 
     cfg = {"num_agents": 16, "sensor_range": 2, "steps_per_episode": 256, "lifelong_mapf": True, "seed": 999,
            "grid": maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32)}
@@ -385,12 +482,16 @@ def benchmark(num_envs: int = 65536, steps: int = 64, max_seq_len: int = 32, rou
     pol = RecurrentActionMaskPolicy(env.flat_obs_dim(include_action_mask=False)).to(env.device)
     torch_col = RecurrentCollector(env, pol, max_seq_len)
     fused_col = FusedRecurrentCollector(env, FusedRecurrentPolicy(pol, env), steps, max_seq_len)
+    per_agent = PerAgentRecurrentPolicy(env.N, env.flat_obs_dim(include_action_mask=False)).to(env.device)
+    per_agent_col = FusedRecurrentCollector(env, FusedRecurrentPolicy(per_agent, env), steps, max_seq_len)
     torch_col.collect(steps)   # warm-up: allocator, cuBLAS / kernel selection, module load
     fused_col.collect()
-    ts, fs = [], []
+    per_agent_col.collect()
+    ts, fs, ps = [], [], []
     for _ in range(rounds):
         ts.append(timed(lambda: torch_col.collect(steps)))
         fs.append(timed(fused_col.collect))
+        ps.append(timed(per_agent_col.collect))
     try:
         gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i",
                               str(env.device.index)], capture_output=True, text=True, timeout=30).stdout.strip()
@@ -401,7 +502,8 @@ def benchmark(num_envs: int = 65536, steps: int = 64, max_seq_len: int = 32, rou
             "max_seq_len": max_seq_len, "env_only_agent_steps_per_s": n / env_s,
             "torch_recurrent_collector_agent_steps_per_s": n / min(ts),
             "fused_recurrent_collector_agent_steps_per_s": n / min(fs),
-            "torch_collect_s": ts, "fused_collect_s": fs}
+            "fused_per_agent_recurrent_collector_agent_steps_per_s": n / min(ps),
+            "torch_collect_s": ts, "fused_collect_s": fs, "fused_per_agent_collect_s": ps}
 
 
 if __name__ == "__main__":

@@ -49,6 +49,87 @@ class ActionMaskPolicy(nn.Module):
         return logits + inf_mask, value
 
 
+def agent_linear(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """Per-agent ``Linear``: x [N, R, in], w [N, out, in], b [N, out] -> [N, R, out] (one batched matmul)."""
+    return torch.baddbmm(b.unsqueeze(1), x, w.transpose(1, 2))
+
+
+def stack_parameters(tensors) -> nn.Parameter:
+    """One parameter stacked along a leading agent dimension from the same parameter of N modules."""
+    return nn.Parameter(torch.stack([t.detach() for t in tensors]).clone())
+
+
+class PerAgentActionMaskPolicy(nn.Module):
+    """One :class:`ActionMaskPolicy` per agent: the reference's DTE mode, where agent j is played and trained by its own
+    module.  The parameters are stacked along a leading agent dimension (``trunk_w[k]`` [N, out, in], ``trunk_b[k]``
+    [N, out], ``logits_w`` / ``logits_b``, ``value_w`` / ``value_b``).  Inputs are flat rows whose count is a multiple of
+    ``num_agents``, and row r belongs to agent ``r % num_agents``: the [..., B, N, ...] order of every buffer of this
+    package, so a [T,B,N,F] block or its [T*B*N, F] view goes in as it is.  The forward is batched matmuls over the
+    agent dimension.  Default initialisation: N independently initialised :class:`ActionMaskPolicy` modules;
+    :meth:`from_modules` / :meth:`module` convert from / to those (RLlib's per-agent modules map to them one to one)."""
+
+    def __init__(self, num_agents: int, feature_dim: int, num_actions: int = 5, hiddens=(64, 64), no_masking: bool = False):
+        super().__init__()
+        self._stack([ActionMaskPolicy(feature_dim, num_actions, hiddens, no_masking) for _ in range(int(num_agents))])
+
+    @classmethod
+    def from_modules(cls, modules) -> "PerAgentActionMaskPolicy":
+        """Agent j's parameters are copies of ``modules[j]``'s (N :class:`ActionMaskPolicy` of one shape)."""
+        self = cls.__new__(cls)
+        nn.Module.__init__(self)
+        self._stack(list(modules))
+        return self
+
+    def _stack(self, mods):
+        shape = lambda m: (_in_features(m), tuple(x.out_features for x in _linears(m)), m.logits.out_features,  # noqa: E731
+                           bool(m.no_masking))
+        if not mods or any(shape(m) != shape(mods[0]) for m in mods):
+            raise ValueError(f"from_modules needs one or more modules of one shape, got {[shape(m) for m in mods]}")
+        self.num_agents = len(mods)
+        self.feature_dim, self.hiddens, self.num_actions, self.no_masking = shape(mods[0])
+        lins = [_linears(m) for m in mods]
+        self.trunk_w = nn.ParameterList([stack_parameters(ls[k].weight for ls in lins) for k in range(len(self.hiddens))])
+        self.trunk_b = nn.ParameterList([stack_parameters(ls[k].bias for ls in lins) for k in range(len(self.hiddens))])
+        self.logits_w, self.logits_b = stack_parameters(m.logits.weight for m in mods), stack_parameters(m.logits.bias for m in mods)
+        self.value_w, self.value_b = stack_parameters(m.value.weight for m in mods), stack_parameters(m.value.bias for m in mods)
+
+    def module(self, j: int) -> ActionMaskPolicy:
+        """Agent j's policy as an ordinary :class:`ActionMaskPolicy` (a copy, on this module's device)."""
+        with torch.random.fork_rng(devices=[]):   # the throw-away default init must not move the caller's RNG
+            m = ActionMaskPolicy(self.feature_dim, self.num_actions, self.hiddens, self.no_masking)
+        m = m.to(self.logits_w.device)
+        with torch.no_grad():
+            for lin, w, b in zip(_linears(m), self.trunk_w, self.trunk_b):
+                lin.weight.copy_(w[j])
+                lin.bias.copy_(b[j])
+            m.logits.weight.copy_(self.logits_w[j])
+            m.logits.bias.copy_(self.logits_b[j])
+            m.value.weight.copy_(self.value_w[j])
+            m.value.bias.copy_(self.value_b[j])
+        return m
+
+    def forward(self, features: torch.Tensor, action_mask: torch.Tensor):
+        """features [..., F] float, action_mask [..., A], flat row r of agent r % N -> (masked logits, value)."""
+        lead, N = features.shape[:-1], self.num_agents
+        z = features.float().reshape(-1, N, features.shape[-1]).transpose(0, 1)   # [N, rows / N, F]
+        for w, b in zip(self.trunk_w, self.trunk_b):
+            z = torch.relu(agent_linear(z, w, b))
+        logits = agent_linear(z, self.logits_w, self.logits_b).transpose(0, 1).reshape(*lead, -1)
+        value = agent_linear(z, self.value_w, self.value_b).transpose(0, 1).reshape(lead)
+        if self.no_masking:
+            return logits, value
+        return logits + torch.clamp(torch.log(action_mask.to(logits.dtype) + 1e-6), min=FLOAT_MIN), value
+
+
+def _linears(m) -> list:
+    return [x for x in m.trunk.modules() if isinstance(x, nn.Linear)]
+
+
+def _in_features(m) -> int:
+    lin = _linears(m)
+    return int(lin[0].in_features if lin else m.logits.in_features)
+
+
 @dataclass
 class Batch:
     features: torch.Tensor   # [T,B,N,F]
@@ -186,6 +267,7 @@ class FusedCollector:
 
         self._couts = [nat.MapfOutputs(**{k: dst(k, t).data_ptr() for k in nat.OUTPUT_FIELDS}) for t in range(T)]
         self._actions_ptr = vp(fused.actions)
+        self._act = getattr(self._lib, fused.entry)   # mapf_policy_act, or its per-agent variant
 
     @torch.no_grad()
     def collect(self) -> Batch:
@@ -201,12 +283,12 @@ class FusedCollector:
             fused.counter += 1
             a = self._pargs[t]
             a.counter = fused.counter
-            check(lib.mapf_policy_act(C.byref(a), stream))
+            check(self._act(C.byref(a), stream))
             check(lib.mapf_step(h, self._actions_ptr, None, None, C.byref(self._couts[t]), 1, stream))
         fused.counter += 1
         a = self._pargs[self.T]
         a.counter = fused.counter
-        check(lib.mapf_policy_act(C.byref(a), stream))
+        check(self._act(C.byref(a), stream))
         dones = (self.term | self.trunc).bool()
         if self.compact:
             for k, r in self.obs_rows.items():   # the env's own buffers show the latest observation again
@@ -271,35 +353,88 @@ def gae(rewards, values, dones, last_value, gamma: float = 0.99, lam: float = 0.
     return adv, adv + values
 
 
+def ppo_loss(lg, v, acts, old_logp, adv, ret, *, clip: float, vf_coeff: float, entropy_coeff: float,
+             num_agents: int | None = None):
+    """The clipped PPO loss of one minibatch (logits ``lg`` [..., A], values / actions / old log-probabilities /
+    advantages / returns [...]) and its stats.  ``num_agents``: the rows are agent-fastest (flat row r of agent
+    r % num_agents, the same number of rows per agent) and every mean is taken per agent, then summed over the agents:
+    N independent learners, agent j's parameters getting agent j's mean loss's gradient."""
+    dist = torch.distributions.Categorical(logits=lg)
+    lp = dist.log_prob(acts)
+    ratio = torch.exp(lp - old_logp)
+    surr = torch.min(ratio * adv, torch.clamp(ratio, 1 - clip, 1 + clip) * adv)
+    mean = (lambda x: x.mean()) if num_agents is None else (lambda x: x.reshape(-1, num_agents).mean(0).sum())  # noqa: E731
+    vf = mean((v - ret).pow(2))
+    ent = mean(dist.entropy())
+    policy_loss = -mean(surr)
+    loss = policy_loss + vf_coeff * vf - entropy_coeff * ent
+    return loss, {"loss": float(loss.detach()), "vf_loss": float(vf.detach()), "entropy": float(ent.detach()),
+                  "policy_loss": float(policy_loss.detach())}
+
+
+def normalize_advantages(adv: torch.Tensor, per_agent: bool) -> torch.Tensor:
+    """(adv - mean) / (std + 1e-8) over the whole [T,B,N] block, or per agent (over T and B) for per-agent policies."""
+    if per_agent:
+        return (adv - adv.mean((0, 1))) / (adv.std((0, 1)) + 1e-8)
+    return (adv - adv.mean()) / (adv.std() + 1e-8)
+
+
+def draw_permutation(n: int, device, generator: torch.Generator | None = None) -> torch.Tensor:
+    """torch.randperm(n) on ``device`` from ``generator`` (the global RNG by default), drawn where the generator lives."""
+    if generator is None or generator.device == torch.device(device):
+        return torch.randperm(n, device=device, generator=generator)
+    return torch.randperm(n, generator=generator).to(device)
+
+
+def per_agent_minibatches(n_per_agent: int, N: int, size: int, device, generator: torch.Generator | None = None):
+    """One epoch of a per-agent learner's minibatches: for every agent j (in order) a permutation of its
+    ``n_per_agent`` samples, then per step ``size`` of each agent's samples.  Yields [size', N] sample numbers s of
+    each agent (column j: agent j's), size' = size except for a shorter last step."""
+    perm = torch.stack([draw_permutation(n_per_agent, device, generator) for _ in range(N)], dim=1)
+    for i in range(0, n_per_agent, size):
+        yield perm[i:i + size]
+
+
 def ppo_update(policy, optimizer, batch: Batch, *, clip: float = 0.05, vf_coeff: float = 0.5,
                entropy_coeff: float = 0.001, epochs: int = 12, minibatch: int = 1024, gamma: float = 0.99,
-               lam: float = 0.95, max_minibatches: int | None = None) -> dict:
+               lam: float = 0.95, max_minibatches: int | None = None, generator: torch.Generator | None = None) -> dict:
+    """PPO epochs over a :class:`Batch` / :class:`CompactBatch`.  ``generator`` (optional) draws the minibatch
+    permutations.  A :class:`PerAgentActionMaskPolicy` is trained as N independent learners run in lockstep: each
+    agent's advantages are normalised over its own samples; every step takes ``minibatch`` of agent j's samples for
+    every j (one permutation per agent and epoch, drawn in agent order), laid out agent-fastest; the loss is the sum of
+    the per-agent mean losses, so one element-wise optimizer over the stacked parameters is N independent ones."""
     adv, ret = gae(batch.rewards, batch.values, batch.dones, batch.last_value, gamma, lam)
+    per_agent = isinstance(policy, PerAgentActionMaskPolicy)
+    N = batch.actions.shape[-1]
     compact = isinstance(batch, CompactBatch)
     feats = None if compact else batch.features.reshape(-1, batch.features.shape[-1])
     masks = batch.masks.reshape(-1, batch.masks.shape[-1])
     acts, old_logp = batch.actions.reshape(-1), batch.logp.reshape(-1)
-    adv, ret = adv.reshape(-1), ret.reshape(-1)
-    adv = (adv - adv.mean()) / (adv.std() + 1e-8)
+    adv = normalize_advantages(adv, per_agent).reshape(-1)
+    ret = ret.reshape(-1)
     n = acts.shape[0]
+    if per_agent and policy.num_agents != N:
+        raise ValueError(f"the policy has {policy.num_agents} agents, the batch {N}")
+
+    def minibatches():
+        if per_agent:   # sample s of agent j is flat row s * N + j
+            cols = torch.arange(N, device=acts.device)
+            for s in per_agent_minibatches(n // N, N, minibatch, acts.device, generator):
+                yield (s * N + cols).reshape(-1)
+        else:
+            perm = draw_permutation(n, acts.device, generator)
+            for i in range(0, n, minibatch):
+                yield perm[i:i + minibatch]
+
     stats, done_mb = {}, 0
     for _ in range(epochs):
-        perm = torch.randperm(n, device=acts.device)
-        for i in range(0, n, minibatch):
-            idx = perm[i:i + minibatch]
+        for idx in minibatches():
             lg, v = policy(batch.features_of(idx) if compact else feats[idx], masks[idx])
-            dist = torch.distributions.Categorical(logits=lg)
-            lp = dist.log_prob(acts[idx])
-            ratio = torch.exp(lp - old_logp[idx])
-            surr = torch.min(ratio * adv[idx], torch.clamp(ratio, 1 - clip, 1 + clip) * adv[idx])
-            vf = (v - ret[idx]).pow(2).mean()
-            ent = dist.entropy().mean()
-            loss = -surr.mean() + vf_coeff * vf - entropy_coeff * ent
+            loss, stats = ppo_loss(lg, v, acts[idx], old_logp[idx], adv[idx], ret[idx], clip=clip, vf_coeff=vf_coeff,
+                                   entropy_coeff=entropy_coeff, num_agents=N if per_agent else None)
             optimizer.zero_grad(set_to_none=True)
             loss.backward()
             optimizer.step()
-            stats = {"loss": float(loss), "vf_loss": float(vf), "entropy": float(ent),
-                     "policy_loss": float(-surr.mean())}
             done_mb += 1
             if max_minibatches is not None and done_mb >= max_minibatches:
                 return stats

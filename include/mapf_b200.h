@@ -489,6 +489,18 @@ int mapf_lstm_policy_pack_weights(int32_t feature_dim, const float *w1, const fl
                                   const float *w_logits, const float *b_logits, const float *w_value, const float *b_value,
                                   void *packed_host);
 int mapf_lstm_policy_act(const mapf_lstm_policy_args *args, void *stream);
+
+/* Per-agent policies (one weight set per agent, the reference's DTE mode): the same arguments, with args->weights
+ * pointing to num_agents consecutive packed blocks; block j, at j * mapf_[lstm_]policy_weights_nbytes(feature_dim),
+ * is written by the pack function above from agent j's parameters.  Agent j's outputs (actions, actions64, logp,
+ * value, logits_out, features_out, action_mask_out; for the LSTM also h_out / c_out) equal, bit for bit, those the
+ * shared entry point writes at agent j's rows when it runs with block j alone: in draw mode (the same Philox key and
+ * counter) and in greedy mode, with episode-start flags, with the state updated in place or not.  The checks are
+ * those of the shared entry points, plus num_agents <= MAPF_MAX_AGENTS (MAPF_ERR_UNSUPPORTED), all before any device
+ * work.  A CTA works on one agent's rows at a time and reloads that agent's block into shared memory when its
+ * agent changes. */
+int mapf_policy_act_per_agent(const mapf_policy_args *args, void *stream);
+int mapf_lstm_policy_act_per_agent(const mapf_lstm_policy_args *args, void *stream);
 /* Per-step bookkeeping of the batched evaluator (main.py:test_trained_model, one episode per env, no auto-reset), in
  * one launch after mapf_step (and after mapf_occupancy_accumulate, which reads `active` before this call clears it).
  * For every env with active[b] != 0: episode_reward[b] += sum of the agents' rewards (main.py:251), agent_reward[b,n]

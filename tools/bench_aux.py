@@ -1,5 +1,6 @@
 """Timings of the kernels next to the hot path (CUDA events, warm-up, L2-sized working sets): the fused policy
-kernels (MLP and LSTM-64), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.  `python tools/bench_aux.py`"""
+kernels (MLP and LSTM-64, shared and per-agent), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.
+`python tools/bench_aux.py`"""
 import json
 import sys
 from pathlib import Path
@@ -26,6 +27,40 @@ def timed(fn, n=50, warm=5):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / n * 1e-3
+
+
+def weight_reloads(B, N, warps, max_blocks):
+    """Weight blocks the per-agent kernels load per launch: one per (CTA, agent) pair of the CTAs' contiguous tile
+    ranges (the grid and the split of mapf_b200.cu / pol_per_agent_tiles)."""
+    tpa = (B + 31) // 32
+    ntiles = tpa * N
+    G = min((ntiles + warps - 1) // warps, max_blocks)
+    q, rm = divmod(ntiles, G)
+    n = 0
+    for b in range(G):
+        k0 = b * q + min(b, rm)
+        k1 = k0 + q + (1 if b < rm else 0)
+        n += (k1 - 1) // tpa - k0 // tpa + 1 if k1 > k0 else 0
+    return n, G
+
+
+def per_agent_entry(shared_fn, per_agent_fn, one_agent_fn, agents, bytes_per_agent, block_bytes, reloads, blocks):
+    """Shared and per-agent launches timed alternately (shared, per-agent, per-agent over the same channels viewed as
+    B*N envs of one agent, twice) in one process.  The one-agent view runs the per-agent kernel's gather and tile loop
+    over consecutive rows with one weight block per CTA: its gap to the shared launch is the per-agent code path, its gap
+    to the per-agent launch the strided rows and the weight reloads."""
+    sh, pa, one = [], [], []
+    for _ in range(2):
+        sh.append(timed(shared_fn, 200))
+        pa.append(timed(per_agent_fn, 200))
+        one.append(timed(one_agent_fn, 200))
+    s = min(pa)
+    nbytes = bytes_per_agent * agents + reloads * block_bytes
+    return {"us_per_launch": s * 1e6, "rounds_us": [x * 1e6 for x in pa], "shared_rounds_us": [x * 1e6 for x in sh],
+            "one_agent_view_rounds_us": [x * 1e6 for x in one],
+            "ratio_to_shared": s / min(sh), "agents": agents, "weight_block_bytes": block_bytes, "ctas": blocks,
+            "weight_reloads": reloads, "reload_bytes": reloads * block_bytes, "GBps": nbytes / s / 1e9,
+            "agent_steps_per_s": agents / s}
 
 
 def main():
@@ -85,6 +120,61 @@ def main():
                               "agent_steps_per_s": B * N / s, "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3),
                               "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops,
                               "hbm_floor_us": lstm_bytes * B * N / (hbm_tbs * 1e12) * 1e6}
+    # per-agent variants (one weight block per agent, mapf_*_policy_act_per_agent): same shapes, same 4-env rotation,
+    # alternated with the shared launches; GB/s = the byte models above plus the per-CTA weight reloads
+    from dl_reference_models_b200.recurrent import PerAgentRecurrentPolicy  # noqa: E402
+    from dl_reference_models_b200.rollout import PerAgentActionMaskPolicy  # noqa: E402
+
+    F = envs[0].flat_obs_dim(include_action_mask=False)
+    pfused = [policy_kernels.FusedPolicy(PerAgentActionMaskPolicy(N, F).cuda(), e) for e in envs]
+    plfused = [policy_kernels.FusedRecurrentPolicy(PerAgentRecurrentPolicy(N, F).cuda(), e) for e in envs]
+
+    def pa_act():
+        k = i[0] % 4
+        pfused[k].act(outs[k])
+        i[0] += 1
+
+    def pa_lstm_act():
+        k = i[0] % 4
+        plfused[k].act(outs[k], lstate[k], *lprev[k])
+        i[0] += 1
+
+    import ctypes as C
+
+    from dl_reference_models_b200 import _native as nat  # noqa: E402
+
+    def one_agent_view(k, lstm_kernel):   # env k's channels as B*N envs of one agent (agent 0's block)
+        f = plfused[k] if lstm_kernel else pfused[k]
+        a = f.args({c: getattr(outs[k], c) for c in ("local_obs", "goal_delta", "blocking_prev", "action_mask")},
+                   lstate[k], *lprev[k], state_out=lstate[k], actions=f.actions, actions64=f.actions64, logp=f.logp,
+                   value=f.value) if lstm_kernel else None
+        if not lstm_kernel:
+            p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
+            a = nat.MapfPolicyArgs(v2=f.env.V * f.env.V, feature_dim=f.F, seed=f.seed, local_obs=p(outs[k].local_obs),
+                                   goal_delta=p(outs[k].goal_delta), blocking_prev=p(outs[k].blocking_prev),
+                                   action_mask=p(outs[k].action_mask), weights=p(f._dev), actions=p(f.actions),
+                                   actions64=p(f.actions64), logp=p(f.logp), value=p(f.value))
+        a.num_envs, a.num_agents, a.counter = B * N, 1, 1
+        return a
+
+    ones = [[one_agent_view(k, False) for k in range(4)], [one_agent_view(k, True) for k in range(4)]]
+    lib, stream = nat.lib(), [e._stream() for e in envs]
+
+    def one_act(lstm_kernel):
+        fn = lib.mapf_lstm_policy_act_per_agent if lstm_kernel else lib.mapf_policy_act_per_agent
+
+        def run():
+            k = i[0] % 4
+            nat.check(fn(C.byref(ones[lstm_kernel][k]), stream[k]))
+            i[0] += 1
+        return run
+
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    n, G = weight_reloads(B, N, 8, 148 * 8)
+    res["policy_act_per_agent"] = per_agent_entry(act, pa_act, one_act(False), B * N, bytes_per_agent, pfused[0]._block, n, G)
+    n, G = weight_reloads(B, N, 16, sms)
+    res["lstm_policy_act_per_agent"] = per_agent_entry(lstm_act, pa_lstm_act, one_act(True), B * N, lstm_bytes,
+                                                       plfused[0]._block, n, G)
     del lstate, lprev
     T = 64
     rewards, values = torch.randn(T, B, N, device="cuda"), torch.randn(T, B, N, device="cuda")
@@ -101,6 +191,13 @@ def main():
     s = timed(lambda: cte.step(acts), 100)
     res["cte_step"] = {"us_per_launch": s * 1e6, "env_steps_per_s": B / s, "agent_steps_per_s": 4 * B / s,
                        "GBps": (cte.D * 4 + 200 + 20 + 40) * B / s / 1e9}
+    try:
+        import subprocess
+
+        res["gpu"] = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                                    capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        res["gpu"] = f"nvidia-smi not readable: {exc}"
     print(json.dumps(res))
 
 
