@@ -5,6 +5,7 @@
 #include "mapf_env_kernel.cuh"
 #include "mapf_pair_kernel.cuh"
 #include "mapf_cte_kernel.cuh"
+#include "mapf_cte_policy_kernel.cuh"
 #include "mapf_policy_kernel.cuh"
 #include "mapf_policy_lstm_kernel.cuh"
 #include "mapf_eval_kernel.cuh"
@@ -1753,6 +1754,70 @@ static int lstm_policy_launch(const mapf_lstm_policy_args *a, bool per_agent, vo
 
 int mapf_lstm_policy_act(const mapf_lstm_policy_args *a, void *stream) { return lstm_policy_launch(a, false, stream); }
 int mapf_lstm_policy_act_per_agent(const mapf_lstm_policy_args *a, void *stream) { return lstm_policy_launch(a, true, stream); }
+
+static bool cte_policy_shape_ok(int cells, int n) {
+    return cells >= 1 && cells <= MAPF_CTE_POLICY_MAX_CELLS && n >= 1 && n <= MAPF_MAX_AGENTS;
+}
+
+int64_t mapf_cte_policy_weights_nbytes(int32_t cells, int32_t num_agents) {
+    if (!cte_policy_shape_ok(cells, num_agents))
+        return fail(MAPF_ERR_UNSUPPORTED, "cte policy: cells %d / num_agents %d outside 1..%d / 1..%d", cells, num_agents,
+                    MAPF_CTE_POLICY_MAX_CELLS, MAPF_MAX_AGENTS);
+    return mapf::cte_weight_bytes(cells, num_agents);
+}
+
+int mapf_cte_policy_pack_weights(int32_t cells, int32_t num_agents, const float *w1, const float *b1, const float *w2,
+                                 const float *b2, const float *wl, const float *bl, const float *wv, const float *bv,
+                                 void *packed) {
+    const int64_t nbytes = mapf_cte_policy_weights_nbytes(cells, num_agents);
+    if (nbytes < 0) return (int)nbytes;
+    if (!w1 || !b1 || !w2 || !b2 || !wl || !bl || !wv || !bv || !packed) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    const int s1 = mapf::cte_s1(cells), H = mapf::POL_H, S2 = mapf::POL_W2_STRIDE, A = 5 * num_agents;
+    memset(packed, 0, (size_t)nbytes);
+    __nv_bfloat16 *p1 = static_cast<__nv_bfloat16 *>(packed), *p2 = p1 + H * s1, *p3 = p2 + H * S2;
+    float *pb = reinterpret_cast<float *>(p3 + 8 * mapf::cte_head_tiles(num_agents) * S2);
+    for (int o = 0; o < H; ++o) {
+        for (int i = 0; i < cells; ++i) p1[(size_t)o * s1 + i] = __float2bfloat16_rn(w1[(size_t)o * cells + i]);
+        for (int i = 0; i < H; ++i) p2[o * S2 + i] = __float2bfloat16_rn(w2[o * H + i]);
+        pb[o] = b1[o];
+        pb[H + o] = b2[o];
+    }
+    for (int o = 0; o < A; ++o) {   // head rows: 5N logits, then the value
+        for (int i = 0; i < H; ++i) p3[o * S2 + i] = __float2bfloat16_rn(wl[o * H + i]);
+        pb[2 * H + o] = bl[o];
+    }
+    for (int i = 0; i < H; ++i) p3[A * S2 + i] = __float2bfloat16_rn(wv[i]);
+    pb[2 * H + A] = bv[0];
+    return MAPF_OK;
+}
+
+int mapf_cte_policy_act(const mapf_cte_policy_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    if (!cte_policy_shape_ok(a->cells, a->num_agents))
+        return fail(MAPF_ERR_UNSUPPORTED, "cte policy: cells %d / num_agents %d outside 1..%d / 1..%d", a->cells,
+                    a->num_agents, MAPF_CTE_POLICY_MAX_CELLS, MAPF_MAX_AGENTS);
+    if (a->num_envs < 1 || !a->obs_grid || !a->action_mask || !a->weights)
+        return fail(MAPF_ERR_INVALID_ARG, "cte policy: num_envs >= 1, obs_grid, action_mask and weights are required");
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "cte policy: reserved is %d, must be 0", a->reserved);
+    int ndev = 0, dev = 0, sms = 0, per_sm = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int threads = mapf::CTE_THREADS, warps = threads / 32;
+    const size_t smem = (size_t)mapf::cte_weight_bytes(a->cells, a->num_agents) + (size_t)warps * mapf::CTE_WARP_BYTES;
+    const auto kernel = mapf::mapf_cte_policy_act_kernel;
+    CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    if (per_sm < 1) return fail(MAPF_ERR_UNSUPPORTED, "cte policy: %zu bytes of shared memory do not fit one SM", smem);
+    // resident blocks load the weights once and loop over the 32-env tiles
+    const long long tiles = ((long long)a->num_envs + 31) / 32;
+    long long blocks = (tiles + warps - 1) / warps;
+    if (blocks > (long long)sms * per_sm) blocks = (long long)sms * per_sm;
+    kernel<<<(unsigned)blocks, threads, smem, static_cast<cudaStream_t>(stream)>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
 
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
              float *ret, int32_t T, int64_t B, int32_t N, float gamma, float lam, void *stream) {

@@ -157,6 +157,23 @@ __device__ __forceinline__ void pol_feature_row(__nv_bfloat16 *xs, const uint32_
     }
 }
 
+// the second ReLU layer of an m-tile: A fragments h1 (64 wide) -> A fragments h2 of the next GEMM (w2 [64][72], b2[64])
+__device__ __forceinline__ void pol_layer2(const uint32_t (&h1)[POL_H / 16][4], const __nv_bfloat16 *w2, const float *b2,
+                                           int g, int t, uint32_t (&h2)[POL_H / 16][4]) {
+#pragma unroll
+    for (int j = 0; j < POL_H / 8; ++j) {
+        const float2 bb = *reinterpret_cast<const float2 *>(b2 + 8 * j + 2 * t);
+        float d[4] = {bb.x, bb.y, bb.x, bb.y};
+#pragma unroll
+        for (int kk = 0; kk < POL_H / 16; ++kk) {
+            const uint32_t *wb = reinterpret_cast<const uint32_t *>(w2 + (8 * j + g) * POL_W2_STRIDE + 16 * kk + 2 * t);
+            mma_bf16_16816(d, h1[kk], wb[0], wb[4]);
+        }
+        h2[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);
+        h2[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);
+    }
+}
+
 // the two ReLU layers of the 16-row m-tile whose rows are row0 and row0 + 8: features xs -> A fragments of the next
 // GEMM (bias = b1[64] b2[64])
 template <int KC1>
@@ -184,19 +201,7 @@ __device__ __forceinline__ void pol_trunk(const __nv_bfloat16 *xs, const __nv_bf
         h1[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);   // row g,   cols 8j + 2t, +1
         h1[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);   // row g+8
     }
-    // ------------------------------------------------------------ layer 2
-#pragma unroll
-    for (int j = 0; j < POL_H / 8; ++j) {
-        const float2 bb = *reinterpret_cast<const float2 *>(bias + POL_H + 8 * j + 2 * t);
-        float d[4] = {bb.x, bb.y, bb.x, bb.y};
-#pragma unroll
-        for (int kk = 0; kk < POL_H / 16; ++kk) {
-            const uint32_t *wb = reinterpret_cast<const uint32_t *>(w2 + (8 * j + g) * POL_W2_STRIDE + 16 * kk + 2 * t);
-            mma_bf16_16816(d, h1[kk], wb[0], wb[4]);
-        }
-        h2[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[0], d[1]);
-        h2[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[2], d[3]);
-    }
+    pol_layer2(h1, w2, bias + POL_H, g, t, h2);
 }
 
 // heads: columns 0..4 logits, 5 value (w3 [8][72], b3[8]) of the m-tile -> os[32][8]
@@ -211,6 +216,20 @@ __device__ __forceinline__ void pol_heads(const uint32_t (&hf)[POL_H / 16][4], c
     }
     *reinterpret_cast<float2 *>(os + row0 * 8 + 2 * t) = make_float2(d[0], d[1]);
     *reinterpret_cast<float2 *>(os + (row0 + 8) * 8 + 2 * t) = make_float2(d[2], d[3]);
+}
+
+// the policy kernels' draw of one agent from the unnormalised probabilities pr (sum = their sum): inverse CDF of one
+// Philox word keyed by (key, env_id), counter (counter, agent)
+__device__ __forceinline__ int pol_draw(unsigned long long key, long long env_id, unsigned long long counter, int agent,
+                                        const float (&pr)[5], float sum) {
+    Philox ph(key, env_id);
+    const uint4 x = ph((uint32_t)counter, (uint32_t)(counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
+    const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
+    int act = 0;
+    float cum = pr[0];
+#pragma unroll
+    for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
+    return act;
 }
 
 // one agent per lane (call for lane < na): mask, stable softmax, then the action: with GREEDY the first index of the
@@ -243,12 +262,7 @@ __device__ __forceinline__ void pol_sample(const Args &a, const float *os, const
     } else {
         const unsigned env = (unsigned)((unsigned long long)ag / (unsigned)N);   // B * N < 2^32 in any batch that fits a GPU
         const int agent = (int)(ag - (long long)env * N);
-        Philox ph(a.seed ^ tag, a.env_id_base + env);
-        const uint4 x = ph((uint32_t)a.counter, (uint32_t)(a.counter >> 32), (uint32_t)agent, 0x53414D50u /* "SAMP" */);
-        const float u = ((float)(x.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;   // uniform in (0, sum)
-        float cum = pr[0];
-#pragma unroll
-        for (int k = 1; k < 5; ++k) { if (u >= cum) act = k; cum += pr[k]; }
+        act = pol_draw(a.seed ^ tag, a.env_id_base + env, a.counter, agent, pr, sum);
     }
     if (a.actions) a.actions[ag] = (int8_t)act;
     if (a.actions64) a.actions64[ag] = (long long)act;

@@ -360,12 +360,20 @@ def ppo_loss(lg, v, acts, old_logp, adv, ret, *, clip: float, vf_coeff: float, e
     r % num_agents, the same number of rows per agent) and every mean is taken per agent, then summed over the agents:
     N independent learners, agent j's parameters getting agent j's mean loss's gradient."""
     dist = torch.distributions.Categorical(logits=lg)
-    lp = dist.log_prob(acts)
+    return ppo_objective(dist.log_prob(acts), dist.entropy(), v, old_logp, adv, ret, clip=clip, vf_coeff=vf_coeff,
+                         entropy_coeff=entropy_coeff, num_agents=num_agents)
+
+
+def ppo_objective(lp, entropy, v, old_logp, adv, ret, *, clip: float, vf_coeff: float, entropy_coeff: float,
+                  num_agents: int | None = None):
+    """:func:`ppo_loss` over precomputed log-probabilities ``lp`` and entropies ``entropy`` of the taken actions [...]:
+    the clipped surrogate, plus ``vf_coeff`` times the value loss, minus ``entropy_coeff`` times the mean entropy (for
+    a joint action, ``lp`` and ``entropy`` are the sums over its independent parts)."""
     ratio = torch.exp(lp - old_logp)
     surr = torch.min(ratio * adv, torch.clamp(ratio, 1 - clip, 1 + clip) * adv)
     mean = (lambda x: x.mean()) if num_agents is None else (lambda x: x.reshape(-1, num_agents).mean(0).sum())  # noqa: E731
     vf = mean((v - ret).pow(2))
-    ent = mean(dist.entropy())
+    ent = mean(entropy)
     policy_loss = -mean(surr)
     loss = policy_loss + vf_coeff * vf - entropy_coeff * ent
     return loss, {"loss": float(loss.detach()), "vf_loss": float(vf.detach()), "entropy": float(ent.detach()),

@@ -150,12 +150,17 @@ class BatchedCteEnv:
             self.goals.copy_(torch.as_tensor(np.asarray(goals), dtype=torch.int16).reshape(self.B, self.N, 2))
         elif not self.deterministic:
             self._draw(None if mask is None else m)
+        self._reset_launch(m, self._args)
+        return self.flat_obs
+
+    def _reset_launch(self, m, args):
+        """Positions of the envs of ``m`` (uint8 [B] device tensor) back to their starts, then ``mapf_cte_reset`` with
+        the output pointers of ``args`` (the env's own, or a rollout's rows)."""
         torch.where(m.bool().view(self.B, 1, 1), self.starts, self.positions, out=self.positions)
         self._reset_mask = m   # outlives the launch (replaced by the next reset, stream-ordered)
-        self._args.reset_mask = m.data_ptr()
-        nat.check(self._lib.mapf_cte_reset(C.byref(self._args), self._stream()))
-        self._args.reset_mask = None
-        return self.flat_obs
+        args.reset_mask = m.data_ptr()
+        nat.check(self._lib.mapf_cte_reset(C.byref(args), self._stream()))
+        args.reset_mask = None
 
     def step(self, actions, auto_reset: bool = False):
         """CTE:237-346 for every env.  ``actions``: int8 [B,N] joint actions.  ``auto_reset`` (no reference counterpart,

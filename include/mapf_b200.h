@@ -501,6 +501,44 @@ int mapf_lstm_policy_act(const mapf_lstm_policy_args *args, void *stream);
  * agent changes. */
 int mapf_policy_act_per_agent(const mapf_policy_args *args, void *stream);
 int mapf_lstm_policy_act_per_agent(const mapf_lstm_policy_args *args, void *stream);
+
+/* The centralised (CTE) policy over the single-agent view (cte_rollout.CteActionMaskPolicy, the restatement of
+ * models/action_mask_model_single.py): the R*C grid codes of mapf_cte_step / mapf_cte_reset's obs_grid as float ->
+ * Linear(R*C, 64)-ReLU-Linear(64, 64)-ReLU -> 5N logits + value, logits + log(mask + 1e-6) element by element over the
+ * 5N action mask, then for every agent an independent masked 5-way draw (RLlib's multi-categorical over
+ * MultiDiscrete([5] * N)), in one launch per step: bf16 tensor-core GEMMs with f32 accumulation, W1 resident in shared
+ * memory.  Each agent's draw is an inverse CDF of one Philox word keyed by (seed ^ "CTEP", env_id_base + env), counter
+ * (counter, agent): a stream of its own, distinct from mapf_policy_act's and mapf_lstm_policy_act's.  logp is the f32
+ * sum of the agents' log-probabilities, added in agent order.
+ * Supported: 1 <= num_agents <= MAPF_MAX_AGENTS and 1 <= cells <= MAPF_CTE_POLICY_MAX_CELLS (MAPF_ERR_UNSUPPORTED
+ * otherwise); null inputs, num_envs < 1 and reserved != 0 give MAPF_ERR_INVALID_ARG; all before any device work. */
+#define MAPF_CTE_POLICY_MAX_CELLS 1024
+
+typedef struct mapf_cte_policy_args {
+    int32_t num_envs, num_agents;
+    int32_t cells;                 /* R * C */
+    int32_t reserved;              /* must be 0 */
+    uint64_t seed;
+    uint64_t counter;
+    int64_t env_id_base;
+    const uint8_t *obs_grid;       /* [B, cells] device, the CTE env's grid codes */
+    const int8_t *action_mask;     /* [B, 5N] */
+    const void *weights;           /* device copy of the block written by mapf_cte_policy_pack_weights */
+    int8_t *actions;               /* [B, N] joint action (feeds mapf_cte_step), may be NULL */
+    int64_t *actions64;            /* [B, N] the same as int64, may be NULL */
+    float *logp;                   /* [B] joint log-probability, may be NULL */
+    float *value;                  /* [B] value head, may be NULL */
+    float *logits_out;             /* [B, N, 5] masked logits, may be NULL */
+} mapf_cte_policy_args;
+
+/* Bytes of the packed CTE policy weight block (negative = unsupported cells / num_agents). */
+int64_t mapf_cte_policy_weights_nbytes(int32_t cells, int32_t num_agents);
+/* HOST float32 weights in torch's Linear layout (w1 [64, cells], w2 [64, 64], w_logits [5N, 64], w_value [1, 64]) ->
+ * HOST packed block (bf16 weights, padded; f32 biases). */
+int mapf_cte_policy_pack_weights(int32_t cells, int32_t num_agents, const float *w1, const float *b1, const float *w2,
+                                 const float *b2, const float *w_logits, const float *b_logits, const float *w_value,
+                                 const float *b_value, void *packed_host);
+int mapf_cte_policy_act(const mapf_cte_policy_args *args, void *stream);
 /* Per-step bookkeeping of the batched evaluator (main.py:test_trained_model, one episode per env, no auto-reset), in
  * one launch after mapf_step (and after mapf_occupancy_accumulate, which reads `active` before this call clears it).
  * For every env with active[b] != 0: episode_reward[b] += sum of the agents' rewards (main.py:251), agent_reward[b,n]

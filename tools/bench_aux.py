@@ -63,6 +63,38 @@ def per_agent_entry(shared_fn, per_agent_fn, one_agent_fn, agents, bytes_per_age
             "agent_steps_per_s": agents / s}
 
 
+def cte_policy_act_entry(B, N=16):
+    """The fused centralised CTE policy (mapf_cte_policy_act) at 65 536 envs x 16 agents on the 32x32 benchmark map,
+    over a rotation of 4 env batches (4 x 72 MB of grid codes and masks: more than L2)."""
+    from dl_reference_models_b200.cte_rollout import CteActionMaskPolicy
+
+    ccfg = {"grid": maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32), "num_agents": N, "steps_per_episode": 256,
+            "seed": 999}
+    envs = [BatchedCteEnv(ccfg, B) for _ in range(4)]
+    for e in envs:
+        e.reset()
+    cells = envs[0].R * envs[0].C
+    policy = CteActionMaskPolicy(cells, N).cuda()
+    fused = [policy_kernels.FusedCtePolicy(policy, e, env_id_base=k * B) for k, e in enumerate(envs)]
+    i = [0]
+
+    def act():
+        fused[i[0] % 4].act()
+        i[0] += 1
+
+    s = timed(act, 200)
+    # byte / FLOP model per env: grid codes R*C + mask 5N in; int8 + int64 actions, joint logp, value out.  GEMMs
+    # without padding: R*C x 64, 64 x 64, 64 x (5N + 1)
+    nbytes = (cells + 5 * N) + (N + 8 * N + 4 + 4)
+    flops = 2 * (cells * 64 + 64 * 64 + 64 * (5 * N + 1))
+    hbm_tbs, bf16_tflops = 6.45, 2250.0   # SURVEY 8d measured copy bandwidth; dense bf16 data-sheet rate (tcgen05)
+    gbps, tflops = nbytes * B / s / 1e9, flops * B / s / 1e12
+    return {"us_per_launch": s * 1e6, "envs": B, "agents": N, "cells": cells, "bytes_per_env": nbytes,
+            "flops_per_env": flops, "GBps": gbps, "TFLOPs": tflops, "env_steps_per_s": B / s,
+            "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3), "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops,
+            "hbm_floor_us": nbytes * B / (hbm_tbs * 1e12) * 1e6}
+
+
 def main():
     res = {}
     B, N = 65536, 16
@@ -191,6 +223,8 @@ def main():
     s = timed(lambda: cte.step(acts), 100)
     res["cte_step"] = {"us_per_launch": s * 1e6, "env_steps_per_s": B / s, "agent_steps_per_s": 4 * B / s,
                        "GBps": (cte.D * 4 + 200 + 20 + 40) * B / s / 1e9}
+    del cte
+    res["cte_policy_act"] = cte_policy_act_entry(B)
     try:
         import subprocess
 
