@@ -48,6 +48,10 @@ constexpr int ENV_ROW_PAD = 2;         // zero rows around the owner masks of th
 
 // stage row of one env and quad: 4 * V2 observation bytes + 20 action-mask bytes, odd word stride
 __host__ __device__ constexpr int env_stage_stride(int V2) { return ((4 * V2 + 20 + 3) / 4) | 1; }
+// the stage also lands the 64-byte env-word rows of the warp's 32 envs after the walk: at least 2 KB
+__host__ __device__ constexpr int env_stage_bytes(int V2) {
+    return 32 * env_stage_stride(V2) * 4 > 32 * 64 ? 32 * env_stage_stride(V2) * 4 : 32 * 64;
+}
 
 struct EnvLayout {
     int tables_bytes;  // multiple of 16
@@ -67,7 +71,7 @@ __host__ __device__ inline EnvLayout make_env_layout(int N, int R, int C, int SR
     if (N > E.board_rows) E.board_rows = N;
     E.board_rows += 2 * ENV_ROW_PAD;
     E.nq = (N + 3) / 4;
-    int w = 32 * env_stage_stride(V2) * 4;   // stage: one row per lane
+    int w = env_stage_bytes(V2);             // stage: one row per lane
     w += E.board_rows * 32 * 4;              // occupancy boards: u32 [row][lane]
     w += E.board_rows * 32 * 4;              // goal boards: u32 [row][lane]
     w += 4 * E.nq * 32 * 4;                  // agent records: u32 [agent][lane]
@@ -300,7 +304,7 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
     constexpr uint32_t M4 = VM << 2;          // a window row, pre-scaled by 4 (byte offset into the tables)
     constexpr int OBS_W = V2;                 // observation words per quad and env (4 * V2 bytes)
     constexpr int STRIDE = env_stage_stride(V2);
-    constexpr int STAGE_BYTES = 32 * STRIDE * 4;
+    constexpr int STAGE_BYTES = env_stage_bytes(V2);
     constexpr int CTR = SR * V + SR;
     constexpr int PADR = ENV_ROW_PAD;
     using WB = typename WinBits<V>::type;
@@ -549,7 +553,6 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
         if (use_ring) ring_n = ldq16<VEC>(p.lock_dist, ((size_t)(ok ? env : 0) * p.lw + slot_next) * N + i0, i0, N, ok);
     };
     load_lock(0);
-    int4 w0 = make_int4(0, 0, 0, 0), w1 = w0, w2 = w0, w3 = w0;   // the rest of the env words: needed behind the walk
     for (int q = 0; q < NQ; ++q) {
         const int i0 = 4 * q;
         uint32_t rv4[4];
@@ -687,10 +690,6 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
                        make_uint2(ds[0] | (ds[1] << 16), ds[2] | (ds[3] << 16)));
         }
         if (q + 1 < NQ) load_lock(i0 + 4);
-        else if (ok) {
-            const int4 *ew4 = p.env_words + (size_t)env * 4;
-            w0 = ew4[0]; w1 = ew4[1]; w2 = ew4[2]; w3 = ew4[3];
-        }
         // Phase B -- the byte rows of the four agents into my stage row (the table look-ups feeding it were issued in
         // phase A and, being loads from immutable tables, are free to complete anywhere in between).
         uint32_t carry = 0;
@@ -803,14 +802,22 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
         __syncwarp();
     }
 
-    // ---------------------------------------------------------------- the rest of the env words
-    int step_count = w0.x + 1;  // ENV:475
-    int lock_prev = w0.z, goals_total = w0.w;
-    int blocking_total = w1.x, dl_events = w1.y, ll_events = w1.z, dl_steps = w1.w;
-    int ll_steps = w2.x;
-    uint32_t rng_counter = (uint32_t)w2.y;
-    int ep_return_x2 = w2.z, wfg_steps = w2.w;
-    int episodes = w3.x;
+    // ---------------------------------------------------------------- the rest of the env words: needed behind the epilogue
+    // Copied global -> shared with cp.async: no registers held while in flight (a row loaded into registers during the
+    // walk stays live through every quad and spills).  16 bytes k of my env's row at ew_s + 512 k: a slot in the stage, which is
+    // dead from here -- the __syncwarp closing the last flush says every lane has drained it -- to the next step's phase
+    // B, behind the __syncwarp that ends this step.  Only this lane touches its slot, after its own wait.
+    const uint32_t ew_s = (uint32_t)__cvta_generic_to_shared(stage_w) + (uint32_t)lane * 16u;
+    {
+        const int4 *src = p.env_words + (size_t)(ok ? env : 0) * 4;
+#pragma unroll
+        for (int k = 0; k < 4; ++k)   // lanes beyond the batch land zeros, as the register loads they replace left them
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(ew_s + 512u * k), "l"(src + k),
+                         "r"(ok ? 16 : 0) : "memory");
+        asm volatile("cp.async.commit_group;" ::: "memory");
+    }
+    int *ew_slot = reinterpret_cast<int *>(stage_w) + lane * 4;   // word w at ew_slot[128 * (w >> 2) + (w & 3)]
+    auto ew_ld = [&](int word) -> int { return ew_slot[128 * (word >> 2) + (word & 3)]; };
 
     // ---------------------------------------------------------------- injected co-location (ENV:658-666), kept off the walk
     // Replays who owns which cell through the moves of this step (ENV:523: a leaving agent clears the owner for
@@ -845,7 +852,6 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
     // ---------------------------------------------------------------- lifelong goal reassignment (ENV:284-304, 547-556)
     if (kLock) lock_head = slot_next;
     const int arrivals = __popc(gstep_m);
-    goals_total += arrivals;  // lifelong: every arrival; else first arrivals (ENV:545,562)
     const uint32_t pend = kLifelong ? gstep_m : 0u;
     const bool reassigned = pend != 0;
     {
@@ -854,13 +860,16 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
         // together -- lane = agent for the roll-back / re-emission, lane = map row for the candidate scan --
         // instead of 32 lanes re-walking their own env for the sake of one.
         unsigned rw = __ballot_sync(full, pend != 0);
+        // the Philox counters of the envs served here come from the env-word slots (each lane reads and updates its own)
+        if (rw) asm volatile("cp.async.wait_all;" ::: "memory");
+        const uint32_t rng_counter0 = rw ? (uint32_t)ew_ld(MAPF_W_RNG_COUNTER) : 0u;
         while (rw) {
             const int e = __ffs(rw) - 1;
             rw &= rw - 1;
             uint32_t pe = __shfl_sync(full, pend, e);
             const uint32_t mv_e = __shfl_sync(full, moved_m, e), bp_e = __shfl_sync(full, bprev_m, e);
             const uint32_t solo_e = __shfl_sync(full, degen ? solo_m : 0xFFFFFFFFu, e);
-            const uint32_t rc_e = __shfl_sync(full, rng_counter, e);
+            const uint32_t rc_e = __shfl_sync(full, rng_counter0, e);
             const int slot_new_e = __shfl_sync(full, slot_new, e), slot_next_e = __shfl_sync(full, slot_next, e);
             const bool use_ring_e = __shfl_sync(full, (int)use_ring, e) != 0;
             const long long eg = p.env_id_base + (long long)(env0 + e);
@@ -948,7 +957,10 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
                 const bool ctr2 = !((solo_e >> lane) & 1u) && ((occ_e[(code >> 5) * 32] >> (code & 31u)) & 1u);
                 emit_final(abe, oo, sctr, eg, occ_e, goal_e, code, gcode, (bp_e >> lane) & 1u, ctr2);
             }
-            if (lane == e) { rng_counter += rng_inc; errs |= err_e; ongoal_m |= ongoal_fix; }
+            if (lane == e) {
+                ew_slot[128 * (MAPF_W_RNG_COUNTER >> 2) + (MAPF_W_RNG_COUNTER & 3)] = (int)(rc_e + rng_inc);
+                errs |= err_e; ongoal_m |= ongoal_fix;
+            }
             __syncwarp();
         }
     }
@@ -1086,6 +1098,16 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
         }
         wf_m = alive;
     }
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    int step_count = ew_ld(MAPF_W_STEP_COUNT) + 1;  // ENV:475
+    int lock_prev = ew_ld(MAPF_W_LOCK_PREV);
+    int goals_total = ew_ld(MAPF_W_GOALS_TOTAL) + arrivals;  // lifelong: every arrival; else first arrivals (ENV:545,562)
+    int blocking_total = ew_ld(MAPF_W_BLOCKING_TOTAL), dl_events = ew_ld(MAPF_W_DEADLOCK_EVENTS);
+    int ll_events = ew_ld(MAPF_W_LIVELOCK_EVENTS), dl_steps = ew_ld(MAPF_W_DEADLOCK_STEPS);
+    int ll_steps = ew_ld(MAPF_W_LIVELOCK_STEPS);
+    uint32_t rng_counter = (uint32_t)ew_ld(MAPF_W_RNG_COUNTER);
+    int ep_return_x2 = ew_ld(MAPF_W_EPISODE_RETURN_X2), wfg_steps = ew_ld(MAPF_W_WFG_CYCLE_STEPS);
+    int episodes = ew_ld(MAPF_W_EPISODES);
     const bool wf_any = wf_m != 0;
     wfg_steps += wf_any;
     const int blocking_step = __popc(blocking_m);
@@ -1282,7 +1304,7 @@ __global__ void __launch_bounds__(448, 1) mapf_step_env_kernel(const KParams p, 
         ew4[0] = make_int4(step_count, lock_count, lock_prev, goals_total);
         ew4[1] = make_int4(blocking_total, dl_events, ll_events, dl_steps);
         ew4[2] = make_int4(ll_steps, (int)rng_counter, ep_return_x2, wfg_steps);
-        ew4[3] = make_int4(episodes, lock_head, w3.z, w3.w);
+        ew4[3] = make_int4(episodes, lock_head, ew_ld(MAPF_W_RESERVED1), ew_ld(MAPF_W_RESERVED2));
     }
     __syncwarp();
     }  // inner steps
