@@ -18,7 +18,8 @@ CSRC = PKG / "csrc"
 LIB_PATH = Path(os.environ.get("MAPF_B200_LIB", PKG / "libmapf_b200.so"))
 SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_kernel.cuh", CSRC / "mapf_pair_kernel.cuh", CSRC / "mapf_cte_kernel.cuh", CSRC / "mapf_policy_kernel.cuh",
            CSRC / "mapf_policy_lstm_kernel.cuh", CSRC / "mapf_eval_kernel.cuh", CSRC / "mapf_cte_policy_kernel.cuh",
-           CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
+           CSRC / "mapf_cte_lstm_policy_kernel.cuh", CSRC / "mapf_cte_trunk.inc",
+           CSRC / "mapf_cte_heads.inc", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
 MAX_AGENTS = 32
@@ -126,6 +127,17 @@ class MapfCtePolicyArgs(C.Structure):
         ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
     ] + [(k, C.c_void_p) for k in (
         "obs_grid", "action_mask", "weights", "actions", "actions64", "logp", "value", "logits_out")]
+
+
+class MapfCteLstmPolicyArgs(C.Structure):
+    """mapf_cte_lstm_policy_args of include/mapf_b200.h (fused recurrent centralised CTE policy + per-agent draws)."""
+
+    _fields_ = [
+        ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("cells", C.c_int32), ("reserved", C.c_int32),
+        ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
+    ] + [(k, C.c_void_p) for k in (
+        "obs_grid", "action_mask", "prev_terminated", "prev_truncated", "prev_action", "prev_reward", "h_in", "c_in",
+        "h_out", "c_out", "trunk", "weights", "actions", "actions64", "logp", "value", "logits_out")]
 
 
 class MapfEvalArgs(C.Structure):
@@ -241,13 +253,18 @@ def lib():
     L.mapf_cte_policy_weights_nbytes.restype = i64
     L.mapf_cte_policy_pack_weights.argtypes = [i32, i32] + [vp] * 9
     L.mapf_cte_policy_act.argtypes = [C.POINTER(MapfCtePolicyArgs), vp]
+    L.mapf_cte_lstm_policy_weights_nbytes.argtypes = [i32, i32]
+    L.mapf_cte_lstm_policy_weights_nbytes.restype = i64
+    L.mapf_cte_lstm_policy_pack_weights.argtypes = [i32, i32] + [vp] * 13
+    L.mapf_cte_lstm_policy_act.argtypes = [C.POINTER(MapfCteLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
     L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
         if name not in ("mapf_version", "mapf_last_error", "mapf_launch_count", "mapf_policy_weights_nbytes",
-                        "mapf_lstm_policy_weights_nbytes", "mapf_cte_policy_weights_nbytes"):
+                        "mapf_lstm_policy_weights_nbytes", "mapf_cte_policy_weights_nbytes",
+                        "mapf_cte_lstm_policy_weights_nbytes"):
             getattr(L, name).restype = C.c_int
     _lib = L
     return L
@@ -266,6 +283,7 @@ EXPORTS = (
     "mapf_lstm_policy_weights_nbytes", "mapf_lstm_policy_pack_weights", "mapf_lstm_policy_act", "mapf_eval_accumulate",
     "mapf_policy_act_per_agent", "mapf_lstm_policy_act_per_agent",
     "mapf_cte_policy_weights_nbytes", "mapf_cte_policy_pack_weights", "mapf_cte_policy_act",
+    "mapf_cte_lstm_policy_weights_nbytes", "mapf_cte_lstm_policy_pack_weights", "mapf_cte_lstm_policy_act",
 )
 
 

@@ -6,6 +6,7 @@
 #include "mapf_pair_kernel.cuh"
 #include "mapf_cte_kernel.cuh"
 #include "mapf_cte_policy_kernel.cuh"
+#include "mapf_cte_lstm_policy_kernel.cuh"
 #include "mapf_policy_kernel.cuh"
 #include "mapf_policy_lstm_kernel.cuh"
 #include "mapf_eval_kernel.cuh"
@@ -1816,6 +1817,91 @@ int mapf_cte_policy_act(const mapf_cte_policy_args *a, void *stream) {
     if (blocks > (long long)sms * per_sm) blocks = (long long)sms * per_sm;
     kernel<<<(unsigned)blocks, threads, smem, static_cast<cudaStream_t>(stream)>>>(*a);
     CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int64_t mapf_cte_lstm_policy_weights_nbytes(int32_t cells, int32_t num_agents) {
+    if (!cte_policy_shape_ok(cells, num_agents))
+        return fail(MAPF_ERR_UNSUPPORTED, "cte lstm policy: cells %d / num_agents %d outside 1..%d / 1..%d", cells,
+                    num_agents, MAPF_CTE_POLICY_MAX_CELLS, MAPF_MAX_AGENTS);
+    return mapf::ctel_trunk_bytes(cells) + mapf::ctel_step_bytes(num_agents);
+}
+
+int mapf_cte_lstm_policy_pack_weights(int32_t cells, int32_t num_agents, const float *w1, const float *b1, const float *w2,
+                                      const float *b2, const float *w_ih, const float *w_hh, const float *b_ih,
+                                      const float *b_hh, const float *wl, const float *bl, const float *wv, const float *bv,
+                                      void *packed) {
+    const int64_t nbytes = mapf_cte_lstm_policy_weights_nbytes(cells, num_agents);
+    if (nbytes < 0) return (int)nbytes;
+    if (!w1 || !b1 || !w2 || !b2 || !w_ih || !w_hh || !b_ih || !b_hh || !wl || !bl || !wv || !bv || !packed)
+        return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    const int s1 = mapf::cte_s1(cells), H = mapf::POL_H, S2 = mapf::POL_W2_STRIDE, A = 5 * num_agents;
+    const int SG = mapf::ctel_sg(num_agents), KH = mapf::ctel_kh(num_agents), KI = H + A + 1;
+    memset(packed, 0, (size_t)nbytes);
+    // trunk part: w1 [64][S1] | w2 [64][72] | b1 b2
+    __nv_bfloat16 *p1 = static_cast<__nv_bfloat16 *>(packed), *p2 = p1 + H * s1;
+    float *pb = reinterpret_cast<float *>(p2 + H * S2);
+    for (int o = 0; o < H; ++o) {
+        for (int i = 0; i < cells; ++i) p1[(size_t)o * s1 + i] = __float2bfloat16_rn(w1[(size_t)o * cells + i]);
+        for (int i = 0; i < H; ++i) p2[o * S2 + i] = __float2bfloat16_rn(w2[o * H + i]);
+        pb[o] = b1[o];
+        pb[H + o] = b2[o];
+    }
+    // step part: wg [256][SG] | w3 [8 NT][72] | bg[256] wr[256] b3[8 NT]
+    const int NT = mapf::cte_head_tiles(num_agents);
+    __nv_bfloat16 *pg = reinterpret_cast<__nv_bfloat16 *>(static_cast<unsigned char *>(packed) + mapf::ctel_trunk_bytes(cells));
+    __nv_bfloat16 *p3 = pg + 4 * H * SG;
+    float *pbg = reinterpret_cast<float *>(p3 + 8 * NT * S2), *pwr = pbg + 4 * H, *pb3 = pbg + 8 * H;
+    for (int o = 0; o < 4 * H; ++o) {   // [W_ih y and one-hot columns | zero to 64 + KH | W_hh]; reward column in f32
+        for (int i = 0; i < H + A; ++i) pg[(size_t)o * SG + i] = __float2bfloat16_rn(w_ih[(size_t)o * KI + i]);
+        for (int i = 0; i < H; ++i) pg[(size_t)o * SG + H + KH + i] = __float2bfloat16_rn(w_hh[o * H + i]);
+        pwr[o] = w_ih[(size_t)o * KI + H + A];
+        pbg[o] = b_ih[o] + b_hh[o];
+    }
+    for (int o = 0; o < A; ++o) {   // head rows: 5N logits, then the value
+        for (int i = 0; i < H; ++i) p3[o * S2 + i] = __float2bfloat16_rn(wl[o * H + i]);
+        pb3[o] = bl[o];
+    }
+    for (int i = 0; i < H; ++i) p3[A * S2 + i] = __float2bfloat16_rn(wv[i]);
+    pb3[A] = bv[0];
+    return MAPF_OK;
+}
+
+int mapf_cte_lstm_policy_act(const mapf_cte_lstm_policy_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    if (!cte_policy_shape_ok(a->cells, a->num_agents))
+        return fail(MAPF_ERR_UNSUPPORTED, "cte lstm policy: cells %d / num_agents %d outside 1..%d / 1..%d", a->cells,
+                    a->num_agents, MAPF_CTE_POLICY_MAX_CELLS, MAPF_MAX_AGENTS);
+    if (a->num_envs < 1 || !a->obs_grid || !a->action_mask || !a->weights || !a->trunk)
+        return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: num_envs >= 1, obs_grid, action_mask, trunk and weights are required");
+    if (!a->prev_action || !a->prev_reward || !a->h_in || !a->c_in)
+        return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: prev_action, prev_reward, h_in and c_in are required");
+    if (!a->h_out != !a->c_out)
+        return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: h_out and c_out are given together (both NULL = state not advanced)");
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: reserved is %d, must be 0", a->reserved);
+    int ndev = 0, dev = 0, sms = 0, per_sm[2] = {0, 0};
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    void (*const kernels[2])(const mapf_cte_lstm_policy_args) = {mapf::mapf_cte_lstm_trunk_kernel, mapf::mapf_cte_lstm_step_kernel};
+    const int threads[2] = {mapf::CTE_THREADS, mapf::CTEL_THREADS};
+    const size_t smem[2] = {(size_t)mapf::ctel_trunk_bytes(a->cells) + (size_t)(mapf::CTE_THREADS / 32) * mapf::CTE_WARP_BYTES,
+                            (size_t)mapf::ctel_step_bytes(a->num_agents) + (size_t)(mapf::CTEL_THREADS / 32) * mapf::CTEL_WARP_BYTES};
+    for (int k = 0; k < 2; ++k) {
+        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernels[k]), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[k]));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[k], kernels[k], threads[k], smem[k]));
+        if (per_sm[k] < 1) return fail(MAPF_ERR_UNSUPPORTED, "cte lstm policy: %zu bytes of shared memory do not fit one SM", smem[k]);
+    }
+    // resident blocks load their weights once and loop over the 32-env tiles
+    const long long tiles = ((long long)a->num_envs + 31) / 32;
+    for (int k = 0; k < 2; ++k) {
+        const int warps = threads[k] / 32;
+        long long blocks = (tiles + warps - 1) / warps;
+        if (blocks > (long long)sms * per_sm[k]) blocks = (long long)sms * per_sm[k];
+        kernels[k]<<<(unsigned)blocks, threads[k], smem[k], static_cast<cudaStream_t>(stream)>>>(*a);
+        CUDA_TRY(cudaGetLastError());
+    }
     return MAPF_OK;
 }
 

@@ -19,6 +19,8 @@
 //     an inverse-CDF draw from one Philox word (pol_draw: key (seed ^ "CTEP", env_id_base + env), counter
 //     (counter, agent)), and adds the agent's log-probability to the env's joint one.
 //
+// Layers 1-2 and the heads + draws are written in mapf_cte_trunk.inc / mapf_cte_heads.inc, which the recurrent CTE
+// kernels (mapf_cte_lstm_policy_kernel.cuh) include as well.
 // Supported: 1 <= N <= MAPF_MAX_AGENTS, 1 <= R*C <= MAPF_CTE_POLICY_MAX_CELLS (1024: W1 of 64 x 1056 bf16, 132 KB,
 // stays resident next to the 8 warps' 6 KB staging buffers within the 227 KB of one block).
 #pragma once
@@ -95,116 +97,13 @@ __global__ void __launch_bounds__(CTE_THREADS, 1) mapf_cte_policy_act_kernel(con
     const int W = (al & 15) == 0 ? 16 : (al & 7) == 0 ? 8 : (al & 3) == 0 ? 4 : 1;
     const int nst = (KP + CTE_KC - 1) / CTE_KC;
     const long long ntiles = ((long long)a.num_envs + 31) >> 5;
+    constexpr unsigned long long draw_tag = 0x43544550ull;   // "CTEP"
     for (long long tile = (long long)blockIdx.x * warps + warp; tile < ntiles; tile += (long long)gridDim.x * warps) {
         const long long e0 = tile << 5;
         const int na = a.num_envs - e0 < 32 ? (int)(a.num_envs - e0) : 32;
         const uint8_t *obs = a.obs_grid + e0 * cells;
-        // ------------------------------------------------------------ layer 1: K = R*C, double-buffered staging
-        float d[2][POL_H / 8][4];
-#pragma unroll
-        for (int j = 0; j < POL_H / 8; ++j) {
-            const float2 bb = *reinterpret_cast<const float2 *>(bias + 8 * j + 2 * t);
-#pragma unroll
-            for (int m = 0; m < 2; ++m) { d[m][j][0] = bb.x; d[m][j][1] = bb.y; d[m][j][2] = bb.x; d[m][j][3] = bb.y; }
-        }
-        cte_stage(obs, cells, na, 0, W, stg, lane);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        for (int s = 0; s < nst; ++s) {
-            if (s + 1 < nst) cte_stage(obs, cells, na, (s + 1) * CTE_KC, W, stg + ((s + 1) & 1) * 32 * CTE_STAGE_STRIDE, lane);
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            asm volatile("cp.async.wait_group 1;" ::: "memory");
-            __syncwarp();
-            const uint8_t *st = stg + (s & 1) * 32 * CTE_STAGE_STRIDE;
-#pragma unroll
-            for (int sc = 0; sc < CTE_KC / 32; ++sc) {
-                const int kb = s * CTE_KC + 32 * sc;
-                if (kb >= KP) break;
-                uint32_t af[2][2][4];   // [m-tile][k16 chunk]
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    const uint2 v0 = *reinterpret_cast<const uint2 *>(st + (16 * m + g) * CTE_STAGE_STRIDE + 32 * sc + 8 * t);
-                    const uint2 v1 = *reinterpret_cast<const uint2 *>(st + (16 * m + g + 8) * CTE_STAGE_STRIDE + 32 * sc + 8 * t);
-                    af[m][0][0] = cte_code_pair(v0.x, 0x4140u); af[m][0][1] = cte_code_pair(v1.x, 0x4140u);
-                    af[m][0][2] = cte_code_pair(v0.x, 0x4342u); af[m][0][3] = cte_code_pair(v1.x, 0x4342u);
-                    af[m][1][0] = cte_code_pair(v0.y, 0x4140u); af[m][1][1] = cte_code_pair(v1.y, 0x4140u);
-                    af[m][1][2] = cte_code_pair(v0.y, 0x4342u); af[m][1][3] = cte_code_pair(v1.y, 0x4342u);
-                }
-#pragma unroll
-                for (int j = 0; j < POL_H / 8; ++j) {
-                    const uint4 wb = *reinterpret_cast<const uint4 *>(w1 + (8 * j + g) * S1 + kb + 8 * t);
-#pragma unroll
-                    for (int m = 0; m < 2; ++m) {
-                        mma_bf16_16816(d[m][j], af[m][0], wb.x, wb.y);
-                        mma_bf16_16816(d[m][j], af[m][1], wb.z, wb.w);
-                    }
-                }
-            }
-            __syncwarp();   // every lane is done with this stage before it is refilled
-        }
-        // ------------------------------------------------------------ layer 2
-        uint32_t h2[2][POL_H / 16][4];
-#pragma unroll
-        for (int m = 0; m < 2; ++m) {
-            uint32_t h1[POL_H / 16][4];
-#pragma unroll
-            for (int j = 0; j < POL_H / 8; ++j) {
-                h1[j >> 1][(j & 1) * 2 + 0] = pack_relu_bf16(d[m][j][0], d[m][j][1]);   // row g,   cols 8j + 2t, +1
-                h1[j >> 1][(j & 1) * 2 + 1] = pack_relu_bf16(d[m][j][2], d[m][j][3]);   // row g+8
-            }
-            pol_layer2(h1, w2, bias + POL_H, g, t, h2[m]);
-        }
-        // ------------------------------------------------------------ heads in groups of 5 n8 tiles, then the draws
-        const long long env = e0 + lane;
-        float lsum = 0.f;
-        for (int j0 = 0; j0 < NT; j0 += 5) {
-            for (int j = j0; j < j0 + 5 && j < NT; ++j) {
-                const float2 bb = *reinterpret_cast<const float2 *>(b3 + 8 * j + 2 * t);
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    float o[4] = {bb.x, bb.y, bb.x, bb.y};
-#pragma unroll
-                    for (int kk = 0; kk < POL_H / 16; ++kk) {
-                        const uint32_t *wb = reinterpret_cast<const uint32_t *>(w3 + (8 * j + g) * POL_W2_STRIDE + 16 * kk + 2 * t);
-                        mma_bf16_16816(o, h2[m][kk], wb[0], wb[4]);
-                    }
-                    float *r0 = os + (16 * m + g) * CTE_OS + 8 * (j - j0) + 2 * t, *r1 = r0 + 8 * CTE_OS;
-                    r0[0] = o[0]; r0[1] = o[1]; r1[0] = o[2]; r1[1] = o[3];
-                }
-            }
-            __syncwarp();
-            if (lane < na) {
-                const float *row = os + lane * CTE_OS;
-                const int ag1 = min(N, j0 / 5 * 8 + 8);
-                for (int ag = j0 / 5 * 8; ag < ag1; ++ag) {
-                    const float *lr = row + 5 * ag - 8 * j0;
-                    const long long idx = env * N + ag;
-                    float l[5];
-                    const int8_t *mk = a.action_mask + idx * 5;
-#pragma unroll
-                    for (int k = 0; k < 5; ++k) l[k] = lr[k] + (mk[k] ? 9.99999e-07f : -13.815511f);   // action_mask_model.py:57-61
-                    float mx = l[0];
-#pragma unroll
-                    for (int k = 1; k < 5; ++k) mx = fmaxf(mx, l[k]);
-                    float pr[5], sum = 0.f;
-#pragma unroll
-                    for (int k = 0; k < 5; ++k) { pr[k] = __expf(l[k] - mx); sum += pr[k]; }
-                    const int act = pol_draw(a.seed ^ 0x43544550ull /* "CTEP" */, a.env_id_base + env, a.counter, ag, pr, sum);
-                    float la = l[0];   // l[act] without a local-memory array
-#pragma unroll
-                    for (int k = 1; k < 5; ++k) la = act == k ? l[k] : la;
-                    lsum += la - mx - __logf(sum);
-                    if (a.actions) a.actions[idx] = (int8_t)act;
-                    if (a.actions64) a.actions64[idx] = (long long)act;
-                    if (a.logits_out) {
-#pragma unroll
-                        for (int k = 0; k < 5; ++k) a.logits_out[idx * 5 + k] = l[k];
-                    }
-                }
-                if (a.value && 5 * N >= 8 * j0 && 5 * N < 8 * j0 + 40) a.value[env] = row[5 * N - 8 * j0];
-            }
-            __syncwarp();
-        }
-        if (a.logp && lane < na) a.logp[env] = lsum;
+#include "mapf_cte_trunk.inc"
+#include "mapf_cte_heads.inc"
     }
 }
 

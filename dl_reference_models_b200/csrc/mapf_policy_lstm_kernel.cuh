@@ -42,11 +42,12 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 }
 
 // the four gate tiles i_j, f_j, g_j, o_j of column block j += A chunk kk x [W_ih | 0 | W_hh] rows q * 64 + 8j + g
+// (bf16 row stride sg: LSTM_SG here, the recurrent CTE kernel's own in mapf_cte_lstm_policy_kernel.cuh)
 __device__ __forceinline__ void lstm_gate_chunk(float (&d)[4][4], const uint32_t (&af)[4], const __nv_bfloat16 *wg, int j,
-                                                int kk, int g, int t) {
+                                                int kk, int g, int t, int sg = LSTM_SG) {
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-        const uint32_t *wb = reinterpret_cast<const uint32_t *>(wg + (q * POL_H + 8 * j + g) * LSTM_SG + 16 * kk + 2 * t);
+        const uint32_t *wb = reinterpret_cast<const uint32_t *>(wg + (q * POL_H + 8 * j + g) * sg + 16 * kk + 2 * t);
         mma_bf16_16816(d[q], af, wb[0], wb[4]);
     }
 }

@@ -2,7 +2,8 @@
 env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tensor-core MLP with f32 accumulation), the
 same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a greedy (argmax) mode for evaluation and a
 per-agent variant (one weight set per agent: ``mapf_policy_act_per_agent`` / ``mapf_lstm_policy_act_per_agent``), the
-centralised CTE policy over the single-agent view with one joint draw (``mapf_cte_policy_act``), and GAE as a backwards
+centralised CTE policy over the single-agent view with one joint draw (``mapf_cte_policy_act``) and its recurrent
+variant (``mapf_cte_lstm_policy_act``), and GAE as a backwards
 scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
@@ -339,6 +340,118 @@ class FusedCtePolicy:
         self.counter += 1
         a.counter = self.counter
         nat.check(self._lib.mapf_cte_policy_act(C.byref(a), env._stream()))
+        return self.actions, logp, value
+
+
+class FusedCteRecurrentPolicy:
+    """Inference view of a :class:`cte_rollout.CteRecurrentPolicy` of the reference's shape (trunk 64-64 over the R*C
+    grid codes, LSTM cell 64 fed with the previous joint action and reward, 5N logits + value) on a
+    :class:`single_agent.BatchedCteEnv`: ``mapf_cte_lstm_policy_act``, two launches per call (trunk, then the recurrent
+    step with the heads and the N masked draws).  The module stays the learner's model: call :meth:`refresh` after
+    every optimizer step.  Other shapes, and maps beyond ``MAPF_CTE_POLICY_MAX_CELLS`` cells, are refused
+    (``ValueError``) before any device work.  ``env_id_base`` keys the draws of env e as global env ``env_id_base + e``."""
+
+    def __init__(self, policy, env, seed: int | None = None, env_id_base: int = 0):
+        from .cte_rollout import CteRecurrentPolicy
+
+        cells, N = int(env.R * env.C), int(env.N)
+        if not FusedCteRecurrentPolicy.matches(policy, env):
+            got = (f"a {type(policy).__name__}" if not isinstance(policy, CteRecurrentPolicy) else
+                   f"cells {policy.cells}, {policy.num_agents} agents, hiddens {tuple(policy.hiddens)}, cell "
+                   f"{policy.cell}, previous action {policy.use_prev_action}, previous reward {policy.use_prev_reward}")
+            raise ValueError("the fused recurrent CTE kernel implements CteRecurrentPolicy with hiddens (64, 64), cell 64 "
+                             f"and the previous action and reward at the env's shape (cells {cells}, {N} agents); got {got}")
+        self._lib = nat.lib()
+        n = int(self._lib.mapf_cte_lstm_policy_weights_nbytes(cells, N))
+        if n < 0:
+            raise ValueError(f"the fused recurrent CTE kernel does not support this env: {self._lib.mapf_last_error().decode()}")
+        self.policy, self.env, self.cells = policy, env, cells
+        self._host = np.zeros(n, np.uint8)
+        self._dev = torch.zeros(n, dtype=torch.uint8, device=env.device)
+        B, dev = env.B, env.device
+        self.trunk = torch.empty((B, 64), dtype=torch.bfloat16, device=dev)   # the first launch's output
+        self.actions = torch.zeros((B, N), dtype=torch.int8, device=dev)
+        self.actions64 = torch.zeros((B, N), dtype=torch.int64, device=dev)
+        self.logp = torch.zeros(B, dtype=torch.float32, device=dev)
+        self.value = torch.zeros(B, dtype=torch.float32, device=dev)
+        self.seed = int((env.seed or 0) if seed is None else seed) & (2 ** 64 - 1)
+        self.env_id_base = int(env_id_base)
+        self.counter = 0
+        self.refresh()
+
+    @staticmethod
+    def matches(policy, env) -> bool:
+        """Whether the fused kernels implement ``policy`` at ``env``'s shape: a :class:`cte_rollout.CteRecurrentPolicy`
+        over cells = R*C with num_agents = N, hiddens (64, 64), cell 64, previous action and reward on."""
+        from .cte_rollout import CteRecurrentPolicy
+
+        return (isinstance(policy, CteRecurrentPolicy) and policy.cells == env.R * env.C and policy.num_agents == env.N
+                and tuple(policy.hiddens) == (64, 64) and policy.cell == 64 and policy.use_prev_action
+                and policy.use_prev_reward)
+
+    def refresh(self):
+        """Re-pack the module's current float32 parameters (bf16, padded; the reward column and b_ih + b_hh in f32)
+        and upload them."""
+        f = lambda t: np.ascontiguousarray(t.detach().float().cpu().numpy())  # noqa: E731
+        p = self.policy
+        lin = [m for m in p.trunk if isinstance(m, torch.nn.Linear)]
+        arrs = [f(lin[0].weight), f(lin[0].bias), f(lin[1].weight), f(lin[1].bias), f(p.lstm.weight_ih),
+                f(p.lstm.weight_hh), f(p.lstm.bias_ih), f(p.lstm.bias_hh), f(p.logits.weight), f(p.logits.bias),
+                f(p.value.weight), f(p.value.bias)]
+        nat.check(self._lib.mapf_cte_lstm_policy_pack_weights(self.cells, self.env.N,
+                                                              *[a.ctypes.data_as(C.c_void_p) for a in arrs],
+                                                              C.c_void_p(self._host.ctypes.data)))
+        self._dev.copy_(torch.from_numpy(self._host))
+
+    def args(self, obs_grid, action_mask, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *,
+             state_out=None, actions=None, actions64=None, logp=None, value=None, logits_out=None,
+             num_envs: int | None = None) -> nat.MapfCteLstmPolicyArgs:
+        """The argument block of one call (counter 0; set ``.counter`` before launching).  ``state_out=None``: the
+        state is not advanced; the outputs may be None."""
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+        h, c = state
+        ho, co = (None, None) if state_out is None else state_out
+        return nat.MapfCteLstmPolicyArgs(
+            num_envs=self.env.B if num_envs is None else int(num_envs), num_agents=self.env.N, cells=self.cells,
+            reserved=0, seed=self.seed, counter=0, env_id_base=self.env_id_base,
+            obs_grid=p(obs_grid), action_mask=p(action_mask), prev_terminated=p(prev_terminated),
+            prev_truncated=p(prev_truncated), prev_action=p(prev_action), prev_reward=p(prev_reward), h_in=p(h),
+            c_in=p(c), h_out=p(ho), c_out=p(co), trunk=p(self.trunk), weights=p(self._dev), actions=p(actions),
+            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out))
+
+    def act(self, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *, obs_grid=None,
+            action_mask=None, advance: bool = True, state_out=None, logits_out: torch.Tensor | None = None,
+            logp: torch.Tensor | None = None, value: torch.Tensor | None = None, actions64: torch.Tensor | None = None,
+            num_envs: int | None = None):
+        """One call on ``obs_grid`` (uint8 [B, R*C]; default: the env's) and ``action_mask`` (int8 [B, 5N]; default:
+        the env's).  ``state`` = (h, c) float32 [B, 64]; ``prev_action`` int8 [B, N] (may be :attr:`actions` itself);
+        ``prev_reward`` float64 [B] (the env's ``reward``); ``prev_terminated`` / ``prev_truncated`` uint8 [B] flag the
+        envs whose episode starts at this step (their state, previous action and reward count as zero).  With
+        ``advance`` the new state goes to ``state_out`` (default: ``state``, in place) and the draw to :attr:`actions`;
+        without it the state and :attr:`actions` are left as they are.  Returns (actions int8 [B, N], joint logp [B],
+        value [B]); ``logits_out`` [B, N, 5] receives the masked logits.  ``num_envs``: the first ``num_envs`` rows of
+        every tensor (with the constructor's ``env_id_base``: one shard of a larger batch)."""
+        env = self.env
+        obs_grid = env.obs_grid if obs_grid is None else obs_grid
+        action_mask = env.action_mask if action_mask is None else action_mask
+        B = env.B if num_envs is None else int(num_envs)
+        for name, t, dt, n in (("obs_grid", obs_grid, torch.uint8, B * self.cells),
+                               ("action_mask", action_mask, torch.int8, B * 5 * env.N),
+                               ("h", state[0], torch.float32, B * 64), ("c", state[1], torch.float32, B * 64),
+                               ("prev_action", prev_action, torch.int8, B * env.N),
+                               ("prev_reward", prev_reward, torch.float64, B)):
+            if t.dtype != dt or not t.is_contiguous() or t.device != env.device or t.numel() < n:
+                raise ValueError(f"{name} must be a contiguous {dt} tensor of at least {n} elements on {env.device}")
+        logp = self.logp if logp is None else logp
+        value = self.value if value is None else value
+        actions64 = self.actions64 if actions64 is None else actions64
+        a = self.args(obs_grid, action_mask, state, prev_action, prev_reward, prev_terminated, prev_truncated,
+                      state_out=(state if state_out is None else state_out) if advance else None,
+                      actions=self.actions if advance else None, actions64=actions64, logp=logp, value=value,
+                      logits_out=logits_out, num_envs=B)
+        self.counter += 1
+        a.counter = self.counter
+        nat.check(self._lib.mapf_cte_lstm_policy_act(C.byref(a), env._stream()))
         return self.actions, logp, value
 
 

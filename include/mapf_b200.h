@@ -539,6 +539,55 @@ int mapf_cte_policy_pack_weights(int32_t cells, int32_t num_agents, const float 
                                  const float *b2, const float *w_logits, const float *b_logits, const float *w_value,
                                  const float *b_value, void *packed_host);
 int mapf_cte_policy_act(const mapf_cte_policy_args *args, void *stream);
+
+/* The recurrent centralised (CTE) policy (cte_rollout.CteRecurrentPolicy, the reference's PPO model of
+ * src/agents/ppo.py:67-75 on the single-agent view): the grid codes -> the 64-64 ReLU trunk of mapf_cte_policy_act ->
+ * an LSTM cell of 64 fed with [trunk output | one-hot of the previous joint action (the N five-way one-hots in agent
+ * order) | previous reward] (torch LSTMCell layout, gate rows [i; f; g; o]) -> 5N logits (masked as above) and the
+ * value, both reading the new h -> the N masked draws.  Two launches per call on `stream`: the trunk (bf16 output
+ * into the caller's `trunk` workspace), then the recurrent step (bf16 gate GEMM with f32 accumulation, the reward
+ * term added in f32, c kept in f32) with the heads and the draws.  Each agent's draw is an inverse CDF of one Philox
+ * word keyed by (seed ^ "CTEL", env_id_base + env), counter (counter, agent): a stream of its own; logp is the f32 sum
+ * of the agents' log-probabilities in agent order.  Supported shapes are mapf_cte_policy_act's
+ * (MAPF_ERR_UNSUPPORTED otherwise); null required pointers, num_envs < 1, reserved != 0 and h_out without c_out (or
+ * the reverse) give MAPF_ERR_INVALID_ARG; all before any device work. */
+typedef struct mapf_cte_lstm_policy_args {
+    int32_t num_envs, num_agents;
+    int32_t cells;                  /* R * C */
+    int32_t reserved;               /* must be 0 */
+    uint64_t seed;
+    uint64_t counter;
+    int64_t env_id_base;
+    const uint8_t *obs_grid;        /* [B, cells] device, the CTE env's grid codes */
+    const int8_t *action_mask;      /* [B, 5N] */
+    const uint8_t *prev_terminated; /* [B] or NULL: nonzero = this step starts an episode (h, c, previous action and */
+    const uint8_t *prev_truncated;  /* [B] or NULL     previous reward count as zero)                                */
+    const int8_t *prev_action;      /* [B, N] in 0..4, may alias `actions` (an env's are read before they are written) */
+    const double *prev_reward;      /* [B] the CTE env's own reward type */
+    const float *h_in;              /* [B, 64] LSTM state, float32 */
+    const float *c_in;              /* [B, 64] */
+    float *h_out;                   /* [B, 64] new state, may equal h_in / c_in; both NULL = do not advance the state */
+    float *c_out;                   /* [B, 64]   (h_in, c_in untouched); one NULL without the other is an error */
+    void *trunk;                    /* [B, 64] bf16 workspace: the trunk output, written by the first launch */
+    const void *weights;            /* device copy of the block written by mapf_cte_lstm_policy_pack_weights */
+    int8_t *actions;                /* [B, N] joint action (feeds mapf_cte_step), may be NULL */
+    int64_t *actions64;             /* [B, N] the same as int64, may be NULL */
+    float *logp;                    /* [B] joint log-probability, may be NULL */
+    float *value;                   /* [B] value head, may be NULL */
+    float *logits_out;              /* [B, N, 5] masked logits, may be NULL */
+} mapf_cte_lstm_policy_args;
+
+/* Bytes of the packed recurrent CTE policy weight block (negative = unsupported cells / num_agents). */
+int64_t mapf_cte_lstm_policy_weights_nbytes(int32_t cells, int32_t num_agents);
+/* HOST float32 weights in torch's layouts (Linear [out, in]: w1 [64, cells], w2 [64, 64], w_logits [5N, 64],
+ * w_value [1, 64]; LSTMCell weight_ih [256, 64 + 5N + 1], weight_hh [256, 64], b_ih / b_hh [256]) -> HOST packed
+ * block (bf16 weights, padded; the reward column of weight_ih and the biases in f32, b_ih + b_hh summed in f32). */
+int mapf_cte_lstm_policy_pack_weights(int32_t cells, int32_t num_agents, const float *w1, const float *b1,
+                                      const float *w2, const float *b2, const float *w_ih, const float *w_hh,
+                                      const float *b_ih, const float *b_hh, const float *w_logits,
+                                      const float *b_logits, const float *w_value, const float *b_value,
+                                      void *packed_host);
+int mapf_cte_lstm_policy_act(const mapf_cte_lstm_policy_args *args, void *stream);
 /* Per-step bookkeeping of the batched evaluator (main.py:test_trained_model, one episode per env, no auto-reset), in
  * one launch after mapf_step (and after mapf_occupancy_accumulate, which reads `active` before this call clears it).
  * For every env with active[b] != 0: episode_reward[b] += sum of the agents' rewards (main.py:251), agent_reward[b,n]

@@ -1,5 +1,5 @@
 """Timings of the kernels next to the hot path (CUDA events, warm-up, L2-sized working sets): the fused policy
-kernels (MLP and LSTM-64, shared and per-agent), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.
+kernels (MLP and LSTM-64, shared and per-agent; the CTE MLP and LSTM-64), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.
 `python tools/bench_aux.py`"""
 import json
 import sys
@@ -93,6 +93,59 @@ def cte_policy_act_entry(B, N=16):
             "flops_per_env": flops, "GBps": gbps, "TFLOPs": tflops, "env_steps_per_s": B / s,
             "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3), "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops,
             "hbm_floor_us": nbytes * B / (hbm_tbs * 1e12) * 1e6}
+
+
+def cte_lstm_policy_act_entry(B, N=16):
+    """The fused recurrent centralised CTE policy (mapf_cte_lstm_policy_act: trunk launch + recurrent step launch) at
+    65 536 envs x 16 agents on the 32x32 benchmark map, state advanced in place, the env's episode-end flags as the
+    episode-start flags, over the same rotation of 4 env batches as cte_policy_act.  The call is timed with CUDA
+    events; each kernel's share comes from a separate torch.profiler run over the same rotation."""
+    from dl_reference_models_b200.cte_rollout import CteRecurrentPolicy
+
+    ccfg = {"grid": maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32), "num_agents": N, "steps_per_episode": 256,
+            "seed": 999}
+    envs = [BatchedCteEnv(ccfg, B) for _ in range(4)]
+    for e in envs:
+        e.reset()
+    cells = envs[0].R * envs[0].C
+    policy = CteRecurrentPolicy(cells, N).cuda()
+    fused = [policy_kernels.FusedCteRecurrentPolicy(policy, e, env_id_base=k * B) for k, e in enumerate(envs)]
+    states = [(torch.zeros((B, 64), device="cuda"), torch.zeros((B, 64), device="cuda")) for _ in envs]
+    i = [0]
+
+    def act():
+        k = i[0] % 4
+        e = envs[k]
+        fused[k].act(states[k], fused[k].actions, e.reward, e.terminated, e.truncated)
+        i[0] += 1
+
+    s = timed(act, 200)
+    from torch.profiler import ProfilerActivity, profile
+
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(40):
+            act()
+        torch.cuda.synchronize()
+    dev_us = {}
+    for ev in prof.key_averages():
+        for kname in ("mapf_cte_lstm_trunk_kernel", "mapf_cte_lstm_step_kernel"):
+            if kname in ev.key:
+                dev_us[kname] = getattr(ev, "device_time_total", getattr(ev, "cuda_time_total", 0.0)) / 40
+    # byte / FLOP models per env.  trunk: grid codes R*C in, bf16 y (128 B) out; GEMMs R*C x 64, 64 x 64.  step: y,
+    # mask 5N, previous actions N, f64 reward, two flags, h / c in and out (4 x 256 B), int8 + int64 actions, joint
+    # logp, value; GEMMs 256 x (64 + 5N + 1 + 64) gates and 64 x (5N + 1) heads, without padding
+    b_trunk, b_step = cells + 128, 128 + 5 * N + N + 8 + 2 + 4 * 256 + N + 8 * N + 4 + 4
+    f_trunk, f_step = 2 * (cells * 64 + 64 * 64), 2 * (256 * (64 + 5 * N + 1 + 64) + 64 * (5 * N + 1))
+    hbm_tbs, bf16_tflops = 6.45, 2250.0   # SURVEY 8d measured copy bandwidth; dense bf16 data-sheet rate (tcgen05)
+    gbps, tflops = (b_trunk + b_step) * B / s / 1e9, (f_trunk + f_step) * B / s / 1e12
+    prof_total = sum(dev_us.values()) or float("nan")
+    return {"us_per_call": s * 1e6, "envs": B, "agents": N, "cells": cells,
+            "kernel_us_profiler": dev_us,
+            "trunk_share": dev_us.get("mapf_cte_lstm_trunk_kernel", float("nan")) / prof_total,
+            "step_share": dev_us.get("mapf_cte_lstm_step_kernel", float("nan")) / prof_total,
+            "bytes_per_env": {"trunk": b_trunk, "step": b_step}, "flops_per_env": {"trunk": f_trunk, "step": f_step},
+            "GBps": gbps, "TFLOPs": tflops, "env_steps_per_s": B / s,
+            "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3), "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops}
 
 
 def main():
@@ -225,6 +278,7 @@ def main():
                        "GBps": (cte.D * 4 + 200 + 20 + 40) * B / s / 1e9}
     del cte
     res["cte_policy_act"] = cte_policy_act_entry(B)
+    res["cte_lstm_policy_act"] = cte_lstm_policy_act_entry(B)
     try:
         import subprocess
 
