@@ -29,6 +29,7 @@ MAX_DIM = 255
 ENV_WORDS = 16
 METRIC_COUNT = 16
 INFO_WORDS = 16
+CTE_INFO_WORDS = 4
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED, ERR_STATE = 0, -1, -2, -3, -4
 DEV_ERR_INVALID_ACTION, DEV_ERR_NO_GOAL_CELL, DEV_ERR_TOO_FEW_CELLS, DEV_ERR_DUPLICATE_LAYOUT = 1, 2, 4, 8
@@ -126,7 +127,8 @@ class MapfCtePolicyArgs(C.Structure):
         ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("cells", C.c_int32), ("reserved", C.c_int32),
         ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
     ] + [(k, C.c_void_p) for k in (
-        "obs_grid", "action_mask", "weights", "actions", "actions64", "logp", "value", "logits_out")]
+        "obs_grid", "action_mask", "weights", "actions", "actions64", "logp", "value", "logits_out")] + [
+        ("greedy", C.c_int32)]
 
 
 class MapfCteLstmPolicyArgs(C.Structure):
@@ -137,7 +139,8 @@ class MapfCteLstmPolicyArgs(C.Structure):
         ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
     ] + [(k, C.c_void_p) for k in (
         "obs_grid", "action_mask", "prev_terminated", "prev_truncated", "prev_action", "prev_reward", "h_in", "c_in",
-        "h_out", "c_out", "trunk", "weights", "actions", "actions64", "logp", "value", "logits_out")]
+        "h_out", "c_out", "trunk", "weights", "actions", "actions64", "logp", "value", "logits_out")] + [
+        ("greedy", C.c_int32)]
 
 
 class MapfEvalArgs(C.Structure):
@@ -146,6 +149,15 @@ class MapfEvalArgs(C.Structure):
     _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("step", C.c_int64)] + [(k, C.c_void_p) for k in (
         "reward", "terminated", "truncated", "info", "active", "episode_reward", "agent_reward", "timesteps", "success",
         "last_info", "active_count")]
+
+
+class MapfCteEvalArgs(C.Structure):
+    """mapf_cte_eval_args of include/mapf_b200.h (the evaluator's per-step bookkeeping over the single-agent view)."""
+
+    _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("rows", C.c_int32), ("cols", C.c_int32),
+                ("step", C.c_int64)] + [(k, C.c_void_p) for k in (
+        "positions", "reward", "terminated", "truncated", "info", "active", "episode_reward", "timesteps", "success",
+        "last_info", "occupancy", "active_count")]
 
 
 class MapfError(RuntimeError):
@@ -259,6 +271,7 @@ def lib():
     L.mapf_cte_lstm_policy_act.argtypes = [C.POINTER(MapfCteLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
     L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
+    L.mapf_cte_eval_accumulate.argtypes = [C.POINTER(MapfCteEvalArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
@@ -284,6 +297,7 @@ EXPORTS = (
     "mapf_policy_act_per_agent", "mapf_lstm_policy_act_per_agent",
     "mapf_cte_policy_weights_nbytes", "mapf_cte_policy_pack_weights", "mapf_cte_policy_act",
     "mapf_cte_lstm_policy_weights_nbytes", "mapf_cte_lstm_policy_pack_weights", "mapf_cte_lstm_policy_act",
+    "mapf_cte_eval_accumulate",
 )
 
 

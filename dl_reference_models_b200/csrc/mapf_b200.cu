@@ -1520,21 +1520,28 @@ int mapf_metrics_reduce(mapf_handle *h, double *out_device, void *stream) {
     return MAPF_OK;
 }
 
-int mapf_occupancy_accumulate(mapf_handle *h, const uint8_t *active, uint64_t *counts, void *stream) {
-    int rc = check_ready(h);
-    if (rc) return rc;
-    if (!counts) return fail(MAPF_ERR_INVALID_ARG, "null argument");
-    DeviceGuard guard(h->cfg.device);
-    const long long BN = (long long)h->cfg.num_envs * h->cfg.num_agents;
-    const int cells = h->cfg.rows * h->cfg.cols;
+// the heat-map launch of mapf_occupancy_accumulate and mapf_cte_eval_accumulate: positions are packed uint32 words
+// (row in the low 16 bits, column in the high 16 bits, both signed), one per agent
+static void occupancy_launch(const uint32_t *positions, const uint8_t *active, int num_envs, int num_agents, int rows,
+                             int cols, uint64_t *counts, void *stream) {
+    const long long BN = (long long)num_envs * num_agents;
+    const int cells = rows * cols;
     const int use_smem = cells * 4 <= 48 * 1024;
     const int threads = 256;
     long long blocks = (BN + threads * 8 - 1) / (threads * 8);
     if (blocks > 1184) blocks = 1184;
     if (blocks < 1) blocks = 1;
     mapf::mapf_occupancy_kernel<<<(unsigned)blocks, threads, use_smem ? cells * 4 : 0, static_cast<cudaStream_t>(stream)>>>(
-        reinterpret_cast<const uint32_t *>(h->st.positions), active, BN, h->cfg.num_agents, h->cfg.rows, h->cfg.cols,
-        reinterpret_cast<unsigned long long *>(counts), use_smem);
+        positions, active, BN, num_agents, rows, cols, reinterpret_cast<unsigned long long *>(counts), use_smem);
+}
+
+int mapf_occupancy_accumulate(mapf_handle *h, const uint8_t *active, uint64_t *counts, void *stream) {
+    int rc = check_ready(h);
+    if (rc) return rc;
+    if (!counts) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    DeviceGuard guard(h->cfg.device);
+    occupancy_launch(reinterpret_cast<const uint32_t *>(h->st.positions), active, h->cfg.num_envs, h->cfg.num_agents,
+                     h->cfg.rows, h->cfg.cols, counts, stream);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
     return MAPF_OK;
@@ -1800,6 +1807,7 @@ int mapf_cte_policy_act(const mapf_cte_policy_args *a, void *stream) {
     if (a->num_envs < 1 || !a->obs_grid || !a->action_mask || !a->weights)
         return fail(MAPF_ERR_INVALID_ARG, "cte policy: num_envs >= 1, obs_grid, action_mask and weights are required");
     if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "cte policy: reserved is %d, must be 0", a->reserved);
+    if (a->greedy != 0 && a->greedy != 1) return fail(MAPF_ERR_INVALID_ARG, "cte policy: greedy %d is neither 0 nor 1", a->greedy);
     int ndev = 0, dev = 0, sms = 0, per_sm = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
@@ -1807,7 +1815,7 @@ int mapf_cte_policy_act(const mapf_cte_policy_args *a, void *stream) {
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int threads = mapf::CTE_THREADS, warps = threads / 32;
     const size_t smem = (size_t)mapf::cte_weight_bytes(a->cells, a->num_agents) + (size_t)warps * mapf::CTE_WARP_BYTES;
-    const auto kernel = mapf::mapf_cte_policy_act_kernel;
+    const auto kernel = a->greedy ? mapf::mapf_cte_policy_act_kernel<true> : mapf::mapf_cte_policy_act_kernel<false>;
     CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
     if (per_sm < 1) return fail(MAPF_ERR_UNSUPPORTED, "cte policy: %zu bytes of shared memory do not fit one SM", smem);
@@ -1879,12 +1887,15 @@ int mapf_cte_lstm_policy_act(const mapf_cte_lstm_policy_args *a, void *stream) {
     if (!a->h_out != !a->c_out)
         return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: h_out and c_out are given together (both NULL = state not advanced)");
     if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: reserved is %d, must be 0", a->reserved);
+    if (a->greedy != 0 && a->greedy != 1)
+        return fail(MAPF_ERR_INVALID_ARG, "cte lstm policy: greedy %d is neither 0 nor 1", a->greedy);
     int ndev = 0, dev = 0, sms = 0, per_sm[2] = {0, 0};
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
     CUDA_TRY(cudaGetDevice(&dev));
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    void (*const kernels[2])(const mapf_cte_lstm_policy_args) = {mapf::mapf_cte_lstm_trunk_kernel, mapf::mapf_cte_lstm_step_kernel};
+    void (*const kernels[2])(const mapf_cte_lstm_policy_args) = {
+        mapf::mapf_cte_lstm_trunk_kernel, a->greedy ? mapf::mapf_cte_lstm_step_kernel<true> : mapf::mapf_cte_lstm_step_kernel<false>};
     const int threads[2] = {mapf::CTE_THREADS, mapf::CTEL_THREADS};
     const size_t smem[2] = {(size_t)mapf::ctel_trunk_bytes(a->cells) + (size_t)(mapf::CTE_THREADS / 32) * mapf::CTE_WARP_BYTES,
                             (size_t)mapf::ctel_step_bytes(a->num_agents) + (size_t)(mapf::CTEL_THREADS / 32) * mapf::CTEL_WARP_BYTES};
@@ -1932,6 +1943,30 @@ int mapf_eval_accumulate(const mapf_eval_args *a, void *stream) {
     long long blocks = ((long long)a->num_envs + envs_per_block - 1) / envs_per_block;
     if (blocks > 148 * 8) blocks = 148 * 8;   // one resident wave; the count then costs one atomic per block
     mapf::mapf_eval_accumulate_kernel<<<(unsigned)blocks, mapf::EVAL_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a, P);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_cte_eval_accumulate(const mapf_cte_eval_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "null argument");
+    if (a->num_envs < 1 || a->num_agents < 1 || a->rows < 1 || a->cols < 1 || !a->positions || !a->reward ||
+        !a->terminated || !a->truncated || !a->info || !a->active || !a->episode_reward || !a->timesteps || !a->success ||
+        !a->last_info || !a->occupancy || !a->active_count)
+        return fail(MAPF_ERR_INVALID_ARG, "cte eval: null or empty argument");
+    if (a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "cte eval: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    // an int16 [B,N,2] (row, col) pair is, byte for byte on a little-endian device, the packed uint32 the heat-map
+    // kernel decodes (prow: low half, pcol: high half); the heat-map reads `active` before the next launch clears it
+    static_assert(sizeof(int16_t) * 2 == sizeof(uint32_t), "an agent's (row, col) pair is one packed position word");
+    occupancy_launch(reinterpret_cast<const uint32_t *>(a->positions), a->active, a->num_envs, a->num_agents, a->rows,
+                     a->cols, a->occupancy, stream);
+    CUDA_TRY(cudaGetLastError());
+    long long blocks = ((long long)a->num_envs + mapf::EVAL_THREADS - 1) / mapf::EVAL_THREADS;
+    if (blocks > 148 * 8) blocks = 148 * 8;   // one resident wave, as mapf_eval_accumulate
+    mapf::mapf_cte_eval_accumulate_kernel<<<(unsigned)blocks, mapf::EVAL_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }

@@ -17,7 +17,8 @@
 //      turns its rows' into a bit mask of the one-hot columns it holds (4 bits per k16 chunk); the A fragments of the
 //      one-hot chunks are rebuilt from that mask in every column block.  Every A fragment of an m-tile (y, one-hot,
 //      h) is read before the first h / c of that m-tile is written, so the state may be updated in place.  The heads
-//      and the draws are mapf_cte_policy_act_kernel's (mapf_cte_heads.inc), with the Philox tag "CTEL".
+//      and the draws (or, GREEDY, the argmax) are mapf_cte_policy_act_kernel's (mapf_cte_heads.inc), with the Philox
+//      tag "CTEL".
 // Shared memory of the step kernel at N = 32: 148 KB of gate weights, 24 KB of heads, 3 KB of f32 vectors and 8 warps'
 // [32][41] f32 head buffers (41 KB, which also hold the staged previous actions): 215 KB.
 #pragma once
@@ -83,6 +84,8 @@ __global__ void __launch_bounds__(CTE_THREADS, 1) mapf_cte_lstm_trunk_kernel(con
     }
 }
 
+// GREEDY = a.greedy: argmax instead of the draw, in the heads only (mapf_cte_heads.inc); the trunk kernel has no mode
+template <bool GREEDY>
 __global__ void __launch_bounds__(CTEL_THREADS, 1) mapf_cte_lstm_step_kernel(const mapf_cte_lstm_policy_args a) {
     extern __shared__ __align__(16) unsigned char psm[];
     const int N = a.num_agents, NH = ctel_kh(N) / 16, SG = ctel_sg(N), NT = cte_head_tiles(N);

@@ -17,7 +17,8 @@
 //     n8 tiles, evaluated in groups of five tiles (40 columns = 8 agents) into a per-warp [32][41] float buffer that
 //     reuses the grid staging; lane e then runs env e's agents of the group in agent order: mask, stable softmax,
 //     an inverse-CDF draw from one Philox word (pol_draw: key (seed ^ "CTEP", env_id_base + env), counter
-//     (counter, agent)), and adds the agent's log-probability to the env's joint one.
+//     (counter, agent)), and adds the agent's log-probability to the env's joint one.  In greedy mode (the template
+//     parameter GREEDY, from a.greedy) the action is the first index of the largest masked logit instead, no Philox.
 //
 // Layers 1-2 and the heads + draws are written in mapf_cte_trunk.inc / mapf_cte_heads.inc, which the recurrent CTE
 // kernels (mapf_cte_lstm_policy_kernel.cuh) include as well.
@@ -72,6 +73,8 @@ __device__ __forceinline__ void cte_stage(const uint8_t *obs, int cells, int na,
     }
 }
 
+// GREEDY = a.greedy: the first argmax of each agent's masked logits instead of the draw (mapf_cte_heads.inc)
+template <bool GREEDY>
 __global__ void __launch_bounds__(CTE_THREADS, 1) mapf_cte_policy_act_kernel(const mapf_cte_policy_args a) {
     extern __shared__ __align__(16) unsigned char psm[];
     const int cells = a.cells, N = a.num_agents, S1 = cte_s1(cells), KP = cte_kpad(cells), NT = cte_head_tiles(N);

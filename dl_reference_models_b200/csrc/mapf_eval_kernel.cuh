@@ -7,6 +7,7 @@
 //   * an inactive env costs one byte read;
 //   * the envs still active after the step are counted per warp, reduced per block and added with one atomic per block
 //     into active_count[step & 1]; block 0 zeroes the other word, the one the next step counts into.
+// mapf_cte_eval_accumulate_kernel does the same for the single-agent (CTE) view, one thread per env.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -48,6 +49,41 @@ __global__ void __launch_bounds__(EVAL_THREADS, 8) mapf_eval_accumulate_kernel(c
             } else {
                 ++still;
             }
+        }
+    }
+    still = __reduce_add_sync(0xFFFFFFFFu, still);
+    if (lane == 0) warp_still[warp] = still;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned s = 0;
+        for (int w = 0; w < warps; ++w) s += warp_still[w];
+        if (s) atomicAdd(a.active_count + slot, s);
+    }
+}
+
+// The CTE view's bookkeeping (mapf_cte_eval_accumulate), one thread per env: the view has one f64 reward per env, so
+// there is nothing to reduce.  Each env adds its rewards in step order, the same sequence of f64 additions as a Python
+// `total += reward` loop.  The heat-map is counted before this launch by mapf_occupancy_kernel.  The block-count tail
+// is mapf_eval_accumulate_kernel's, written out again: shared as a device function it changed that kernel's code.
+__global__ void __launch_bounds__(EVAL_THREADS) mapf_cte_eval_accumulate_kernel(const mapf_cte_eval_args a) {
+    __shared__ unsigned warp_still[EVAL_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
+    const int slot = (int)(a.step & 1);
+    if (blockIdx.x == 0 && threadIdx.x == 0) a.active_count[slot ^ 1] = 0u;
+    unsigned still = 0;
+#pragma unroll 1
+    for (long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x; b < a.num_envs; b += (long long)gridDim.x * blockDim.x) {
+        if (!a.active[b]) continue;
+        a.episode_reward[b] += a.reward[b];
+        a.timesteps[b] += 1;
+#pragma unroll
+        for (int w = 0; w < MAPF_CTE_INFO_WORDS; ++w) a.last_info[b * MAPF_CTE_INFO_WORDS + w] = a.info[b * MAPF_CTE_INFO_WORDS + w];
+        const bool term = a.terminated[b] != 0, trunc = a.truncated[b] != 0;
+        if (term || trunc) {
+            a.success[b] = (uint8_t)(term && !trunc);
+            a.active[b] = 0;
+        } else {
+            ++still;
         }
     }
     still = __reduce_add_sync(0xFFFFFFFFu, still);

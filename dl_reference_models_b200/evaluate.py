@@ -15,6 +15,12 @@ reference's shape (and the per-agent variants :class:`rollout.PerAgentActionMask
 :class:`recurrent.PerAgentRecurrentPolicy`, one module per agent, of that shape) run as one fused kernel launch per step (``mapf_policy_act`` / ``mapf_lstm_policy_act`` in greedy
 mode), any other shape through its PyTorch forward.
 
+The reference's third execution mode, CTE (``env_config["training_execution_mode"] == "CTE"``, or a
+:class:`cte_rollout.CteActionMaskPolicy` / :class:`cte_rollout.CteRecurrentPolicy`), plays the single-agent view
+instead: episode e is env e of a :class:`single_agent.BatchedCteEnv`, one joint action and one scalar reward per step,
+the heat-map and the per-episode sums accumulated by ``mapf_cte_eval_accumulate``.  Centralised modules of the fused
+shape run ``mapf_cte_policy_act`` / ``mapf_cte_lstm_policy_act`` in greedy mode, other shapes their PyTorch forward.
+
 ``python -m dl_reference_models_b200.evaluate`` times the evaluator (:func:`benchmark`).
 """
 from __future__ import annotations
@@ -26,13 +32,16 @@ import numpy as np
 import torch
 
 from . import _native as nat
-from . import rollout
+from . import maps, rollout
 from .batched_env import BatchedMapfEnv
-from .policy_kernels import FusedPolicy, FusedRecurrentPolicy
+from .cte_rollout import CteActionMaskPolicy, CteRecurrentPolicy
+from .policy_kernels import FusedCtePolicy, FusedCteRecurrentPolicy, FusedPolicy, FusedRecurrentPolicy
 from .recurrent import PerAgentRecurrentPolicy, RecurrentActionMaskPolicy
+from .single_agent import BatchedCteEnv
 
 MODULE_TYPES = (rollout.ActionMaskPolicy, RecurrentActionMaskPolicy, rollout.PerAgentActionMaskPolicy, PerAgentRecurrentPolicy)
 RECURRENT_TYPES = (RecurrentActionMaskPolicy, PerAgentRecurrentPolicy)
+CTE_MODULE_TYPES = (CteActionMaskPolicy, CteRecurrentPolicy)
 
 
 @dataclass
@@ -169,13 +178,182 @@ def _play(env, policy="random", max_steps: int | None = None, explore: bool = Fa
     return acc
 
 
+def _cte_view(env_config: dict, policy) -> bool:
+    """Whether ``policy`` is evaluated on the single-agent (CTE) view: a centralised module, or, for the other
+    policies, ``training_execution_mode == "CTE"`` (the reference's switch, main.py:71-77).  A module of one view with
+    a config that names another mode is refused."""
+    mode = env_config.get("training_execution_mode")
+    if isinstance(policy, CTE_MODULE_TYPES):
+        if mode is not None and mode != "CTE":
+            raise ValueError(f"a {type(policy).__name__} is a centralised (CTE) policy; the env_config names "
+                             f"training_execution_mode = {mode!r}")
+        return True
+    if isinstance(policy, MODULE_TYPES):
+        if mode == "CTE":
+            raise ValueError(f"a {type(policy).__name__} plays the multi-agent view; the env_config names "
+                             "training_execution_mode = 'CTE' (use a CteActionMaskPolicy or CteRecurrentPolicy)")
+        return False
+    return mode == "CTE"
+
+
+def _check_cte_module(policy, env_config: dict, device) -> None:
+    """Refuse a centralised module whose cells, num_agents or device do not match the env, before any device work."""
+    grid = env_config.get("grid")
+    R, C_ = (np.asarray(grid) if grid is not None else maps.get_grid(env_config["env_name"])).shape
+    N = int(env_config.get("num_agents", 2))
+    if policy.cells != R * C_:
+        raise ValueError(f"the policy reads {policy.cells} grid cells, the env's map has {R}x{C_} = {R * C_}")
+    if policy.num_agents != N:
+        raise ValueError(f"the policy has num_agents = {policy.num_agents}, the env has num_agents = {N} agents")
+    dev = torch.device(device)
+    if dev.type == "cuda" and dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device() if torch.cuda.is_available() else 0)
+    wrong = {str(p.device) for p in policy.parameters() if p.device != dev}
+    if wrong:
+        raise ValueError(f"the policy's parameters are on {sorted(wrong)}, the evaluation runs on {dev}")
+
+
+def _cte_module_actor(env, policy, explore: bool):
+    """``act() -> int8 [B,N]`` for a centralised module on the CTE env's current ``obs_grid`` / ``action_mask``: one
+    fused call (greedy unless ``explore``) where the kernels implement the module's shape, its PyTorch forward
+    otherwise.  The LSTM carries (h, c), the previous joint action and the previous float64 reward, zero at reset."""
+    B, dev = env.B, env.device
+    if isinstance(policy, CteRecurrentPolicy) and FusedCteRecurrentPolicy.matches(policy, env):
+        fused = FusedCteRecurrentPolicy(policy, env)
+        state = (torch.zeros((B, 64), device=dev), torch.zeros((B, 64), device=dev))
+        prev_reward = [torch.zeros(B, dtype=torch.float64, device=dev)]
+
+        def act():
+            a, _, _ = fused.act(state, fused.actions, prev_reward[0], greedy=not explore)
+            prev_reward[0] = env.reward   # read by the next call before the next step overwrites it
+            return a
+        return act
+    if isinstance(policy, CteActionMaskPolicy) and FusedCtePolicy.matches(policy, env):
+        fused = FusedCtePolicy(policy, env)
+        return lambda: fused.act(greedy=not explore)[0]
+    return _cte_torch_actor(env, policy, explore)
+
+
+def _cte_torch_actor(env, policy, explore: bool):
+    """The centralised module's own forward / step (any shape), with the same carry as the fused path."""
+    B, N, dev = env.B, env.N, env.device
+    cells = env.R * env.C
+    recurrent = isinstance(policy, CteRecurrentPolicy)
+    carry = {}
+    if recurrent:
+        carry.update(state=policy.initial_state(B, dev), prev_action=torch.zeros((B, N), dtype=torch.int64, device=dev),
+                     prev_reward=torch.zeros(B, dtype=torch.float64, device=dev))
+
+    @torch.no_grad()
+    def act():
+        grid = env.obs_grid.view(B, cells)
+        if recurrent:
+            logits, _, carry["state"] = policy.step(grid, env.action_mask, carry["prev_action"], carry["prev_reward"],
+                                                    carry["state"])
+        else:
+            logits, _ = policy(grid, env.action_mask)
+        a = rollout.sample_categorical(logits)[0] if explore else torch.argmax(logits, dim=-1)
+        if recurrent:
+            carry["prev_action"] = a
+            carry["prev_reward"] = env.reward   # read by the next step() before the next env step
+        return a.to(torch.int8)
+    return act
+
+
+def _play_cte(env, policy="random", max_steps: int | None = None, explore: bool = False) -> dict:
+    """:func:`_play` on the single-agent view: reset ``env`` (a :class:`single_agent.BatchedCteEnv`) once and play
+    every env's first episode to its end (or ``max_steps`` steps).  Per step: the policy, the env step (without the
+    float32 ``flat_obs`` output: the policies read ``obs_grid`` and ``action_mask``) and ``mapf_cte_eval_accumulate``
+    (heat-map and bookkeeping); the loop's one host sync is the 4-byte read of the still-active count.  A callable
+    policy is called as ``policy(env, (env.obs_grid, env.action_mask))``.  Returns the device accumulators."""
+    B, N, dev = env.B, env.N, env.device
+    env.reset()
+    if isinstance(policy, CTE_MODULE_TYPES):
+        module_act = _cte_module_actor(env, policy, explore)
+        policy = lambda env, out: module_act()  # noqa: E731
+    elif policy in ("random", "masked"):
+        gen = torch.Generator(device=dev).manual_seed(int(env.seed or 0))
+        masked = policy == "masked"
+
+        def policy(env, out):
+            if not masked:
+                return torch.randint(0, 5, (B, N), dtype=torch.int8, device=dev, generator=gen)
+            u = torch.rand((B, N, 5), device=dev, generator=gen)   # uniform over each agent's allowed actions
+            return torch.argmax(u * env.action_mask.view(B, N, 5), dim=-1).to(torch.int8)
+    elif not callable(policy):
+        raise ValueError(f"policy must be 'random', 'masked', a callable or a centralised module, got {policy!r}")
+    z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
+    acc = {"starts": env.starts.cpu().numpy().copy(), "goals": env.goals.cpu().numpy().copy(),
+           "active": torch.ones(B, dtype=torch.uint8, device=dev), "episode_reward": z(B, torch.float64),
+           "timesteps": z(B, torch.int64), "success": z(B, torch.uint8),
+           "last_info": z((B, nat.CTE_INFO_WORDS), torch.float64), "occupancy": z((env.R, env.C), torch.int64),
+           "active_count": z(2, torch.int32)}
+    p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
+    sargs = nat.MapfCteArgs.from_buffer_copy(env._args)   # the env's own block, without the float32 observation
+    sargs.flat_obs = None
+    args = nat.MapfCteEvalArgs(
+        num_envs=B, num_agents=N, rows=env.R, cols=env.C, positions=p(env.positions), reward=p(env.reward),
+        terminated=p(env.terminated), truncated=p(env.truncated), info=p(env.info), active=p(acc["active"]),
+        episode_reward=p(acc["episode_reward"]), timesteps=p(acc["timesteps"]), success=p(acc["success"]),
+        last_info=p(acc["last_info"]), occupancy=p(acc["occupancy"]), active_count=p(acc["active_count"]))
+    counts = (acc["active_count"][0], acc["active_count"][1])
+    lib, stream = nat.lib(), env._stream()
+    limit = max_steps if max_steps is not None else env.steps_per_episode + 1
+    out = (env.obs_grid, env.action_mask)
+    still = B
+    for step in range(limit):
+        if still == 0:
+            break
+        actions = policy(env, out)
+        a = torch.as_tensor(actions).to(device=dev, dtype=torch.int8).reshape(B, N).contiguous()
+        sargs.actions = a.data_ptr()
+        nat.check(lib.mapf_cte_step(C.byref(sargs), stream))
+        args.step = step
+        nat.check(lib.mapf_cte_eval_accumulate(C.byref(args), stream))
+        still = int(counts[step & 1])
+    return acc
+
+
+def _cte_result(env, acc) -> EvalResult:
+    """The CSV rows and summary of the CTE view (DESIGN.md §7 N2b): the multi-agent schema without per-agent rewards
+    (the view has one scalar reward), the two CTE counters of the episode's last step instead of the lifelong ones."""
+    B, N = env.B, env.N
+    starts, goals0 = acc["starts"], acc["goals"]
+    info = acc["last_info"].cpu().numpy()
+    ep_r, st = acc["episode_reward"].cpu().numpy(), acc["timesteps"].cpu().numpy()
+    succ = acc["success"].cpu().numpy().astype(np.float64)
+    res = EvalResult()
+    for e in range(B):
+        row = {"episode": e + 1, "cpu_time": 0.0, "seed": env.env_config.get("seed"), "total_reward": float(ep_r[e]),
+               "timesteps": int(st[e]), "goals_reached_total": float(info[e, 2]), "blocking_count_total": float(info[e, 3])}
+        for i in range(N):
+            row[f"agent_{i}_start_x"], row[f"agent_{i}_start_y"] = int(starts[e, i, 0]), int(starts[e, i, 1])
+            row[f"agent_{i}_goal_x"], row[f"agent_{i}_goal_y"] = int(goals0[e, i, 0]), int(goals0[e, i, 1])
+        res.rows.append(row)
+    res.occupancy_grid = acc["occupancy"].cpu().numpy()
+    res.success_rate = float(np.mean(succ)) if B else 0.0
+    res.average_reward = float(ep_r.sum() / max(B, 1))
+    res.average_timesteps = float(st.sum() / max(B, 1))
+    return res
+
+
 def evaluate(env_config: dict, num_episodes: int, policy="random", device="cuda:0", max_steps: int | None = None,
              explore: bool = False) -> EvalResult:
     """Play ``num_episodes`` episodes, one per env of a batch.  ``policy``: ``"random"``, ``"masked"``, a callable
     ``policy(env, out) -> int8 [B,N]``, or a trained :class:`rollout.ActionMaskPolicy` /
     :class:`recurrent.RecurrentActionMaskPolicy` / :class:`rollout.PerAgentActionMaskPolicy` /
     :class:`recurrent.PerAgentRecurrentPolicy` (``num_agents`` = the env's) on ``device``, played as the reference's ``forward_inference`` (argmax
-    of the masked logits; ``explore=True``: a draw from them)."""
+    of the masked logits; ``explore=True``: a draw from them).
+
+    A :class:`cte_rollout.CteActionMaskPolicy` / :class:`cte_rollout.CteRecurrentPolicy`, or any other policy with
+    ``env_config["training_execution_mode"] == "CTE"``, plays the single-agent view (:class:`single_agent.BatchedCteEnv`);
+    there the callable receives the CTE env and ``(env.obs_grid, env.action_mask)``, and the rows carry the episode's
+    scalar return and its last ``goals_reached_total`` / ``blocking_count_total`` instead of per-agent rewards."""
+    if _cte_view(env_config, policy):
+        if isinstance(policy, CTE_MODULE_TYPES):
+            _check_cte_module(policy, env_config, device)
+        env = BatchedCteEnv(env_config, num_episodes, device)
+        return _cte_result(env, _play_cte(env, policy, max_steps, explore))
     env = BatchedMapfEnv(env_config, num_episodes, device)
     acc = _play(env, policy, max_steps, explore)
     B, N = env.B, env.N
@@ -219,7 +397,10 @@ def benchmark(num_episodes: int = 65536, rounds: int = 3, device: str = "cuda:0"
     LSTM-64 module greedy on their fused kernels, and the LSTM-64 module through its PyTorch forward (the path of
     non-reference shapes).  Agent-steps count every env at every loop step (finished envs are still stepped).  Best of
     ``rounds`` after a short warm-up each; host clock around work that ends in a device synchronise (the loop's last
-    count read).  ``evaluate_masked_s`` is one whole :func:`evaluate` call, env construction and rows included."""
+    count read).  ``evaluate_masked_s`` is one whole :func:`evaluate` call, env construction and rows included.  The
+    ``cte_*`` keys time :func:`_play_cte` the same way on the single-agent view of the same map and shape: the uniform
+    masked policy, the centralised MLP and LSTM-64 modules greedy on their fused kernels, and the LSTM-64 module through
+    its PyTorch forward."""
     import subprocess
     import time
 
@@ -257,6 +438,29 @@ def benchmark(num_episodes: int = 65536, rounds: int = 3, device: str = "cuda:0"
     t0 = time.perf_counter()
     evaluate(cfg, num_episodes, "masked", device)
     res["evaluate_masked_s"] = time.perf_counter() - t0
+    ccfg = {"num_agents": 16, "steps_per_episode": 256, "seed": 999, "grid": cfg["grid"]}
+    cenv = BatchedCteEnv(ccfg, num_episodes, device)
+    torch.manual_seed(0)
+    cmlp = CteActionMaskPolicy(cenv.R * cenv.C, cenv.N).to(cenv.device)
+    clstm = CteRecurrentPolicy(cenv.R * cenv.C, cenv.N).to(cenv.device)
+    ccases = {"cte_masked": lambda: "masked", "cte_mlp_greedy_fused": lambda: cmlp, "cte_lstm_greedy_fused": lambda: clstm,
+              "cte_lstm_greedy_torch": lambda: (lambda e, o, act=_cte_torch_actor(cenv, clstm, False): act())}
+    for name, make in ccases.items():
+        def crun(max_steps=None):
+            return _play_cte(cenv, make(), max_steps)
+
+        crun(8)
+        times, steps = [], 0
+        for _ in range(rounds):
+            torch.cuda.synchronize(cenv.device)
+            t0 = time.perf_counter()
+            acc = crun()
+            times.append(time.perf_counter() - t0)
+            steps = int(acc["timesteps"].max())
+        n = num_episodes * cenv.N * steps
+        res[name] = {"loop_s": min(times), "rounds_s": times, "loop_steps": steps,
+                     "episodes_per_s": num_episodes / min(times), "agent_steps_per_s": n / min(times)}
+    del cenv
     try:
         gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i",
                               str(torch.device(device).index or 0)], capture_output=True, text=True, timeout=30).stdout.strip()

@@ -307,23 +307,26 @@ class FusedCtePolicy:
         self._dev.copy_(torch.from_numpy(self._host))
 
     def args(self, obs_grid, action_mask, *, actions=None, actions64=None, logp=None, value=None, logits_out=None,
-             num_envs: int | None = None) -> nat.MapfCtePolicyArgs:
+             num_envs: int | None = None, greedy: bool = False) -> nat.MapfCtePolicyArgs:
         """The argument block of one launch (counter 0; set ``.counter`` before launching).  Tensor arguments may be
-        None, except the inputs ``obs_grid`` (uint8 [B, R*C]) and ``action_mask`` (int8 [B, 5N])."""
+        None, except the inputs ``obs_grid`` (uint8 [B, R*C]) and ``action_mask`` (int8 [B, 5N]).  ``greedy``: each
+        agent's first argmax of its masked logits instead of the draw."""
         p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
         return nat.MapfCtePolicyArgs(
             num_envs=self.env.B if num_envs is None else int(num_envs), num_agents=self.env.N, cells=self.cells,
             reserved=0, seed=self.seed, counter=0, env_id_base=self.env_id_base,
             obs_grid=p(obs_grid), action_mask=p(action_mask), weights=p(self._dev), actions=p(actions),
-            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out))
+            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out), greedy=int(bool(greedy)))
 
     def act(self, obs_grid=None, action_mask=None, *, logits_out: torch.Tensor | None = None,
             logp: torch.Tensor | None = None, value: torch.Tensor | None = None, actions64: torch.Tensor | None = None,
-            num_envs: int | None = None):
+            num_envs: int | None = None, greedy: bool = False):
         """One launch on ``obs_grid`` (uint8 [B, R, C] or [B, R*C]; default: the env's) and ``action_mask`` (int8
         [B, 5N]; default: the env's).  Returns (actions int8 [B, N], joint logp [B], value [B]); ``logits_out``
         [B, N, 5] receives the masked logits.  ``num_envs``: launch on the first ``num_envs`` rows of the given tensors
-        (with the constructor's ``env_id_base``: one shard of a larger batch)."""
+        (with the constructor's ``env_id_base``: one shard of a larger batch).  ``greedy``: every agent takes the first
+        argmax of its masked logits (RLlib's deterministic MultiDiscrete sample), logp is the sum of their
+        log-probabilities, the other outputs are what the draw mode writes."""
         env = self.env
         obs_grid = env.obs_grid if obs_grid is None else obs_grid
         action_mask = env.action_mask if action_mask is None else action_mask
@@ -336,7 +339,7 @@ class FusedCtePolicy:
         value = self.value if value is None else value
         actions64 = self.actions64 if actions64 is None else actions64
         a = self.args(obs_grid, action_mask, actions=self.actions, actions64=actions64, logp=logp, value=value,
-                      logits_out=logits_out, num_envs=B)
+                      logits_out=logits_out, num_envs=B, greedy=greedy)
         self.counter += 1
         a.counter = self.counter
         nat.check(self._lib.mapf_cte_policy_act(C.byref(a), env._stream()))
@@ -405,9 +408,9 @@ class FusedCteRecurrentPolicy:
 
     def args(self, obs_grid, action_mask, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *,
              state_out=None, actions=None, actions64=None, logp=None, value=None, logits_out=None,
-             num_envs: int | None = None) -> nat.MapfCteLstmPolicyArgs:
+             num_envs: int | None = None, greedy: bool = False) -> nat.MapfCteLstmPolicyArgs:
         """The argument block of one call (counter 0; set ``.counter`` before launching).  ``state_out=None``: the
-        state is not advanced; the outputs may be None."""
+        state is not advanced; the outputs may be None.  ``greedy``: each agent's first argmax instead of the draw."""
         p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
         h, c = state
         ho, co = (None, None) if state_out is None else state_out
@@ -417,12 +420,12 @@ class FusedCteRecurrentPolicy:
             obs_grid=p(obs_grid), action_mask=p(action_mask), prev_terminated=p(prev_terminated),
             prev_truncated=p(prev_truncated), prev_action=p(prev_action), prev_reward=p(prev_reward), h_in=p(h),
             c_in=p(c), h_out=p(ho), c_out=p(co), trunk=p(self.trunk), weights=p(self._dev), actions=p(actions),
-            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out))
+            actions64=p(actions64), logp=p(logp), value=p(value), logits_out=p(logits_out), greedy=int(bool(greedy)))
 
     def act(self, state, prev_action, prev_reward, prev_terminated=None, prev_truncated=None, *, obs_grid=None,
             action_mask=None, advance: bool = True, state_out=None, logits_out: torch.Tensor | None = None,
             logp: torch.Tensor | None = None, value: torch.Tensor | None = None, actions64: torch.Tensor | None = None,
-            num_envs: int | None = None):
+            num_envs: int | None = None, greedy: bool = False):
         """One call on ``obs_grid`` (uint8 [B, R*C]; default: the env's) and ``action_mask`` (int8 [B, 5N]; default:
         the env's).  ``state`` = (h, c) float32 [B, 64]; ``prev_action`` int8 [B, N] (may be :attr:`actions` itself);
         ``prev_reward`` float64 [B] (the env's ``reward``); ``prev_terminated`` / ``prev_truncated`` uint8 [B] flag the
@@ -430,7 +433,8 @@ class FusedCteRecurrentPolicy:
         ``advance`` the new state goes to ``state_out`` (default: ``state``, in place) and the draw to :attr:`actions`;
         without it the state and :attr:`actions` are left as they are.  Returns (actions int8 [B, N], joint logp [B],
         value [B]); ``logits_out`` [B, N, 5] receives the masked logits.  ``num_envs``: the first ``num_envs`` rows of
-        every tensor (with the constructor's ``env_id_base``: one shard of a larger batch)."""
+        every tensor (with the constructor's ``env_id_base``: one shard of a larger batch).  ``greedy``: every agent
+        takes the first argmax of its masked logits; the state, value, logp and logits are what the draw mode writes."""
         env = self.env
         obs_grid = env.obs_grid if obs_grid is None else obs_grid
         action_mask = env.action_mask if action_mask is None else action_mask
@@ -448,7 +452,7 @@ class FusedCteRecurrentPolicy:
         a = self.args(obs_grid, action_mask, state, prev_action, prev_reward, prev_terminated, prev_truncated,
                       state_out=(state if state_out is None else state_out) if advance else None,
                       actions=self.actions if advance else None, actions64=actions64, logp=logp, value=value,
-                      logits_out=logits_out, num_envs=B)
+                      logits_out=logits_out, num_envs=B, greedy=greedy)
         self.counter += 1
         a.counter = self.counter
         nat.check(self._lib.mapf_cte_lstm_policy_act(C.byref(a), env._stream()))

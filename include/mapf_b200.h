@@ -511,7 +511,8 @@ int mapf_lstm_policy_act_per_agent(const mapf_lstm_policy_args *args, void *stre
  * (counter, agent): a stream of its own, distinct from mapf_policy_act's and mapf_lstm_policy_act's.  logp is the f32
  * sum of the agents' log-probabilities, added in agent order.
  * Supported: 1 <= num_agents <= MAPF_MAX_AGENTS and 1 <= cells <= MAPF_CTE_POLICY_MAX_CELLS (MAPF_ERR_UNSUPPORTED
- * otherwise); null inputs, num_envs < 1 and reserved != 0 give MAPF_ERR_INVALID_ARG; all before any device work. */
+ * otherwise); null inputs, num_envs < 1, reserved != 0 and greedy outside {0, 1} give MAPF_ERR_INVALID_ARG; all
+ * before any device work.  greedy = 1 replaces the draws by each agent's argmax (the evaluator's mode). */
 #define MAPF_CTE_POLICY_MAX_CELLS 1024
 
 typedef struct mapf_cte_policy_args {
@@ -529,6 +530,11 @@ typedef struct mapf_cte_policy_args {
     float *logp;                   /* [B] joint log-probability, may be NULL */
     float *value;                  /* [B] value head, may be NULL */
     float *logits_out;             /* [B, N, 5] masked logits, may be NULL */
+    int32_t greedy;                /* 0 = the per-agent draws above; 1 = per agent the first index of the largest masked
+                                      logit (torch.argmax, RLlib's deterministic MultiDiscrete sample), no Philox call, so
+                                      seed and counter do not matter; logp is then the sum of the chosen actions'
+                                      log-probabilities, every other output is what draw mode writes.  Other values:
+                                      MAPF_ERR_INVALID_ARG */
 } mapf_cte_policy_args;
 
 /* Bytes of the packed CTE policy weight block (negative = unsupported cells / num_agents). */
@@ -549,8 +555,8 @@ int mapf_cte_policy_act(const mapf_cte_policy_args *args, void *stream);
  * term added in f32, c kept in f32) with the heads and the draws.  Each agent's draw is an inverse CDF of one Philox
  * word keyed by (seed ^ "CTEL", env_id_base + env), counter (counter, agent): a stream of its own; logp is the f32 sum
  * of the agents' log-probabilities in agent order.  Supported shapes are mapf_cte_policy_act's
- * (MAPF_ERR_UNSUPPORTED otherwise); null required pointers, num_envs < 1, reserved != 0 and h_out without c_out (or
- * the reverse) give MAPF_ERR_INVALID_ARG; all before any device work. */
+ * (MAPF_ERR_UNSUPPORTED otherwise); null required pointers, num_envs < 1, reserved != 0, greedy outside {0, 1} and
+ * h_out without c_out (or the reverse) give MAPF_ERR_INVALID_ARG; all before any device work. */
 typedef struct mapf_cte_lstm_policy_args {
     int32_t num_envs, num_agents;
     int32_t cells;                  /* R * C */
@@ -575,6 +581,9 @@ typedef struct mapf_cte_lstm_policy_args {
     float *logp;                    /* [B] joint log-probability, may be NULL */
     float *value;                   /* [B] value head, may be NULL */
     float *logits_out;              /* [B, N, 5] masked logits, may be NULL */
+    int32_t greedy;                 /* 0 = draw; 1 = per agent the first argmax of the masked logits, no Philox call
+                                       (h_out, c_out, trunk, value, logp and logits_out as in draw mode); other values:
+                                       MAPF_ERR_INVALID_ARG.  As mapf_cte_policy_args.greedy */
 } mapf_cte_lstm_policy_args;
 
 /* Bytes of the packed recurrent CTE policy weight block (negative = unsupported cells / num_agents). */
@@ -614,6 +623,37 @@ typedef struct mapf_eval_args {
 } mapf_eval_args;
 
 int mapf_eval_accumulate(const mapf_eval_args *args, void *stream);
+
+/* The same bookkeeping for the single-agent (CTE) view (mapf_cte_step's outputs: one f64 reward per env, f64 [B,4]
+ * info, int16 [B,N,2] positions), stateless, one call per step after mapf_cte_step.  It first adds the heat-map:
+ * occupancy[r * cols + c] += 1 for every agent of every env with active[b] != 0 at its position (r, c) after the step
+ * (main.py:264-267, positions outside the map are skipped).  Then, for every env with active[b] != 0:
+ * episode_reward[b] += reward[b] (in step order, bit for bit a Python `total += reward` loop), timesteps[b] += 1,
+ * last_info[b,:] = info[b,:]; if terminated[b] | truncated[b]: success[b] = terminated[b] && !truncated[b] and
+ * active[b] = 0.  active_count follows mapf_eval_accumulate's parity scheme (word step & 1 counts the envs still
+ * active, the other word is zeroed).  Every pointer is a device pointer and is required; null pointers or a
+ * non-positive num_envs / num_agents / rows / cols give MAPF_ERR_INVALID_ARG, num_agents > MAPF_MAX_AGENTS
+ * MAPF_ERR_UNSUPPORTED, all before any device work. */
+#define MAPF_CTE_INFO_WORDS 4
+
+typedef struct mapf_cte_eval_args {
+    int32_t num_envs, num_agents, rows, cols;
+    int64_t step;               /* selects the counter word */
+    const int16_t *positions;   /* [B,N,2] (row, col) after the step */
+    const double *reward;       /* [B] */
+    const uint8_t *terminated;  /* [B] */
+    const uint8_t *truncated;   /* [B] */
+    const double *info;         /* [B,4] as mapf_cte_args.info */
+    uint8_t *active;            /* [B] 1 while the env's first episode runs; cleared by this call at its end */
+    double *episode_reward;     /* [B] */
+    int64_t *timesteps;         /* [B] */
+    uint8_t *success;           /* [B] */
+    double *last_info;          /* [B,4] info of the env's last active step */
+    uint64_t *occupancy;        /* [rows * cols] */
+    uint32_t *active_count;     /* [2] envs still active after this step, in word step & 1 */
+} mapf_cte_eval_args;
+
+int mapf_cte_eval_accumulate(const mapf_cte_eval_args *args, void *stream);
 
 /* rewards / values / adv / ret: device float32 [T,B,N]; dones uint8 [T,B]; last_value float32 [B,N]. */
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
