@@ -19,7 +19,7 @@ LIB_PATH = Path(os.environ.get("MAPF_B200_LIB", PKG / "libmapf_b200.so"))
 SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_kernel.cuh", CSRC / "mapf_pair_kernel.cuh", CSRC / "mapf_cte_kernel.cuh", CSRC / "mapf_policy_kernel.cuh",
            CSRC / "mapf_policy_lstm_kernel.cuh", CSRC / "mapf_eval_kernel.cuh", CSRC / "mapf_cte_policy_kernel.cuh",
            CSRC / "mapf_cte_lstm_policy_kernel.cuh", CSRC / "mapf_cte_trunk.inc",
-           CSRC / "mapf_cte_heads.inc", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
+           CSRC / "mapf_cte_heads.inc", CSRC / "mapf_vtrace_kernel.cuh", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
 MAX_AGENTS = 32
@@ -160,6 +160,15 @@ class MapfCteEvalArgs(C.Structure):
         "last_info", "occupancy", "active_count")]
 
 
+class MapfVtraceArgs(C.Structure):
+    """mapf_vtrace_args of include/mapf_b200.h (V-trace targets over time columns of a rollout)."""
+
+    _fields_ = [("T", C.c_int32), ("num_agents", C.c_int32), ("num_columns", C.c_int64), ("M", C.c_int64)] + [
+        (k, C.c_void_p) for k in ("columns", "rewards", "behaviour_logp", "dones", "bootstrap_value", "target_logp",
+                                  "values", "vs", "pg_advantages")] + [
+        ("gamma", C.c_float), ("clip_rho", C.c_float), ("clip_pg_rho", C.c_float), ("reserved", C.c_int32)]
+
+
 class MapfError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"libmapf_b200 error {code}: {message}")
@@ -271,6 +280,7 @@ def lib():
     L.mapf_cte_lstm_policy_act.argtypes = [C.POINTER(MapfCteLstmPolicyArgs), vp]
     L.mapf_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, i32, C.c_float, C.c_float, vp]
     L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
+    L.mapf_vtrace.argtypes = [C.POINTER(MapfVtraceArgs), vp]
     L.mapf_cte_eval_accumulate.argtypes = [C.POINTER(MapfCteEvalArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
@@ -297,7 +307,7 @@ EXPORTS = (
     "mapf_policy_act_per_agent", "mapf_lstm_policy_act_per_agent",
     "mapf_cte_policy_weights_nbytes", "mapf_cte_policy_pack_weights", "mapf_cte_policy_act",
     "mapf_cte_lstm_policy_weights_nbytes", "mapf_cte_lstm_policy_pack_weights", "mapf_cte_lstm_policy_act",
-    "mapf_cte_eval_accumulate",
+    "mapf_cte_eval_accumulate", "mapf_vtrace",
 )
 
 

@@ -10,10 +10,12 @@
 #include "mapf_policy_kernel.cuh"
 #include "mapf_policy_lstm_kernel.cuh"
 #include "mapf_eval_kernel.cuh"
+#include "mapf_vtrace_kernel.cuh"
 #include "mapf_pack_kernel.cuh"
 #include "mapf_host_unpack.h"
 
 #include <chrono>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -1923,6 +1925,35 @@ int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, co
     const long long BN = (long long)B * N;
     mapf::mapf_gae_kernel<<<(unsigned)((BN + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         rewards, values, dones, last_value, adv, ret, T, BN, N, gamma, lam);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_vtrace(const mapf_vtrace_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "vtrace: null argument");
+    if (!a->rewards || !a->behaviour_logp || !a->dones || !a->bootstrap_value || !a->target_logp || !a->values || !a->vs ||
+        !a->pg_advantages)
+        return fail(MAPF_ERR_INVALID_ARG, "vtrace: null required pointer");
+    if (a->T < 1 || a->M < 1 || a->num_agents < 1)
+        return fail(MAPF_ERR_INVALID_ARG, "vtrace: T %d, M %lld and num_agents %d must be >= 1", a->T, (long long)a->M,
+                    a->num_agents);
+    if (a->num_columns < 1 || a->num_columns % a->num_agents != 0)
+        return fail(MAPF_ERR_INVALID_ARG, "vtrace: num_columns %lld is not a positive multiple of num_agents %d",
+                    (long long)a->num_columns, a->num_agents);
+    if (!a->columns && a->M != a->num_columns)
+        return fail(MAPF_ERR_INVALID_ARG, "vtrace: columns is NULL but M %lld != num_columns %lld", (long long)a->M,
+                    (long long)a->num_columns);
+    if (!(a->gamma >= 0.f && a->gamma <= 1.f)) return fail(MAPF_ERR_INVALID_ARG, "vtrace: gamma %g outside [0, 1]", a->gamma);
+    if (!(std::isfinite(a->clip_rho) && a->clip_rho > 0.f) || !(std::isfinite(a->clip_pg_rho) && a->clip_pg_rho > 0.f))
+        return fail(MAPF_ERR_INVALID_ARG, "vtrace: clip_rho %g and clip_pg_rho %g must be finite and positive", a->clip_rho,
+                    a->clip_pg_rho);
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "vtrace: reserved is %d, must be 0", a->reserved);
+    const long long blocks = (a->M + mapf::VTRACE_THREADS - 1) / mapf::VTRACE_THREADS;
+    if (blocks > 0x7fffffffLL) return fail(MAPF_ERR_UNSUPPORTED, "vtrace: M %lld needs more than 2^31 - 1 blocks", (long long)a->M);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    mapf::mapf_vtrace_kernel<<<(unsigned)blocks, mapf::VTRACE_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }

@@ -3,8 +3,8 @@ env's output channels and sampled in one launch (``mapf_policy_act``: bf16 tenso
 same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a greedy (argmax) mode for evaluation and a
 per-agent variant (one weight set per agent: ``mapf_policy_act_per_agent`` / ``mapf_lstm_policy_act_per_agent``), the
 centralised CTE policy over the single-agent view with one joint draw (``mapf_cte_policy_act``) and its recurrent
-variant (``mapf_cte_lstm_policy_act``), and GAE as a backwards
-scan (``mapf_gae``).  Thin ctypes wrappers; torch is the allocator / stream provider.
+variant (``mapf_cte_lstm_policy_act``), GAE as a backwards
+scan (``mapf_gae``) and IMPALA's V-trace targets as another (``mapf_vtrace``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
 
@@ -469,3 +469,39 @@ def gae(rewards, values, dones, last_value, gamma: float = 0.99, lam: float = 0.
     nat.check(nat.lib().mapf_gae(p(rewards.contiguous()), p(values.contiguous()), p(d), p(last_value.contiguous()), p(adv),
                                  p(ret), int(T), int(B), int(N), C.c_float(gamma), C.c_float(lam), st))
     return adv, ret
+
+
+def vtrace(target_logp, behaviour_logp, values, rewards, dones, bootstrap_value, *, columns=None, gamma: float = 0.99,
+           clip_rho: float = 1.0, clip_pg_rho: float = 1.0):
+    """V-trace targets with the ``mapf_vtrace`` scan on the current stream: (vs, pg_advantages), float32 [T,M].
+    ``rewards`` / ``behaviour_logp``: float32 [T,B,N] or [T,B] (the batch's own rows); ``dones``: [T,B] bool / uint8;
+    ``bootstrap_value``: [B,N] or [B]; ``target_logp`` / ``values``: float32 [T,M], column m of batch column
+    ``columns[m]`` (int64 [M], flat index b * N + n; None: all B*N columns in order).  :func:`impala.vtrace` is the
+    same recurrence in PyTorch."""
+    T, B = int(rewards.shape[0]), int(rewards.shape[1])
+    N = int(rewards.shape[2]) if rewards.dim() == 3 else 1
+    if rewards.dim() not in (2, 3) or tuple(behaviour_logp.shape) != tuple(rewards.shape):
+        raise ValueError(f"rewards {tuple(rewards.shape)} and behaviour_logp {tuple(behaviour_logp.shape)} must be one "
+                         "[T,B,N] or [T,B] shape")
+    if tuple(dones.shape) != (T, B) or bootstrap_value.numel() != B * N:
+        raise ValueError(f"dones {tuple(dones.shape)} must be [T,B] = [{T},{B}] and bootstrap_value "
+                         f"{tuple(bootstrap_value.shape)} hold B*N = {B * N} values")
+    M = B * N if columns is None else int(columns.numel())
+    if tuple(target_logp.shape) != (T, M) or tuple(values.shape) != (T, M):
+        raise ValueError(f"target_logp {tuple(target_logp.shape)} and values {tuple(values.shape)} must be [T,M] = [{T},{M}]")
+    floats = [x.contiguous() for x in (target_logp, behaviour_logp, values, rewards, bootstrap_value)]
+    dev = rewards.device
+    if any(x.dtype != torch.float32 or x.device != dev or not x.is_cuda for x in floats):
+        raise ValueError(f"the V-trace kernel takes float32 tensors on one CUDA device (got {[(x.dtype, x.device) for x in floats]})")
+    tl, mu, v, r, boot = floats
+    d = dones.contiguous()
+    d = d.view(torch.uint8) if d.dtype == torch.bool else d if d.dtype == torch.uint8 else (d != 0).to(torch.uint8)
+    cols = None if columns is None else columns.to(device=dev, dtype=torch.int64).contiguous()
+    vs, pg = torch.empty((T, M), device=dev), torch.empty((T, M), device=dev)
+    p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+    a = nat.MapfVtraceArgs(T=T, num_agents=N, num_columns=B * N, M=M, columns=p(cols), rewards=p(r),
+                           behaviour_logp=p(mu), dones=p(d), bootstrap_value=p(boot), target_logp=p(tl), values=p(v),
+                           vs=p(vs), pg_advantages=p(pg), gamma=float(gamma), clip_rho=float(clip_rho),
+                           clip_pg_rho=float(clip_pg_rho), reserved=0)
+    nat.check(nat.lib().mapf_vtrace(C.byref(a), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+    return vs, pg

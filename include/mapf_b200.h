@@ -659,6 +659,38 @@ int mapf_cte_eval_accumulate(const mapf_cte_eval_args *args, void *stream);
 int mapf_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_value, float *adv,
              float *ret, int32_t T, int64_t B, int32_t N, float gamma, float lam, void *stream);
 
+/* V-trace targets (IMPALA, Espeholt et al. 2018; RLlib's vtrace_torch recurrence with c_bar fixed at 1) over M time
+ * columns of a rollout, one thread per column, a backwards scan in f32.  A batch column is one (env, agent) series,
+ * col = env * num_agents + agent (num_agents = 1 for the CTE view).  Processed column m reads batch column
+ * col = columns[m] (columns == NULL: col = m, M = num_columns).  For t = T-1 .. 0, with mu / pi the behaviour / target
+ * log-probabilities, V the values, r the rewards, d the episode ends (terminated or truncated) and V_T the bootstrap:
+ *   rho_t = exp(pi_t - mu_t); rho_bar_t = min(clip_rho, rho_t); c_t = min(1, rho_t); rho_pg_t = min(clip_pg_rho, rho_t)
+ *   disc_t = gamma * (1 - d_t); delta_t = rho_bar_t * (r_t + disc_t * V_{t+1} - V_t)      (V_{t+1} = V_T at t = T-1)
+ *   acc_T = 0; acc_t = delta_t + disc_t * c_t * acc_{t+1}; vs_t = V_t + acc_t
+ *   pg_adv_t = rho_pg_t * (r_t + disc_t * vs_{t+1} - V_t)                                  (vs_T = V_T)
+ * Every pointer is a device pointer; all are required except `columns`.  Null required pointers, T < 1, M < 1,
+ * num_agents < 1, num_columns not a positive multiple of num_agents, columns == NULL with M != num_columns, gamma
+ * outside [0, 1], a non-finite or non-positive clip threshold and reserved != 0 give MAPF_ERR_INVALID_ARG, all before
+ * any device work.  On the device, a column id outside [0, num_columns) writes NaN to that column's outputs and reads
+ * no input. */
+typedef struct mapf_vtrace_args {
+    int32_t T, num_agents;          /* time steps; columns per env (1 for the CTE view) */
+    int64_t num_columns, M;         /* batch columns (B * num_agents); processed columns */
+    const int64_t *columns;         /* [M] batch column ids, or NULL for 0 .. M-1 */
+    const float *rewards;           /* [T, num_columns] */
+    const float *behaviour_logp;    /* [T, num_columns] */
+    const uint8_t *dones;           /* [T, num_columns / num_agents], 0 / nonzero (torch bool bytes as they are) */
+    const float *bootstrap_value;   /* [num_columns] value of the observation after step T-1 */
+    const float *target_logp;       /* [T, M] */
+    const float *values;            /* [T, M] */
+    float *vs;                      /* [T, M] out */
+    float *pg_advantages;           /* [T, M] out */
+    float gamma, clip_rho, clip_pg_rho;
+    int32_t reserved;               /* must be 0 */
+} mapf_vtrace_args;
+
+int mapf_vtrace(const mapf_vtrace_args *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,6 +1,6 @@
 """Timings of the kernels next to the hot path (CUDA events, warm-up, L2-sized working sets): the fused policy
-kernels (MLP and LSTM-64, shared and per-agent; the CTE MLP and LSTM-64), the GAE scan, the single-agent (CTE) step.  Prints one JSON object.
-`python tools/bench_aux.py`"""
+kernels (MLP and LSTM-64, shared and per-agent; the CTE MLP and LSTM-64), the GAE scan, the V-trace scan, the single-agent (CTE) step.  Prints one JSON object.
+`python tools/bench_aux.py` (every entry) or `python tools/bench_aux.py vtrace` (the V-trace entry alone)"""
 import json
 import sys
 from pathlib import Path
@@ -148,7 +148,44 @@ def cte_lstm_policy_act_entry(B, N=16):
             "frac_of_hbm_6450GBps": gbps / (hbm_tbs * 1e3), "frac_of_bf16_2250TFLOPs": tflops / bf16_tflops}
 
 
+def vtrace_entry(T=64, B=65536, N=16):
+    """The V-trace scan (mapf_vtrace) at C3: the identity launch over [T, B*N] (24 B per column-step -- rewards,
+    behaviour and target logp, values in, vs and pg_advantages out -- plus T*B bytes of dones: 1.6 GB, more than L2),
+    and the learner-shaped launch, 1024 // T = 16 gathered columns of the same batch."""
+    from dl_reference_models_b200 import impala
+
+    g = torch.Generator(device="cuda").manual_seed(0)
+    mu, r = torch.randn(T, B, N, device="cuda", generator=g) - 1.5, torch.randn(T, B, N, device="cuda", generator=g)
+    dones = torch.rand(T, B, device="cuda", generator=g) < 0.01
+    boot = torch.randn(B, N, device="cuda", generator=g)
+    pi, v = mu.reshape(T, -1) + 0.1 * torch.randn(T, B * N, device="cuda", generator=g), torch.randn(T, B * N, device="cuda", generator=g)
+    s = timed(lambda: policy_kernels.vtrace(pi, mu, v, r, dones, boot), 20)
+    nbytes = 24 * T * B * N + T * B
+    hbm_tbs = 6.45   # SURVEY 8d measured copy bandwidth
+    cols = torch.randperm(B * N, device="cuda", generator=g)[:1024 // T]
+    pic, vc = pi[:, cols].contiguous(), v[:, cols].contiguous()
+    sg = timed(lambda: policy_kernels.vtrace(pic, mu, vc, r, dones, boot, columns=cols), 500)
+    st = timed(lambda: impala.vtrace(pic, mu, vc, r, dones, boot, columns=cols), 50)
+    return {"identity": {"T": T, "columns": B * N, "us_per_launch": s * 1e6, "bytes": nbytes, "GBps": nbytes / s / 1e9,
+                         "hbm_floor_us_at_6450GBps": nbytes / (hbm_tbs * 1e12) * 1e6,
+                         "frac_of_hbm_6450GBps": nbytes / s / 1e9 / (hbm_tbs * 1e3)},
+            "gathered": {"T": T, "columns": cols.numel(), "us_per_launch": sg * 1e6, "torch_vtrace_us": st * 1e6}}
+
+
+def gpu_name():
+    import subprocess
+
+    try:
+        return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i",
+                               "0"], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        return f"nvidia-smi not readable: {exc}"
+
+
 def main():
+    if sys.argv[1:] == ["vtrace"]:
+        print(json.dumps({"vtrace": vtrace_entry(), "gpu": gpu_name()}))
+        return
     res = {}
     B, N = 65536, 16
     cfg = {"num_agents": N, "sensor_range": 2, "steps_per_episode": 256, "lifelong_mapf": True, "seed": 999,
@@ -279,6 +316,7 @@ def main():
     del cte
     res["cte_policy_act"] = cte_policy_act_entry(B)
     res["cte_lstm_policy_act"] = cte_lstm_policy_act_entry(B)
+    res["vtrace"] = vtrace_entry()
     try:
         import subprocess
 
