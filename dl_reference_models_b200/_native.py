@@ -19,7 +19,8 @@ LIB_PATH = Path(os.environ.get("MAPF_B200_LIB", PKG / "libmapf_b200.so"))
 SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_kernel.cuh", CSRC / "mapf_pair_kernel.cuh", CSRC / "mapf_cte_kernel.cuh", CSRC / "mapf_policy_kernel.cuh",
            CSRC / "mapf_policy_lstm_kernel.cuh", CSRC / "mapf_eval_kernel.cuh", CSRC / "mapf_cte_policy_kernel.cuh",
            CSRC / "mapf_cte_lstm_policy_kernel.cuh", CSRC / "mapf_cte_trunk.inc",
-           CSRC / "mapf_cte_heads.inc", CSRC / "mapf_vtrace_kernel.cuh", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
+           CSRC / "mapf_cte_heads.inc", CSRC / "mapf_vtrace_kernel.cuh", CSRC / "mapf_q_kernel.cuh",
+           CSRC / "mapf_replay_kernel.cuh", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
 MAX_AGENTS = 32
@@ -169,6 +170,40 @@ class MapfVtraceArgs(C.Structure):
         ("gamma", C.c_float), ("clip_rho", C.c_float), ("clip_pg_rho", C.c_float), ("reserved", C.c_int32)]
 
 
+class MapfQActArgs(C.Structure):
+    """mapf_q_act_args of include/mapf_b200.h (fused dueling Q MLP + epsilon-greedy choice)."""
+
+    _fields_ = [
+        ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("v2", C.c_int32), ("feature_dim", C.c_int32),
+        ("no_masking", C.c_int32), ("epsilon", C.c_float),
+        ("seed", C.c_uint64), ("counter", C.c_uint64), ("env_id_base", C.c_int64),
+    ] + [(k, C.c_void_p) for k in ("local_obs", "goal_delta", "blocking_prev", "action_mask", "weights", "actions",
+                                   "q_out")] + [("reserved", C.c_int32)]
+
+
+class MapfReplayTree(C.Structure):
+    """mapf_replay_tree of include/mapf_b200.h (the prioritized replay sum tree's shape and device arrays)."""
+
+    _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("capacity", C.c_int32)] + [
+        (k, C.c_void_p) for k in ("leaves", "sums", "mins", "max_priority")]
+
+
+class MapfReplayAdvanceArgs(C.Structure):
+    _fields_ = [("tree", MapfReplayTree), ("complete", C.c_int32), ("clear", C.c_int32), ("alpha", C.c_float),
+                ("reserved", C.c_int32)]
+
+
+class MapfReplaySampleArgs(C.Structure):
+    _fields_ = [("tree", MapfReplayTree), ("M", C.c_int64), ("seed", C.c_uint64), ("counter", C.c_uint64),
+                ("beta", C.c_float), ("per_agent", C.c_int32)] + [
+        (k, C.c_void_p) for k in ("indices", "weights", "uniforms")] + [("reserved", C.c_int32)]
+
+
+class MapfReplayUpdateArgs(C.Structure):
+    _fields_ = [("tree", MapfReplayTree), ("M", C.c_int64), ("indices", C.c_void_p), ("td_abs", C.c_void_p),
+                ("alpha", C.c_float), ("reserved", C.c_int32)]
+
+
 class MapfError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"libmapf_b200 error {code}: {message}")
@@ -282,12 +317,19 @@ def lib():
     L.mapf_eval_accumulate.argtypes = [C.POINTER(MapfEvalArgs), vp]
     L.mapf_vtrace.argtypes = [C.POINTER(MapfVtraceArgs), vp]
     L.mapf_cte_eval_accumulate.argtypes = [C.POINTER(MapfCteEvalArgs), vp]
+    L.mapf_q_act.argtypes = [C.POINTER(MapfQActArgs), vp]
+    L.mapf_q_act_per_agent.argtypes = [C.POINTER(MapfQActArgs), vp]
+    L.mapf_replay_tree_leaves.argtypes = [i32, i32, i32]
+    L.mapf_replay_tree_leaves.restype = i64
+    L.mapf_replay_advance.argtypes = [C.POINTER(MapfReplayAdvanceArgs), vp]
+    L.mapf_replay_sample.argtypes = [C.POINTER(MapfReplaySampleArgs), vp]
+    L.mapf_replay_update.argtypes = [C.POINTER(MapfReplayUpdateArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
         if name not in ("mapf_version", "mapf_last_error", "mapf_launch_count", "mapf_policy_weights_nbytes",
                         "mapf_lstm_policy_weights_nbytes", "mapf_cte_policy_weights_nbytes",
-                        "mapf_cte_lstm_policy_weights_nbytes"):
+                        "mapf_cte_lstm_policy_weights_nbytes", "mapf_replay_tree_leaves"):
             getattr(L, name).restype = C.c_int
     _lib = L
     return L
@@ -308,6 +350,8 @@ EXPORTS = (
     "mapf_cte_policy_weights_nbytes", "mapf_cte_policy_pack_weights", "mapf_cte_policy_act",
     "mapf_cte_lstm_policy_weights_nbytes", "mapf_cte_lstm_policy_pack_weights", "mapf_cte_lstm_policy_act",
     "mapf_cte_eval_accumulate", "mapf_vtrace",
+    "mapf_q_act", "mapf_q_act_per_agent", "mapf_replay_tree_leaves", "mapf_replay_advance", "mapf_replay_sample",
+    "mapf_replay_update",
 )
 
 

@@ -11,6 +11,8 @@
 #include "mapf_policy_lstm_kernel.cuh"
 #include "mapf_eval_kernel.cuh"
 #include "mapf_vtrace_kernel.cuh"
+#include "mapf_q_kernel.cuh"
+#include "mapf_replay_kernel.cuh"
 #include "mapf_pack_kernel.cuh"
 #include "mapf_host_unpack.h"
 
@@ -1954,6 +1956,122 @@ int mapf_vtrace(const mapf_vtrace_args *a, void *stream) {
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
         return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
     mapf::mapf_vtrace_kernel<<<(unsigned)blocks, mapf::VTRACE_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+static int q_act_launch(const mapf_q_act_args *a, bool per_agent, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "q_act: null argument");
+    if (!a->local_obs || !a->goal_delta || !a->action_mask || !a->weights || !a->actions)
+        return fail(MAPF_ERR_INVALID_ARG, "q_act: local_obs, goal_delta, action_mask, weights and actions are required");
+    if (a->num_envs < 1 || a->num_agents < 1)
+        return fail(MAPF_ERR_INVALID_ARG, "q_act: num_envs %d and num_agents %d must be >= 1", a->num_envs, a->num_agents);
+    if (!(a->epsilon >= 0.f && a->epsilon <= 1.f)) return fail(MAPF_ERR_INVALID_ARG, "q_act: epsilon %g outside [0, 1]", a->epsilon);
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "q_act: reserved is %d, must be 0", a->reserved);
+    const int kc1 = policy_kc1(a->feature_dim);
+    if (!kc1 || a->v2 < 1 || a->feature_dim != a->v2 + 2 + (a->blocking_prev ? 1 : 0))
+        return fail(MAPF_ERR_UNSUPPORTED, "q_act: feature_dim %d does not match v2 %d (+2 goal delta, +1 pressure) or exceeds 64",
+                    a->feature_dim, a->v2);
+    if (per_agent && a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "q_act: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    const int threads = 256, warps = threads / 32;
+    const size_t smem = (size_t)mapf_policy_weights_nbytes(a->feature_dim) + (size_t)warps * mapf::pol_warp_bytes(kc1, a->v2);
+    const long long tiles = per_agent ? ((long long)a->num_envs + 31) / 32 * a->num_agents
+                                      : ((long long)a->num_envs * a->num_agents + 31) / 32;
+    long long blocks = (tiles + warps - 1) / warps;
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    void (*const kernels[2][2])(const mapf_q_act_args) = {
+        {mapf::mapf_q_act_kernel<2, false>, mapf::mapf_q_act_kernel<4, false>},
+        {mapf::mapf_q_act_kernel<2, true>, mapf::mapf_q_act_kernel<4, true>}};
+    const auto kernel = kernels[per_agent][kc1 == 4];
+    CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<(unsigned)blocks, threads, smem, static_cast<cudaStream_t>(stream)>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_q_act(const mapf_q_act_args *a, void *stream) { return q_act_launch(a, false, stream); }
+int mapf_q_act_per_agent(const mapf_q_act_args *a, void *stream) { return q_act_launch(a, true, stream); }
+
+// the leaf count L = N' K' B' of a ring shape, or an error (the shape checks every replay entry point shares)
+static int64_t replay_leaves(int32_t B, int32_t N, int32_t K, const char *who) {
+    if (B < 1 || N < 1 || K < 2)
+        return fail(MAPF_ERR_INVALID_ARG, "%s: num_envs %d and num_agents %d must be >= 1 and capacity %d >= 2", who, B, N, K);
+    const int bits = mapf::replay_log2_ceil(B) + mapf::replay_log2_ceil(K) + mapf::replay_log2_ceil(N);
+    if (bits > 40) return fail(MAPF_ERR_UNSUPPORTED, "%s: 2^%d leaves", who, bits);
+    return (int64_t)1 << bits;
+}
+
+int64_t mapf_replay_tree_leaves(int32_t B, int32_t N, int32_t K) { return replay_leaves(B, N, K, "replay"); }
+
+static int replay_tree_check(const mapf_replay_tree &t, const char *who) {
+    const int64_t L = replay_leaves(t.num_envs, t.num_agents, t.capacity, who);
+    if (L < 0) return (int)L;
+    if (!t.leaves || !t.sums || !t.mins || !t.max_priority) return fail(MAPF_ERR_INVALID_ARG, "%s: null tree array", who);
+    return MAPF_OK;
+}
+
+static int replay_exponent_check(float x, const char *name, const char *who) {
+    if (!(std::isfinite(x) && x >= 0.f)) return fail(MAPF_ERR_INVALID_ARG, "%s: %s %g must be finite and >= 0", who, name, x);
+    return MAPF_OK;
+}
+
+static int device_check() {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
+        return fail(MAPF_ERR_CUDA, "no CUDA device (libmapf_b200 has no CPU fallback)");
+    return MAPF_OK;
+}
+
+int mapf_replay_advance(const mapf_replay_advance_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "replay_advance: null argument");
+    if (int rc = replay_tree_check(a->tree, "replay_advance")) return rc;
+    if (int rc = replay_exponent_check(a->alpha, "alpha", "replay_advance")) return rc;
+    const int K = a->tree.capacity;
+    if (a->complete < 0 || a->complete >= K || a->clear < 0 || a->clear >= K || a->complete == a->clear)
+        return fail(MAPF_ERR_INVALID_ARG, "replay_advance: complete %d and clear %d must be distinct slots of [0, %d)",
+                    a->complete, a->clear, K);
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "replay_advance: reserved is %d, must be 0", a->reserved);
+    if (int rc = device_check()) return rc;
+    const long long Bp = 1ll << mapf::replay_log2_ceil(a->tree.num_envs);
+    const int ch = (int)(Bp < mapf::REPLAY_CHUNK ? Bp : mapf::REPLAY_CHUNK);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    mapf::mapf_replay_advance_kernel<<<(unsigned)(2 * a->tree.num_agents * (Bp / ch)), ch, 0, st>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    mapf::mapf_replay_advance_top_kernel<<<1, mapf::REPLAY_THREADS, 0, st>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_replay_sample(const mapf_replay_sample_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "replay_sample: null argument");
+    if (int rc = replay_tree_check(a->tree, "replay_sample")) return rc;
+    if (!a->indices || !a->weights) return fail(MAPF_ERR_INVALID_ARG, "replay_sample: indices and weights are required");
+    if (a->M < 1) return fail(MAPF_ERR_INVALID_ARG, "replay_sample: M %lld must be >= 1", (long long)a->M);
+    if (int rc = replay_exponent_check(a->beta, "beta", "replay_sample")) return rc;
+    if (a->per_agent != 0 && a->per_agent != 1)
+        return fail(MAPF_ERR_INVALID_ARG, "replay_sample: per_agent %d is neither 0 nor 1", a->per_agent);
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "replay_sample: reserved is %d, must be 0", a->reserved);
+    const long long blocks = (a->M + 255) / 256;
+    if (blocks > 0x7fffffffLL) return fail(MAPF_ERR_UNSUPPORTED, "replay_sample: M %lld is too large", (long long)a->M);
+    if (int rc = device_check()) return rc;
+    mapf::mapf_replay_sample_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(*a);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_replay_update(const mapf_replay_update_args *a, void *stream) {
+    if (!a) return fail(MAPF_ERR_INVALID_ARG, "replay_update: null argument");
+    if (int rc = replay_tree_check(a->tree, "replay_update")) return rc;
+    if (!a->indices || !a->td_abs) return fail(MAPF_ERR_INVALID_ARG, "replay_update: indices and td_abs are required");
+    if (a->M < 1) return fail(MAPF_ERR_INVALID_ARG, "replay_update: M %lld must be >= 1", (long long)a->M);
+    if (int rc = replay_exponent_check(a->alpha, "alpha", "replay_update")) return rc;
+    if (a->reserved != 0) return fail(MAPF_ERR_INVALID_ARG, "replay_update: reserved is %d, must be 0", a->reserved);
+    if (int rc = device_check()) return rc;
+    mapf::mapf_replay_update_kernel<<<1, mapf::REPLAY_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a);
     CUDA_TRY(cudaGetLastError());
     return MAPF_OK;
 }

@@ -4,7 +4,8 @@ same for the LSTM-64 recurrent policy (``mapf_lstm_policy_act``), both with a gr
 per-agent variant (one weight set per agent: ``mapf_policy_act_per_agent`` / ``mapf_lstm_policy_act_per_agent``), the
 centralised CTE policy over the single-agent view with one joint draw (``mapf_cte_policy_act``) and its recurrent
 variant (``mapf_cte_lstm_policy_act``), GAE as a backwards
-scan (``mapf_gae``) and IMPALA's V-trace targets as another (``mapf_vtrace``).  Thin ctypes wrappers; torch is the allocator / stream provider.
+scan (``mapf_gae``), IMPALA's V-trace targets as another (``mapf_vtrace``) and DQN's epsilon-greedy dueling Q head
+over the MLP (``mapf_q_act``).  Thin ctypes wrappers; torch is the allocator / stream provider.
 """
 from __future__ import annotations
 
@@ -126,6 +127,44 @@ class FusedPolicy:
             logits_out=p(logits_out), features_out=p(features_out), action_mask_out=p(mask_out))
         nat.check(self._act(C.byref(args), env._stream()))
         return self.actions, logp, value
+
+
+class FusedQPolicy(FusedPolicy):
+    """The same MLP read as a dueling Q network for DQN (``mapf_q_act`` / ``mapf_q_act_per_agent``, :attr:`entry`): the
+    logits head is the advantage A, the value head V, Q = V + A - mean(A), masked to FLOAT_MIN where an action is
+    illegal, then an epsilon-greedy choice (one Philox block per agent, keyed apart from the policy draws).  Packing,
+    :meth:`refresh` and the accepted modules are :class:`FusedPolicy`'s."""
+
+    def __init__(self, policy, env, seed: int | None = None):
+        super().__init__(policy, env, seed)
+        self.entry = "mapf_q_act_per_agent" if self.per_agent else "mapf_q_act"
+        self._act = getattr(self._lib, self.entry)
+
+    def args(self, channels: dict, epsilon: float, actions: torch.Tensor, q_out: torch.Tensor | None = None) -> nat.MapfQActArgs:
+        """The argument block of one launch (counter 0; set ``.counter`` before launching): ``channels`` maps
+        local_obs / goal_delta / blocking_prev / action_mask to device tensors, ``actions`` int8 [B,N] receives the
+        choice, ``q_out`` (optional) float32 [B,N,5] the masked Q."""
+        env = self.env
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+        return nat.MapfQActArgs(
+            num_envs=env.B, num_agents=env.N, v2=env.V * env.V, feature_dim=self.F,
+            no_masking=int(bool(self.policy.no_masking)), epsilon=float(epsilon), seed=self.seed, counter=0,
+            env_id_base=int(env.cfg.env_id_base), local_obs=p(channels["local_obs"]), goal_delta=p(channels["goal_delta"]),
+            blocking_prev=p(channels["blocking_prev"]) if self.with_bp else None, action_mask=p(channels["action_mask"]),
+            weights=p(self._dev), actions=p(actions), q_out=p(q_out), reserved=0)
+
+    def act(self, out, epsilon: float, q_out: torch.Tensor | None = None, actions: torch.Tensor | None = None):
+        """One launch on ``out`` (the env's StepOutput, or a dict of its observation channels): masked dueling Q, then
+        with probability ``epsilon`` a uniform legal action, otherwise the first argmax of the masked Q.  Returns the
+        int8 [B,N] actions (``actions``, default :attr:`actions`); ``q_out`` [B,N,5] receives the masked Q."""
+        ch = out if isinstance(out, dict) else {k: getattr(out, k) for k in ("local_obs", "goal_delta", "blocking_prev",
+                                                                             "action_mask")}
+        actions = self.actions if actions is None else actions
+        a = self.args(ch, epsilon, actions, q_out)
+        self.counter += 1
+        a.counter = self.counter
+        nat.check(self._act(C.byref(a), self.env._stream()))
+        return actions
 
 
 class FusedRecurrentPolicy:

@@ -38,11 +38,15 @@ class ActionMaskPolicy(nn.Module):
         self.value = nn.Linear(last, 1)
         self.no_masking = no_masking
 
+    def heads(self, features: torch.Tensor):
+        """features [..., F] float -> (unmasked logits [..., A], value [...]): the two heads as they are (DQN reads them
+        as a dueling network's advantage and value, :func:`dqn.q_values`)."""
+        z = self.trunk(features.float())
+        return self.logits(z), self.value(z).squeeze(-1)
+
     def forward(self, features: torch.Tensor, action_mask: torch.Tensor):
         """features [..., F] float, action_mask [..., A] (0/1 of any dtype) -> (masked logits, value)."""
-        z = self.trunk(features.float())
-        logits = self.logits(z)
-        value = self.value(z).squeeze(-1)
+        logits, value = self.heads(features)
         if self.no_masking:
             return logits, value
         inf_mask = torch.clamp(torch.log(action_mask.to(logits.dtype) + 1e-6), min=FLOAT_MIN)
@@ -108,14 +112,19 @@ class PerAgentActionMaskPolicy(nn.Module):
             m.value.bias.copy_(self.value_b[j])
         return m
 
-    def forward(self, features: torch.Tensor, action_mask: torch.Tensor):
-        """features [..., F] float, action_mask [..., A], flat row r of agent r % N -> (masked logits, value)."""
+    def heads(self, features: torch.Tensor):
+        """features [..., F] float, flat row r of agent r % N -> (unmasked logits [..., A], value [...])."""
         lead, N = features.shape[:-1], self.num_agents
         z = features.float().reshape(-1, N, features.shape[-1]).transpose(0, 1)   # [N, rows / N, F]
         for w, b in zip(self.trunk_w, self.trunk_b):
             z = torch.relu(agent_linear(z, w, b))
         logits = agent_linear(z, self.logits_w, self.logits_b).transpose(0, 1).reshape(*lead, -1)
         value = agent_linear(z, self.value_w, self.value_b).transpose(0, 1).reshape(lead)
+        return logits, value
+
+    def forward(self, features: torch.Tensor, action_mask: torch.Tensor):
+        """features [..., F] float, action_mask [..., A], flat row r of agent r % N -> (masked logits, value)."""
+        logits, value = self.heads(features)
         if self.no_masking:
             return logits, value
         return logits + torch.clamp(torch.log(action_mask.to(logits.dtype) + 1e-6), min=FLOAT_MIN), value

@@ -691,6 +691,108 @@ typedef struct mapf_vtrace_args {
 
 int mapf_vtrace(const mapf_vtrace_args *args, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * DQN (the reference's src/agents/dqn.py, SURVEY §2 row 6): an epsilon-greedy dueling Q kernel over the fused MLP's
+ * packed weights, and a prioritized replay sum tree on the device.
+ *
+ * mapf_q_act / mapf_q_act_per_agent: the MLP of mapf_policy_act (the same packed block, per agent: num_agents blocks)
+ * read as a dueling network: logits head = advantage A[5], value head = V, Q = V + (A - mean(A)) in f32 with the mean
+ * over all 5 actions; masked Q = Q where the mask allows the action, FLOAT_MIN (-3.4e38) elsewhere (no_masking: Q as it
+ * is).  Per agent, with one Philox block keyed (seed ^ "DQNE", env_id_base + env), counter (counter, agent): explore
+ * iff word0 * 2^-32 < epsilon, then take the k-th legal action (all 5 with no_masking), k = floor(word1 * n_legal /
+ * 2^32); otherwise the first index of the largest masked Q (torch.argmax's tie rule).  epsilon = 0 makes no Philox
+ * call.  Null required pointers (local_obs, goal_delta, action_mask, weights, actions), num_envs or num_agents < 1,
+ * epsilon outside [0, 1] or NaN and reserved != 0 give MAPF_ERR_INVALID_ARG; a feature_dim that does not match v2 (as
+ * in mapf_policy_act), and for the per-agent entry num_agents > MAPF_MAX_AGENTS, give MAPF_ERR_UNSUPPORTED; all
+ * before any device work. */
+typedef struct mapf_q_act_args {
+    int32_t num_envs, num_agents;
+    int32_t v2;           /* window cells, V * V */
+    int32_t feature_dim;  /* F = v2 + 2 + (blocking_prev ? 1 : 0), <= 64 */
+    int32_t no_masking;   /* action_mask_model.py:33: nonzero = Q unmasked, explore over all 5 actions */
+    float epsilon;        /* exploration probability in [0, 1] */
+    uint64_t seed;        /* Philox key (with env_id_base + env), counter = (counter, agent) */
+    uint64_t counter;
+    int64_t env_id_base;
+    const uint8_t *local_obs;     /* [B,N,V,V]   device, the env's outputs */
+    const float *goal_delta;      /* [B,N,2] */
+    const uint8_t *blocking_prev; /* [B,N] or NULL */
+    const int8_t *action_mask;    /* [B,N,5] */
+    const void *weights;          /* device copy of the block(s) written by mapf_policy_pack_weights */
+    int8_t *actions;              /* [B,N] chosen action */
+    float *q_out;                 /* [B,N,5] masked Q, may be NULL */
+    int32_t reserved;             /* must be 0 */
+} mapf_q_act_args;
+
+int mapf_q_act(const mapf_q_act_args *args, void *stream);
+int mapf_q_act_per_agent(const mapf_q_act_args *args, void *stream);
+
+/* Prioritized replay over a ring of `capacity` env steps (K slots) of num_envs (B) envs x num_agents (N) agents.
+ * Transition (slot k, env b, agent j) has the flat index (k * B + b) * N + j.  The tree is an implicit binary heap
+ * over L = N' K' B' leaves (N', K', B' = N, K, B rounded up to powers of two), leaves ordered (agent, slot, env): leaf
+ * (j K' + k) B' + b.  Arrays (device, allocated by the caller):
+ *   leaves [L] float32: p^alpha of a complete transition, 0 for a slot without one (never drawn) and for padding;
+ *   sums   [L] float64: node i in 1 .. L-1 holds the sum of its children 2i, 2i+1 (node L + l is leaf l);
+ *   mins   [L] float32: the minimum over the nonzero leaves below node i, +inf when there are none;
+ *   max_priority [1] float32: the largest priority (not raised to alpha) seen so far, 1.0 for a new buffer.
+ * A fresh tree is leaves 0, sums 0, mins +inf.  Agent j's transitions form the subtree of node N' + j.
+ * Every entry point refuses null pointers, num_envs, num_agents or M < 1, capacity < 2, a negative or non-finite
+ * alpha / beta and reserved != 0 with MAPF_ERR_INVALID_ARG, before any device work. */
+int64_t mapf_replay_tree_leaves(int32_t num_envs, int32_t num_agents, int32_t capacity);   /* L, or a MAPF_ERR_* */
+
+typedef struct mapf_replay_tree {
+    int32_t num_envs, num_agents, capacity;
+    float *leaves;
+    double *sums;
+    float *mins;
+    float *max_priority;
+} mapf_replay_tree;
+
+/* One env step of the ring: every (b, j) leaf of slot `complete` becomes max_priority^alpha, every leaf of slot `clear`
+ * becomes 0, then the nodes above them are recomputed.  Deterministic: every node is the sum (minimum) of its two
+ * children, with no float atomics.  complete and clear must differ and lie in [0, capacity) (MAPF_ERR_INVALID_ARG). */
+typedef struct mapf_replay_advance_args {
+    mapf_replay_tree tree;
+    int32_t complete, clear;
+    float alpha;
+    int32_t reserved;             /* must be 0 */
+} mapf_replay_advance_args;
+
+/* M i.i.d. proportional draws (RLlib's _sample_proportional): u in [0, 1) from one Philox block keyed (seed ^ "PRPS",
+ * draw), counter (counter); target = u * total; descend from the root to the first leaf whose prefix sum exceeds the
+ * target.  per_agent: draw i descends from agent (i mod N)'s subtree, with that agent's total and minimum.  Writes
+ * the transition's flat index and the importance weight w = (P(i) n)^-beta / ((p_min / total) n)^-beta
+ * = (p_i / p_min)^-beta, computed in f64 (n cancels); `uniforms` (optional) receives u.  An empty (sub)tree writes
+ * index -1 and weight 0. */
+typedef struct mapf_replay_sample_args {
+    mapf_replay_tree tree;
+    int64_t M;
+    uint64_t seed, counter;
+    float beta;
+    int32_t per_agent;
+    int64_t *indices;             /* [M] out */
+    float *weights;               /* [M] out */
+    double *uniforms;             /* [M] out, may be NULL */
+    int32_t reserved;             /* must be 0 */
+} mapf_replay_sample_args;
+
+/* New priorities for M transitions: leaf = (|delta| + 1e-6)^alpha for every in-range index whose leaf is nonzero
+ * (out-of-range indices and transitions of cleared slots are skipped; among duplicates the largest value is kept, so
+ * the result does not depend on thread order), max_priority = max(max_priority, |delta| + 1e-6) over those, then the
+ * ancestors are recomputed level by level.  One block. */
+typedef struct mapf_replay_update_args {
+    mapf_replay_tree tree;
+    int64_t M;
+    const int64_t *indices;       /* [M] flat transition indices */
+    const float *td_abs;          /* [M] |TD error| */
+    float alpha;
+    int32_t reserved;             /* must be 0 */
+} mapf_replay_update_args;
+
+int mapf_replay_advance(const mapf_replay_advance_args *args, void *stream);
+int mapf_replay_sample(const mapf_replay_sample_args *args, void *stream);
+int mapf_replay_update(const mapf_replay_update_args *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

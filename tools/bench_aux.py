@@ -1,6 +1,7 @@
 """Timings of the kernels next to the hot path (CUDA events, warm-up, L2-sized working sets): the fused policy
-kernels (MLP and LSTM-64, shared and per-agent; the CTE MLP and LSTM-64), the GAE scan, the V-trace scan, the single-agent (CTE) step.  Prints one JSON object.
-`python tools/bench_aux.py` (every entry) or `python tools/bench_aux.py vtrace` (the V-trace entry alone)"""
+kernels (MLP and LSTM-64, shared and per-agent; the CTE MLP and LSTM-64), the GAE scan, the V-trace scan, the single-agent (CTE) step, DQN's Q kernel and replay kernels.  Prints one JSON
+object.  `python tools/bench_aux.py` (every entry), `python tools/bench_aux.py vtrace` (the V-trace entry alone) or
+`python tools/bench_aux.py dqn` (the DQN entries alone)"""
 import json
 import sys
 from pathlib import Path
@@ -172,6 +173,76 @@ def vtrace_entry(T=64, B=65536, N=16):
             "gathered": {"T": T, "columns": cols.numel(), "us_per_launch": sg * 1e6, "torch_vtrace_us": st * 1e6}}
 
 
+def dqn_entries(B=65536, N=16, K=64):
+    """DQN's kernels at C3: q_act and q_act_per_agent (epsilon 0.1) alternated with policy_act over the same 4-env
+    rotation (working set > L2), and the replay kernels on a K-slot tree of 2^26 leaves (1 GiB: leaves f32, sums f64,
+    minimums f32): advance (2 N B leaves written, plus their f64 / f32 subtree nodes), sample and update at the
+    learner's sizes (1024 draws shared, 1024 x N per agent)."""
+    from dl_reference_models_b200 import dqn
+    from dl_reference_models_b200.rollout import PerAgentActionMaskPolicy
+
+    cfg = {"num_agents": N, "sensor_range": 2, "steps_per_episode": 256, "lifelong_mapf": True, "seed": 999,
+           "grid": maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32)}
+    envs = [BatchedMapfEnv(cfg, B, "cuda:0", env_id_base=r * B) for r in range(4)]
+    outs = [e.reset() for e in envs]
+    F = envs[0].flat_obs_dim(include_action_mask=False)
+    policy = ActionMaskPolicy(F).cuda()
+    fused = [policy_kernels.FusedPolicy(policy, e) for e in envs]
+    qf = [policy_kernels.FusedQPolicy(policy, e) for e in envs]
+    pq = [policy_kernels.FusedQPolicy(PerAgentActionMaskPolicy(N, F).cuda(), e) for e in envs]
+    i = [0]
+
+    def rot(fn):
+        def run():
+            k = i[0] % 4
+            fn(k)
+            i[0] += 1
+        return run
+
+    pol, q, qp = [], [], []
+    for _ in range(2):
+        pol.append(timed(rot(lambda k: fused[k].act(outs[k])), 200))
+        q.append(timed(rot(lambda k: qf[k].act(outs[k], 0.1)), 200))
+        qp.append(timed(rot(lambda k: pq[k].act(outs[k], 0.1)), 200))
+    q_bytes = 25 + 8 + 1 + 5 + 1   # window, goal delta, pressure, mask in; int8 action out
+    flops = 2 * (28 * 64 + 64 * 64 + 64 * 6)
+    res = {"policy_act_same_run_us": min(pol) * 1e6,
+           "q_act": {"us_per_launch": min(q) * 1e6, "rounds_us": [x * 1e6 for x in q], "bytes_per_agent": q_bytes,
+                     "flops_per_agent": flops, "GBps": q_bytes * B * N / min(q) / 1e9,
+                     "TFLOPs": flops * B * N / min(q) / 1e12},
+           "q_act_per_agent": {"us_per_launch": min(qp) * 1e6, "rounds_us": [x * 1e6 for x in qp],
+                               "bytes_per_agent": q_bytes, "GBps": q_bytes * B * N / min(qp) / 1e9}}
+    for e in envs[1:]:
+        e.close()
+    buf = dqn.ReplayBuffer(envs[0], K)
+    L = buf.sums.numel()
+    t = [0]
+
+    def advance():
+        buf.advance(t[0] % K, (t[0] + 1) % K)
+        t[0] += 1
+    for _ in range(K):
+        advance()
+    buf.filled = K - 1
+    s = timed(advance, 100)
+    adv_bytes = 2 * N * B * 4 + 2 * N * B * (8 + 4)   # leaves written; about one node (f64 sum + f32 min) per leaf
+    res["replay_advance"] = {"us_per_launch": s * 1e6, "leaves": L, "tree_bytes": 16 * L, "bytes": adv_bytes,
+                             "GBps": adv_bytes / s / 1e9}
+    for name, M, per_agent in (("replay_sample", 1024, False), ("replay_sample_per_agent", 1024 * N, True)):
+        buf.per_agent = per_agent
+        s = timed(lambda: buf.sample(M), 200)
+        res[name] = {"us_per_launch": s * 1e6, "draws": M, "levels": L.bit_length() - 1,
+                     "node_reads_per_draw": 2 * (L.bit_length() - 1)}
+    buf.per_agent = False
+    for name, M in (("replay_update", 1024), ("replay_update_per_agent", 1024 * N)):
+        idx, _ = buf.sample(M)
+        td = torch.rand(M, device="cuda")
+        s = timed(lambda: buf.update_priorities(idx, td), 100)
+        res[name] = {"us_per_launch": s * 1e6, "updates": M, "node_writes": M * (L.bit_length() - 1)}
+    envs[0].close()
+    return res
+
+
 def gpu_name():
     import subprocess
 
@@ -185,6 +256,9 @@ def gpu_name():
 def main():
     if sys.argv[1:] == ["vtrace"]:
         print(json.dumps({"vtrace": vtrace_entry(), "gpu": gpu_name()}))
+        return
+    if sys.argv[1:] == ["dqn"]:
+        print(json.dumps({"dqn": dqn_entries(), "gpu": gpu_name()}))
         return
     res = {}
     B, N = 65536, 16
@@ -317,6 +391,7 @@ def main():
     res["cte_policy_act"] = cte_policy_act_entry(B)
     res["cte_lstm_policy_act"] = cte_lstm_policy_act_entry(B)
     res["vtrace"] = vtrace_entry()
+    res["dqn"] = dqn_entries()
     try:
         import subprocess
 
