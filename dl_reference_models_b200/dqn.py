@@ -165,7 +165,11 @@ class ReplayBuffer:
         cs = P.cumsum(1)
         total = cs[:, -1]
         last = torch.searchsorted(cs, total.unsqueeze(1).contiguous()).squeeze(1)   # each row's last nonzero leaf
-        pos = torch.searchsorted(cs[j], (u * total[j]).unsqueeze(1), right=True).squeeze(1)
+        # one search per row over that row's draws: gathering cs[j] would copy a whole row per draw (M x K B N f64)
+        pos = torch.empty(M, dtype=torch.int64)
+        for r in range(cs.shape[0]):
+            sel = j == r
+            pos[sel] = torch.searchsorted(cs[r], u[sel] * total[r], right=True)
         pos = torch.minimum(pos, last[j])
         if self.per_agent:
             agent, k, b = j, pos // self.B, pos % self.B
