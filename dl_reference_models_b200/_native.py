@@ -205,7 +205,7 @@ class MapfReplayUpdateArgs(C.Structure):
 
 
 class MapfPlanArgs(C.Structure):
-    """mapf_plan_args of include/mapf_b200.h (prioritized planner)."""
+    """mapf_plan_args of include/mapf_b200.h (prioritized and windowed planners)."""
 
     _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("horizon", C.c_int32), ("reserved", C.c_int32),
                 ("starts", C.c_void_p), ("goals", C.c_void_p), ("distance_table", C.c_void_p), ("workspace", C.c_void_p),
@@ -335,6 +335,7 @@ def lib():
     L.mapf_plan_workspace_bytes.argtypes = [i32, i32, i32, i32]
     L.mapf_plan_workspace_bytes.restype = i64
     L.mapf_plan_prioritized.argtypes = [vp, C.POINTER(MapfPlanArgs), vp]
+    L.mapf_plan_windowed.argtypes = [vp, C.POINTER(MapfPlanArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
@@ -363,7 +364,7 @@ EXPORTS = (
     "mapf_cte_lstm_policy_weights_nbytes", "mapf_cte_lstm_policy_pack_weights", "mapf_cte_lstm_policy_act",
     "mapf_cte_eval_accumulate", "mapf_vtrace",
     "mapf_q_act", "mapf_q_act_per_agent", "mapf_replay_tree_leaves", "mapf_replay_advance", "mapf_replay_sample",
-    "mapf_replay_update", "mapf_plan_workspace_bytes", "mapf_plan_prioritized",
+    "mapf_replay_update", "mapf_plan_workspace_bytes", "mapf_plan_prioritized", "mapf_plan_windowed",
 )
 
 

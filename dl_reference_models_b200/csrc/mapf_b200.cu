@@ -2129,7 +2129,8 @@ int64_t mapf_plan_workspace_bytes(int32_t rows, int32_t cols, int32_t num_envs, 
     return (int64_t)num_envs * mapf::plan_env_words(rows, cols, horizon) * 4;
 }
 
-int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *a, void *stream) {
+// mapf_plan_prioritized and mapf_plan_windowed: the same checks and launch shape, the kernel's mode apart
+static int plan_launch(mapf_handle *h, const mapf_plan_args *a, void *stream, bool windowed) {
     if (!h || !a) return fail(MAPF_ERR_INVALID_ARG, "plan: null argument");
     if (a->num_envs < 1 || a->num_agents < 1 || a->horizon < 1 || a->reserved != 0 || !a->starts || !a->goals ||
         !a->distance_table || !a->workspace || !a->actions || !a->arrival || !a->status)
@@ -2151,7 +2152,8 @@ int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *a, void *stream)
     const int warps = mapf::PLAN_THREADS / 32;
     long long blocks = ((long long)a->num_envs + warps - 1) / warps;
     if (blocks > (long long)sms * 16) blocks = (long long)sms * 16;   // 64 resident warps per SM; the rest loop
-    mapf::mapf_plan_kernel<<<(unsigned)blocks, mapf::PLAN_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
+    auto kernel = windowed ? mapf::mapf_plan_kernel<true> : mapf::mapf_plan_kernel<false>;
+    kernel<<<(unsigned)blocks, mapf::PLAN_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
         h->d_free_bits, h->cfg.rows, h->cfg.cols, a->num_envs, a->num_agents, a->horizon,
         reinterpret_cast<const uint32_t *>(a->starts), reinterpret_cast<const uint32_t *>(a->goals), a->distance_table,
         static_cast<uint32_t *>(a->workspace), mapf::plan_env_words(h->cfg.rows, h->cfg.cols, a->horizon), a->actions,
@@ -2160,6 +2162,10 @@ int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *a, void *stream)
     h->launches++;
     return MAPF_OK;
 }
+
+int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *a, void *stream) { return plan_launch(h, a, stream, false); }
+
+int mapf_plan_windowed(mapf_handle *h, const mapf_plan_args *a, void *stream) { return plan_launch(h, a, stream, true); }
 
 int64_t mapf_launch_count(const mapf_handle *h) { return h ? h->launches : 0; }
 

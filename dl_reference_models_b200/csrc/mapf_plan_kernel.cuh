@@ -16,6 +16,15 @@
 // F_t is stored for the backtrack, which walks from (goal, t_a) back to t = 0 taking at every step the first
 // predecessor in the action order NO_OP, UP, RIGHT, DOWN, LEFT (actions.py), so plans are deterministic.
 //
+// Windowed mode (WINDOWED = true, mapf_plan_windowed; DESIGN.md §7 N4c): the same rule with H read as the window W,
+// for rolling-horizon replanning from mid-episode states, where arrival within W is not required.  The target is the
+// goal if the distance table reaches it from the start (!= 255), else the start itself.  An agent whose target is its
+// goal arrives as above (first t <= W with the goal in F_t and t >= max(d, last[goal] + 1)) and holds it to W.  An
+// agent with no arrival searches on to t = W and ends on the cell of F_W with the smallest (d(target, cell), cell
+// index), each lane scanning its row word against the target's distance-table row and one warp min-reduce picking
+// the key; it backtracks from (end cell, W), reserves that path, last[end] = W, and gets arrival -1.  Only a wavefront
+// that empties by W (or a start / goal off the map) fails as above.  status = 1 iff every agent got a path.
+//
 // Per-env workspace (mapf_plan_workspace_bytes): R[(H+1) * rows] and F[(H+1) * rows] uint32 row words, then
 // last[R*C] int16 = the last t at which a planned agent holds the cell (-1 = never), which gives the arrival bound
 // last[goal] + 1 with one load.
@@ -36,6 +45,7 @@ __host__ __device__ inline int64_t plan_env_words(int rows, int cols, int horizo
     return (words + 3) & ~3LL;
 }
 
+template <bool WINDOWED>
 __global__ void __launch_bounds__(PLAN_THREADS) mapf_plan_kernel(
     const uint32_t *__restrict__ free_bits, int R, int C, long long B, int N, int H,
     const uint32_t *__restrict__ starts, const uint32_t *__restrict__ goals, const uint8_t *__restrict__ dist,
@@ -81,13 +91,16 @@ __global__ void __launch_bounds__(PLAN_THREADS) mapf_plan_kernel(
                 all_ok = false;
                 continue;
             }
-            const int sr = prow(s), sc = pcol(s), gr = prow(g), gc = pcol(g);
+            const int sr = prow(s), sc = pcol(s);
+            int gr = prow(g), gc = pcol(g);
             if (lane == sr) hi &= ~(1u << sc);
             const int d = dist[(long long)(gr * C + gc) * cells + sr * C + sc];
             const int lo = last[gr * C + gc] + 1;
-            const int tmin = d > lo ? d : lo;
+            // windowed: an unreachable goal makes the start the target, which is never arrived at
+            const int tmin = WINDOWED && d == 255 ? H + 1 : (d > lo ? d : lo);
             int ta = -1;
-            if (d != 255 && tmin <= H) {
+            bool end_cell = false;   // windowed: the path ends at (end cell, W) without an arrival
+            if (WINDOWED || (d != 255 && tmin <= H)) {
                 uint32_t F = lane == sr ? 1u << sc : 0u;
                 if (lane < R) Fw[lane] = F;
                 if (tmin == 0) {
@@ -112,8 +125,23 @@ __global__ void __launch_bounds__(PLAN_THREADS) mapf_plan_kernel(
                         rn = rnn;
                     }
                 }
+                if (WINDOWED && ta < 0 && __any_sync(full, F != 0u)) {
+                    // F = F_W: the end cell is its cell of least (d(target, cell), cell index)
+                    const uint8_t *drow = dist + (long long)(d == 255 ? sr * C + sc : gr * C + gc) * cells;
+                    unsigned key = 0xFFFFFFFFu;
+                    for (uint32_t f = F; f; f &= f - 1) {
+                        const unsigned cell = (unsigned)(lane * C + __ffs(f) - 1);
+                        const unsigned k = (unsigned)drow[cell] << 10 | cell;
+                        key = k < key ? k : key;
+                    }
+                    key = __reduce_min_sync(full, key) & 1023u;
+                    gr = (int)key / C;
+                    gc = (int)key % C;
+                    ta = H;
+                    end_cell = true;
+                }
             }
-            if (lane == 0) arrival[b * N + i] = (int16_t)ta;
+            if (lane == 0) arrival[b * N + i] = (int16_t)(end_cell ? -1 : ta);
             __syncwarp();
             if (ta < 0) {
                 all_ok = false;

@@ -22,6 +22,28 @@ not truncated) at step ``makespan`` = max(1, max arrival) with every agent on it
 env; :func:`plan_reference` is the PyTorch reference (any device, vectorised over envs), which is also the CPU path.
 :class:`PlannedPolicy` plays plans through :func:`evaluate.evaluate`.  ``python -m dl_reference_models_b200.planner``
 times the kernel (:func:`benchmark`).
+
+**Windowed plans** (rolling-horizon planning, RHCR, Li et al. 2021; DESIGN.md §7 N4c): :func:`plan_windowed` plans from
+the env's current positions to its current goals, lifelong envs included, with the rule above and H read as the window
+W, and does not require arrival:
+
+* the target is the goal if the distance table reaches it from the start (!= 255), else the agent's own start: an
+  agent with an unreachable goal tries to stay put and gets out of the way when it must;
+* an agent whose target is its goal arrives as above (the first t <= W with the goal in the wavefront and
+  t >= max(d, last[goal] + 1)) and holds its goal to W; ``arrival`` = t;
+* otherwise the search runs to t = W and the path ends on the cell of F_W with the smallest distance-table value
+  d(target, cell), ties to the first cell in row-major order; the agent reserves that path (last[end] = W) and gets
+  ``arrival`` -1;
+* an agent whose wavefront empties before W, or whose start or goal lies off the map, fails as above (NO_OPs, start
+  reserved for every t, env status 0); the later agents are still planned.
+
+status[b] = 1 iff every agent of env b got a path; then the W actions replay through the env's step from the planned
+state with no failed move and every agent on its planned cells -- in lifelong mode too, since goal reassignment never
+moves an agent -- and an agent that arrived stands on its goal from its arrival on.  Makespan and sum of costs are as
+above for envs where every agent arrived, -1 otherwise.  On an env where :func:`plan_prioritized` at H has status 1,
+the windowed plan at W = H has the same actions and arrivals.  :class:`ReplanningPolicy` replans every h steps and
+plays the first h actions of each plan through :func:`evaluate.evaluate`; ``python -m dl_reference_models_b200.planner
+--windowed`` measures it (:func:`benchmark_windowed`).
 """
 from __future__ import annotations
 
@@ -39,13 +61,13 @@ from .batched_env import BatchedMapfEnv
 class Plan:
     actions: torch.Tensor        # int8  [H,B,N]: action of agent n of env b at step t (NO_OP after arrival)
     arrival: torch.Tensor        # int16 [B,N]: arrival step (0 = starts on its goal), -1 = none within H
-    status: torch.Tensor         # uint8 [B]: 1 = every agent arrived (the plan replays through the env)
+    status: torch.Tensor         # uint8 [B]: 1 = every agent arrived (windowed: got a path); the plan replays
     makespan: torch.Tensor       # int32 [B]: max(1, max arrival) = the step the episode terminates at; -1 for status 0
-    sum_of_costs: torch.Tensor   # int32 [B]: sum of the arrivals; -1 for status 0
+    sum_of_costs: torch.Tensor   # int32 [B]: sum of the arrivals; -1 for status 0 (windowed: or an agent not arrived)
 
 
 def _finish(actions, arrival, status) -> Plan:
-    ok = status.bool()
+    ok = status.bool() & (arrival >= 0).all(1)
     a = arrival.to(torch.int32)
     makespan = torch.where(ok, a.amax(1).clamp(min=1), torch.full_like(a[:, 0], -1))
     soc = torch.where(ok, a.sum(1), torch.full_like(a[:, 0], -1))
@@ -61,6 +83,19 @@ def plan_prioritized(env: BatchedMapfEnv, starts=None, goals=None, horizon: int 
     if env.lifelong:
         raise ValueError("a lifelong env assigns new goals during the episode: a plan to the first goals is not a plan")
     H = int(env.cfg.steps_per_episode if horizon is None else horizon)
+    return _plan_native(env, starts, goals, H, "mapf_plan_prioritized")
+
+
+def plan_windowed(env: BatchedMapfEnv, window: int, starts=None, goals=None) -> Plan:
+    """Windowed plans of every env of ``env`` on the device (``mapf_plan_windowed``): W = ``window`` steps from
+    ``starts`` to ``goals`` (int16 [B,N,2]; default: the env's current positions and current goals), lifelong or
+    episodic.  ``actions`` is [W,B,N]; see the module docstring for what a windowed plan is."""
+    if not isinstance(env, BatchedMapfEnv):
+        raise TypeError(f"plan_windowed plans a BatchedMapfEnv; use plan_reference on the CPU (got {type(env).__name__})")
+    return _plan_native(env, starts, goals, int(window), "mapf_plan_windowed")
+
+
+def _plan_native(env: BatchedMapfEnv, starts, goals, H: int, entry: str) -> Plan:
     s = (env.state["positions"] if starts is None else torch.as_tensor(starts)).to(env.device, torch.int16).contiguous()
     g = (env.state["goals"] if goals is None else torch.as_tensor(goals)).to(env.device, torch.int16).contiguous()
     if s.ndim != 3 or s.shape[2] != 2 or s.shape != g.shape:
@@ -78,7 +113,7 @@ def plan_prioritized(env: BatchedMapfEnv, starts=None, goals=None, horizon: int 
     args = nat.MapfPlanArgs(num_envs=B, num_agents=N, horizon=H, starts=p(s), goals=p(g),
                             distance_table=p(env.distance_table()), workspace=p(ws), workspace_bytes=ws.numel(),
                             actions=p(actions), arrival=p(arrival), status=p(status))
-    nat.check(L.mapf_plan_prioritized(env._h, C.byref(args), env._stream()))
+    nat.check(getattr(L, entry)(env._h, C.byref(args), env._stream()))
     return _finish(actions, arrival, status)
 
 
@@ -90,11 +125,33 @@ def _components(grid: np.ndarray) -> np.ndarray:
     return lab
 
 
+def _distances(grid: np.ndarray) -> np.ndarray:
+    """Moves between any two cells around the obstacles, as the distance table stores them: int64 [R*C, R*C],
+    255 = unreachable (an obstacle at either end) or more than 254 moves."""
+    from scipy.sparse import coo_matrix
+    from scipy.sparse.csgraph import shortest_path
+
+    Rr, Cc = grid.shape
+    free = (grid == 0).reshape(-1)
+    idx = np.arange(Rr * Cc).reshape(Rr, Cc)
+    right = np.stack([idx[:, :-1].reshape(-1), idx[:, 1:].reshape(-1)], 1)
+    down = np.stack([idx[:-1].reshape(-1), idx[1:].reshape(-1)], 1)
+    e = np.concatenate([right, down])
+    e = e[free[e[:, 0]] & free[e[:, 1]]]
+    adj = coo_matrix((np.ones(len(e)), (e[:, 0], e[:, 1])), shape=(Rr * Cc, Rr * Cc))
+    d = shortest_path(adj, directed=False, unweighted=True)
+    d[~free, :] = np.inf
+    d[:, ~free] = np.inf
+    return np.where(np.isfinite(d) & (d <= 254), d, 255).astype(np.int64)
+
+
 @torch.no_grad()
-def plan_reference(grid, starts, goals, horizon: int, device=None) -> Plan:
+def plan_reference(grid, starts, goals, horizon: int, device=None, window: bool = False) -> Plan:
     """The planner in PyTorch, vectorised over envs (``device``: default the starts' device, else the CPU): the same
     semantics and tie rule as the kernel, bit for bit, written from the rule itself: [B, H+1, rows] planes of int64 row
-    words for R_t and F_t, and a reachability test by connected components instead of the distance table."""
+    words for R_t and F_t, and a reachability test by connected components instead of the distance table.
+    ``window=True``: the windowed plan of ``mapf_plan_windowed`` with W = ``horizon`` (targets and end cells from a
+    breadth-first distance table with the kernel's 255 cap)."""
     grid = np.ascontiguousarray(np.asarray(grid), dtype=np.uint8)
     if grid.ndim != 2 or grid.shape[0] > 32 or grid.shape[1] > 32:
         raise ValueError(f"the planner needs one map of at most 32x32 cells, got shape {grid.shape}")
@@ -108,6 +165,8 @@ def plan_reference(grid, starts, goals, horizon: int, device=None) -> Plan:
     Rr, Cc = grid.shape
     free = torch.as_tensor((((grid == 0).astype(np.int64)) << np.arange(Cc, dtype=np.int64)).sum(1), device=dev)   # [R]
     comp = torch.as_tensor(_components(grid).reshape(-1), dtype=torch.int64, device=dev)
+    dist = torch.as_tensor(_distances(grid), device=dev) if window else None
+    cell_ix = torch.arange(Rr * Cc, device=dev)
     ar = torch.arange(B, device=dev)
     one = torch.ones((), dtype=torch.int64, device=dev)
     Res = torch.zeros((B, H + 1, Rr), dtype=torch.int64, device=dev)
@@ -128,14 +187,17 @@ def plan_reference(grid, starts, goals, horizon: int, device=None) -> Plan:
         m = on_map[:, i]
         sr, sc = sr_all[:, i].clamp(0, Rr - 1), sc_all[:, i].clamp(0, Cc - 1)
         gr, gc = gr_all[:, i].clamp(0, Rr - 1), gc_all[:, i].clamp(0, Cc - 1)
-        sbit, gbit = one << sc, one << gc
+        sbit = one << sc
         hi[ar[m], sr[m]] &= ~sbit[m]
         s_cell, g_cell = sr * Cc + sc, gr * Cc + gc
-        reach = m & (comp[s_cell] > 0) & (comp[s_cell] == comp[g_cell])
+        if window:   # the goal is the target where the table reaches it; the search runs for every agent on the map
+            reach = m & (dist[g_cell, s_cell] != 255)
+        else:
+            reach = m & (comp[s_cell] > 0) & (comp[s_cell] == comp[g_cell])
         lo = last[ar, g_cell] + 1
         ta = torch.full((B,), -1, dtype=torch.int64, device=dev)
         ta[reach & (s_cell == g_cell) & (lo <= 0)] = 0
-        search = reach & (ta < 0) & (lo <= H)
+        search = (m if window else reach & (lo <= H)) & (ta < 0)
         F = torch.zeros((B, Rr), dtype=torch.int64, device=dev)
         F[ar[search], sr[search]] = sbit[search]
         Fh[:, 0] = F
@@ -150,11 +212,23 @@ def plan_reference(grid, starts, goals, horizon: int, device=None) -> Plan:
                 w = w & ~hi
             F = torch.where(search[:, None], nf & w, torch.zeros_like(F))
             Fh[:, t] = F
-            hit = search & (t >= lo) & ((F[ar, gr] >> gc) & 1).bool()
+            hit = search & reach & (t >= lo) & ((F[ar, gr] >> gc) & 1).bool()
             ta[hit] = t
             search = search & ~hit & (F != 0).any(1)
-        ok = ta >= 0
         arrival[:, i] = ta.to(torch.int16)
+        if window and bool(search.any()):
+            # still searching at t = W: the path ends on F_W's cell of least (d(target, cell), cell index)
+            e = ar[search]
+            target = torch.where(reach, g_cell, s_cell)[e]
+            inF = ((F[e, :, None] >> torch.arange(Cc, device=dev)) & 1).bool().reshape(len(e), Rr * Cc)
+            key = torch.where(inF, dist[target] * 1024 + cell_ix, 1 << 30)
+            end = key.argmin(1)
+            gr, gc = gr.clone(), gc.clone()
+            gr[e], gc[e] = end // Cc, end % Cc
+            g_cell = gr * Cc + gc
+            ta[e] = H
+        gbit = one << gc
+        ok = ta >= 0
         status &= ok.to(torch.uint8)
         # failed agents on the map hold their start for every t
         bad = m & ~ok
@@ -216,6 +290,44 @@ class PlannedPolicy:
         return torch.zeros((env.B, env.N), dtype=torch.int8, device=env.device)
 
 
+class ReplanningPolicy:
+    """Rolling-horizon replanning as a callable policy for :func:`evaluate.evaluate`, lifelong or episodic: on call k
+    with k % ``replan_every`` == 0 it plans the env's current state with :func:`plan_windowed` at W = ``window``, and
+    it returns action row k % ``replan_every`` of the last plan.  Handed a different env it starts again at k = 0.
+    Only the multi-agent view (:class:`BatchedMapfEnv`) is planned; 1 <= ``replan_every`` <= ``window``."""
+
+    def __init__(self, window: int, replan_every: int = 1):
+        window, replan_every = int(window), int(replan_every)
+        if replan_every < 1 or replan_every > window:
+            raise ValueError(f"replan_every must be in 1..window, got {replan_every} with window {window}")
+        self.window, self.replan_every = window, replan_every
+        self.plan: Plan | None = None
+        self._env = None
+        self._k = 0
+
+    def __call__(self, env, out):
+        if not isinstance(env, BatchedMapfEnv):
+            raise ValueError("ReplanningPolicy plays the multi-agent view (BatchedMapfEnv), not the CTE view")
+        if env is not self._env:
+            self._env, self._k = env, 0
+        j = self._k % self.replan_every
+        if j == 0:
+            self.plan = plan_windowed(env, self.window)
+        self._k += 1
+        return self.plan.actions[j]
+
+
+def _gpu_name(device) -> str:
+    import subprocess
+
+    try:
+        gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader",
+                              "-i", str(torch.device(device).index or 0)], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        gpu = f"nvidia-smi not readable: {exc}"
+    return gpu or torch.cuda.get_device_name(device)
+
+
 def benchmark(num_envs: int = 65536, num_agents: int = 16, horizon: int = 256, rounds: int = 5,
               device: str = "cuda:0") -> dict:
     """Plans/s and agent-plans/s of the kernel for ``num_envs`` Philox layouts of ``num_agents`` agents on the 32x32
@@ -223,8 +335,6 @@ def benchmark(num_envs: int = 65536, num_agents: int = 16, horizon: int = 256, r
     warm-up, CUDA events around the launch (workspace and outputs allocated once, outside the window).  Also the
     success rate, the mean makespan of the status-1 envs and, for the same envs, the mean makespan lower bound from
     ``mapf_goal_path_lengths`` (max over agents of the single-agent distance, at least 1)."""
-    import subprocess
-
     from . import maps
 
     cfg = {"num_agents": num_agents, "sensor_range": 2, "steps_per_episode": horizon, "lifelong_mapf": False,
@@ -245,12 +355,7 @@ def benchmark(num_envs: int = 65536, num_agents: int = 16, horizon: int = 256, r
     lb = env.goal_path_lengths().to(torch.int32).amax(1).clamp(min=1)
     n_ok = int(ok.sum())
     t = min(times)
-    try:
-        gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader",
-                              "-i", str(env.device.index or 0)], capture_output=True, text=True, timeout=30).stdout.strip()
-    except (OSError, subprocess.SubprocessError) as exc:
-        gpu = f"nvidia-smi not readable: {exc}"
-    res = {"gpu": gpu or torch.cuda.get_device_name(env.device), "envs": num_envs, "agents": num_agents,
+    res = {"gpu": _gpu_name(env.device), "envs": num_envs, "agents": num_agents,
            "horizon": horizon, "call_s": t, "rounds_s": times, "plans_per_s": num_envs / t,
            "agent_plans_per_s": num_envs * num_agents / t, "success_rate": n_ok / num_envs,
            "mean_makespan": float(plan.makespan[ok].float().mean()) if n_ok else None,
@@ -260,7 +365,83 @@ def benchmark(num_envs: int = 65536, num_agents: int = 16, horizon: int = 256, r
     return res
 
 
+def benchmark_windowed(num_envs: int = 65536, num_agents: int = 16, windows=(8, 16, 32), rounds: int = 5,
+                       device: str = "cuda:0") -> dict:
+    """The windowed planner and rolling-horizon replanning on the 32x32 benchmark map, ``num_envs`` x ``num_agents``:
+
+    * ``kernel``: per W in ``windows``, the :func:`plan_windowed` call on the mid-episode states of a lifelong env
+      (C3 config, after 64 masked steps): best of ``rounds`` calls after one warm-up, CUDA events around the call, with
+      the share of status-1 envs and of agents that arrived;
+    * ``lifelong``: the evaluator's step loop (:func:`evaluate._play`) at the C3 shape (lifelong, 256 steps) for
+      ``ReplanningPolicy(16, 1)``, ``ReplanningPolicy(16, 4)`` and ``"masked"``: episodes/s (host clock around the loop,
+      which ends in a device synchronise, after a 4-step warm-up), and over the envs the mean throughput, completion
+      ratio and goals reached, and the deadlock / livelock event totals summed over the batch;
+    * ``episodic``: the success rate of ``ReplanningPolicy(32, 1)`` and of :class:`PlannedPolicy` on the layouts of
+      :func:`benchmark` (episodic, 256 steps).
+
+    The GPU's name, power limit and SM clocks are read in the same call."""
+    import time
+
+    from . import maps
+    from .evaluate import _play
+
+    grid = maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32)
+    base = {"num_agents": num_agents, "sensor_range": 2, "steps_per_episode": 256, "enable_lock_metrics": True,
+            "seed": 999, "grid": grid}
+    res = {"envs": num_envs, "agents": num_agents, "kernel": {}, "lifelong": {}, "episodic": {}}
+    env = BatchedMapfEnv(dict(base, lifelong_mapf=True), num_envs, device)
+    env.reset()
+    for _ in range(64):
+        env.step(env.sample_actions(masked=True), auto_reset=False)
+    for W in windows:
+        plan = plan_windowed(env, W)   # warm-up: module load, distance table, allocator
+        times = []
+        for _ in range(rounds):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize(env.device)
+            e0.record()
+            plan = plan_windowed(env, W)
+            e1.record()
+            e1.synchronize()
+            times.append(e0.elapsed_time(e1) / 1e3)
+        t = min(times)
+        res["kernel"][f"W{W}"] = {"call_s": t, "rounds_s": times, "plans_per_s": num_envs / t,
+                                  "agent_plans_per_s": num_envs * num_agents / t,
+                                  "status1_rate": float(plan.status.float().mean()),
+                                  "arrived_rate": float((plan.arrival >= 0).float().mean())}
+    env.close()
+    policies = {"replan_w16_h1": lambda: ReplanningPolicy(16, 1), "replan_w16_h4": lambda: ReplanningPolicy(16, 4),
+                "masked": lambda: "masked"}
+    env = BatchedMapfEnv(dict(base, lifelong_mapf=True), num_envs, device)
+    for name, make in policies.items():
+        _play(env, make(), 4)
+        torch.cuda.synchronize(env.device)
+        t0 = time.perf_counter()
+        acc = _play(env, make())
+        dt = time.perf_counter() - t0
+        info = acc["last_info"].cpu().numpy().astype(np.float64)
+        g_tot = info[:, nat.I_GOALS_REACHED_TOTAL]
+        res["lifelong"][name] = {
+            "loop_s": dt, "episodes_per_s": num_envs / dt,
+            "throughput": float((g_tot / np.maximum(info[:, nat.I_STEP_COUNT], 1)).mean()),
+            "completion_ratio": float((info[:, nat.I_COMPLETED_COUNT] / num_agents).mean()),
+            "goals_reached_total": float(g_tot.mean()),
+            "deadlock_events_total": float(info[:, nat.I_DEADLOCK_EVENTS_TOTAL].sum()),
+            "livelock_events_total": float(info[:, nat.I_LIVELOCK_EVENTS_TOTAL].sum())}
+    env.close()
+    for name, pol in (("replan_w32_h1", ReplanningPolicy(32, 1)), ("planned", PlannedPolicy())):
+        env = BatchedMapfEnv(dict(base, lifelong_mapf=False), num_envs, device)   # a fresh env: the first reset's layouts
+        acc = _play(env, pol)
+        ok = acc["success"].bool()
+        res["episodic"][name] = {"success_rate": float(ok.float().mean()),
+                                 "mean_timesteps_of_successes": float(acc["timesteps"][ok].float().mean()) if bool(ok.any()) else None}
+        env.close()
+    res["gpu"] = _gpu_name(device)
+    return res
+
+
 if __name__ == "__main__":
     import json
+    import sys
 
-    print(json.dumps(benchmark()))
+    print(json.dumps(benchmark_windowed() if "--windowed" in sys.argv[1:] else benchmark()))

@@ -829,6 +829,22 @@ typedef struct mapf_plan_args {
 int64_t mapf_plan_workspace_bytes(int32_t rows, int32_t cols, int32_t num_envs, int32_t horizon);
 int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *args, void *stream);
 
+/* Windowed prioritized planner for rolling-horizon replanning (RHCR, Li et al. 2021) from any state, lifelong envs
+ * included: the rule of mapf_plan_prioritized with the horizon read as the window W (args->horizon; actions [W,B,N]),
+ * resolving conflicts only within W and not requiring arrival.  The target is the goal if distance_table reaches it
+ * from the start (!= 255), else the start.  An agent with the goal as target arrives at the first t <= W with the
+ * goal in its wavefront and t >= max(d, last hold of the goal + 1), and holds it to W (arrival = t).  Otherwise the
+ * search runs to t = W and the path ends on the cell of the wavefront at W with the smallest distance-table value
+ * from the target, ties to the first cell in row-major order; the agent reserves that path and gets arrival -1.  An
+ * agent whose wavefront empties before W, or whose start or goal lies off the map, fails as in mapf_plan_prioritized
+ * (NO_OPs, start reserved for every t); the later agents are still planned.  status[b] = 1 iff every agent of env b
+ * got a path; then replaying the W actions through mapf_step from the planned state gives no failed move and every
+ * agent follows its planned cells (also in lifelong mode: goal reassignment never moves an agent), and an agent that
+ * arrived stands on its goal from its arrival on.  On envs where mapf_plan_prioritized at H gives status 1, the
+ * windowed plan at W = H has the same actions and arrivals.  Refusals are those of mapf_plan_prioritized, before any
+ * device work; mapf_plan_workspace_bytes(rows, cols, B, W) sizes the workspace.  DESIGN.md §7 N4c. */
+int mapf_plan_windowed(mapf_handle *h, const mapf_plan_args *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
