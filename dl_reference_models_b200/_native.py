@@ -20,7 +20,7 @@ SOURCES = (CSRC / "mapf_b200.cu", CSRC / "mapf_kernels.cuh", CSRC / "mapf_env_ke
            CSRC / "mapf_policy_lstm_kernel.cuh", CSRC / "mapf_eval_kernel.cuh", CSRC / "mapf_cte_policy_kernel.cuh",
            CSRC / "mapf_cte_lstm_policy_kernel.cuh", CSRC / "mapf_cte_trunk.inc",
            CSRC / "mapf_cte_heads.inc", CSRC / "mapf_vtrace_kernel.cuh", CSRC / "mapf_q_kernel.cuh",
-           CSRC / "mapf_replay_kernel.cuh", CSRC / "mapf_plan_kernel.cuh", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
+           CSRC / "mapf_replay_kernel.cuh", CSRC / "mapf_plan_kernel.cuh", CSRC / "mapf_cbs_kernel.cuh", CSRC / "mapf_pack_kernel.cuh", CSRC / "mapf_host_unpack.h", CSRC / "mapf_host_unpack.cpp",
            REPO / "include" / "mapf_b200.h")
 
 MAX_AGENTS = 32
@@ -212,6 +212,15 @@ class MapfPlanArgs(C.Structure):
                 ("workspace_bytes", C.c_int64), ("actions", C.c_void_p), ("arrival", C.c_void_p), ("status", C.c_void_p)]
 
 
+class MapfCbsArgs(C.Structure):
+    """mapf_cbs_args of include/mapf_b200.h (conflict-based search)."""
+
+    _fields_ = [("num_envs", C.c_int32), ("num_agents", C.c_int32), ("horizon", C.c_int32), ("max_nodes", C.c_int32),
+                ("starts", C.c_void_p), ("goals", C.c_void_p), ("distance_table", C.c_void_p), ("workspace", C.c_void_p),
+                ("workspace_bytes", C.c_int64), ("actions", C.c_void_p), ("arrival", C.c_void_p), ("status", C.c_void_p),
+                ("expanded", C.c_void_p), ("reserved", C.c_int32)]
+
+
 class MapfError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"libmapf_b200 error {code}: {message}")
@@ -336,13 +345,16 @@ def lib():
     L.mapf_plan_workspace_bytes.restype = i64
     L.mapf_plan_prioritized.argtypes = [vp, C.POINTER(MapfPlanArgs), vp]
     L.mapf_plan_windowed.argtypes = [vp, C.POINTER(MapfPlanArgs), vp]
+    L.mapf_cbs_workspace_bytes.argtypes = [i32] * 6
+    L.mapf_cbs_workspace_bytes.restype = i64
+    L.mapf_plan_cbs.argtypes = [vp, C.POINTER(MapfCbsArgs), vp]
     L.mapf_cte_step.argtypes = [C.POINTER(MapfCteArgs), vp]
     L.mapf_cte_reset.argtypes = [C.POINTER(MapfCteArgs), vp]
     for name in EXPORTS:
         if name not in ("mapf_version", "mapf_last_error", "mapf_launch_count", "mapf_policy_weights_nbytes",
                         "mapf_lstm_policy_weights_nbytes", "mapf_cte_policy_weights_nbytes",
                         "mapf_cte_lstm_policy_weights_nbytes", "mapf_replay_tree_leaves",
-                        "mapf_plan_workspace_bytes"):
+                        "mapf_plan_workspace_bytes", "mapf_cbs_workspace_bytes"):
             getattr(L, name).restype = C.c_int
     _lib = L
     return L
@@ -365,6 +377,7 @@ EXPORTS = (
     "mapf_cte_eval_accumulate", "mapf_vtrace",
     "mapf_q_act", "mapf_q_act_per_agent", "mapf_replay_tree_leaves", "mapf_replay_advance", "mapf_replay_sample",
     "mapf_replay_update", "mapf_plan_workspace_bytes", "mapf_plan_prioritized", "mapf_plan_windowed",
+    "mapf_cbs_workspace_bytes", "mapf_plan_cbs",
 )
 
 

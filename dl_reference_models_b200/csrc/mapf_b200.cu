@@ -14,6 +14,7 @@
 #include "mapf_q_kernel.cuh"
 #include "mapf_replay_kernel.cuh"
 #include "mapf_plan_kernel.cuh"
+#include "mapf_cbs_kernel.cuh"
 #include "mapf_pack_kernel.cuh"
 #include "mapf_host_unpack.h"
 
@@ -2166,6 +2167,59 @@ static int plan_launch(mapf_handle *h, const mapf_plan_args *a, void *stream, bo
 int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *a, void *stream) { return plan_launch(h, a, stream, false); }
 
 int mapf_plan_windowed(mapf_handle *h, const mapf_plan_args *a, void *stream) { return plan_launch(h, a, stream, true); }
+
+int64_t mapf_cbs_workspace_bytes(int32_t rows, int32_t cols, int32_t num_envs, int32_t num_agents, int32_t horizon,
+                                 int32_t max_nodes) {
+    if (rows < 1 || cols < 1 || num_envs < 1 || num_agents < 1 || horizon < 1 || max_nodes < 1)
+        return fail(MAPF_ERR_INVALID_ARG, "cbs: rows %d, cols %d, num_envs %d, num_agents %d, horizon %d and max_nodes %d "
+                    "must be positive", rows, cols, num_envs, num_agents, horizon, max_nodes);
+    if (max_nodes > 65536 || horizon > 32767)
+        return fail(MAPF_ERR_INVALID_ARG, "cbs: max_nodes %d (at most 65536) or horizon %d (at most 32767) too large",
+                    max_nodes, horizon);
+    if (rows > 32 || cols > 32) return fail(MAPF_ERR_UNSUPPORTED, "cbs: maps are at most 32x32 (got %dx%d)", rows, cols);
+    if (num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "cbs: num_agents %d exceeds %d", num_agents, MAPF_MAX_AGENTS);
+    return 16 + (int64_t)num_envs * mapf::cbs_env_bytes(rows, num_agents, horizon, max_nodes);
+}
+
+int mapf_plan_cbs(mapf_handle *h, const mapf_cbs_args *a, void *stream) {
+    if (!h || !a) return fail(MAPF_ERR_INVALID_ARG, "cbs: null argument");
+    if (a->num_envs < 1 || a->num_agents < 1 || a->horizon < 1 || a->reserved != 0 || !a->starts || !a->goals ||
+        !a->distance_table || !a->workspace || !a->actions || !a->arrival || !a->status || !a->expanded)
+        return fail(MAPF_ERR_INVALID_ARG, "cbs: null or empty argument");
+    if (a->max_nodes < 1 || a->max_nodes > 65536 || a->horizon > 32767)
+        return fail(MAPF_ERR_INVALID_ARG, "cbs: max_nodes %d must be in 1..65536 and horizon %d at most 32767",
+                    a->max_nodes, a->horizon);
+    if (a->num_agents > MAPF_MAX_AGENTS)
+        return fail(MAPF_ERR_UNSUPPORTED, "cbs: num_agents %d exceeds %d", a->num_agents, MAPF_MAX_AGENTS);
+    if (!h->map_set) return fail(MAPF_ERR_STATE, "mapf_set_map has not been called");
+    if (h->cfg.per_env_maps || h->cfg.rows > 32 || h->cfg.cols > 32)
+        return fail(MAPF_ERR_UNSUPPORTED, "cbs: needs one shared map of at most 32x32 cells (got %dx%d, per_env_maps=%d)",
+                    h->cfg.rows, h->cfg.cols, h->cfg.per_env_maps);
+    const int64_t need = mapf_cbs_workspace_bytes(h->cfg.rows, h->cfg.cols, a->num_envs, a->num_agents, a->horizon,
+                                                  a->max_nodes);
+    if (need < 0) return (int)need;
+    if (a->workspace_bytes < need)
+        return fail(MAPF_ERR_INVALID_ARG, "cbs: workspace of %lld bytes, %lld needed", (long long)a->workspace_bytes,
+                    (long long)need);
+    DeviceGuard guard(h->cfg.device);
+    int sms = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    CUDA_TRY(cudaMemsetAsync(a->workspace, 0, 16, s));   // the env counter
+    const int warps = mapf::CBS_THREADS / 32;
+    long long blocks = ((long long)a->num_envs + warps - 1) / warps;
+    if (blocks > (long long)sms * 16) blocks = (long long)sms * 16;   // 64 resident warps per SM; they take envs in turn
+    mapf::mapf_cbs_kernel<<<(unsigned)blocks, mapf::CBS_THREADS, 0, s>>>(
+        h->d_free_bits, h->cfg.rows, h->cfg.cols, a->num_envs, a->num_agents, a->horizon, a->max_nodes,
+        reinterpret_cast<const uint32_t *>(a->starts), reinterpret_cast<const uint32_t *>(a->goals), a->distance_table,
+        static_cast<unsigned char *>(a->workspace),
+        mapf::cbs_env_bytes(h->cfg.rows, a->num_agents, a->horizon, a->max_nodes), a->actions, a->arrival, a->status,
+        a->expanded);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+    return MAPF_OK;
+}
 
 int64_t mapf_launch_count(const mapf_handle *h) { return h ? h->launches : 0; }
 

@@ -44,6 +44,17 @@ above for envs where every agent arrived, -1 otherwise.  On an env where :func:`
 the windowed plan at W = H has the same actions and arrivals.  :class:`ReplanningPolicy` replans every h steps and
 plays the first h actions of each plan through :func:`evaluate.evaluate`; ``python -m dl_reference_models_b200.planner
 --windowed`` measures it (:func:`benchmark_windowed`).
+
+**Conflict-based search** (CBS, Sharon et al. 2015; DESIGN.md §7 N4d): :func:`plan_cbs` finds, per env, a plan with the
+least sum of arrivals within H that replays under the env's move rule, for small agent counts (2-8), with an
+``outcome`` that says why there is none (0: no plan within H, 2: the ``max_nodes`` expansion budget ran out).  Two
+conflicts exist under this rule: a vertex conflict (two agents on one cell at t + 1) and a following conflict (agent a
+moves at t into the cell a higher index b holds at t); they split into the constraints (a, c, t+1) / (b, c, t+1) and
+(a, c, t+1) / (b, c, t).  The low level is the wavefront above with the agent's constraints as the obstacles; the high
+level pops the least (sum of arrivals, creation id), takes the first conflict (smallest t, vertex before following,
+lowest a, then lowest b) and creates the child constraining a, then b.  :func:`cbs_reference` is the pure Python
+reference and CPU path; ``PlannedPolicy("cbs")`` plays the plans through :func:`evaluate.evaluate`; ``python -m
+dl_reference_models_b200.planner --cbs`` measures it (:func:`benchmark_cbs`).
 """
 from __future__ import annotations
 
@@ -66,12 +77,23 @@ class Plan:
     sum_of_costs: torch.Tensor   # int32 [B]: sum of the arrivals; -1 for status 0 (windowed: or an agent not arrived)
 
 
+@dataclass
+class CbsPlan(Plan):
+    outcome: torch.Tensor        # uint8 [B]: 1 = optimal plan found, 0 = no plan within H, 2 = max_nodes expansions hit
+    expanded: torch.Tensor       # int32 [B]: high-level nodes popped
+
+
 def _finish(actions, arrival, status) -> Plan:
     ok = status.bool() & (arrival >= 0).all(1)
     a = arrival.to(torch.int32)
     makespan = torch.where(ok, a.amax(1).clamp(min=1), torch.full_like(a[:, 0], -1))
     soc = torch.where(ok, a.sum(1), torch.full_like(a[:, 0], -1))
     return Plan(actions, arrival, status, makespan, soc)
+
+
+def _finish_cbs(actions, arrival, outcome, expanded) -> CbsPlan:
+    p = _finish(actions, arrival, (outcome == 1).to(torch.uint8))
+    return CbsPlan(**vars(p), outcome=outcome, expanded=expanded)
 
 
 def plan_prioritized(env: BatchedMapfEnv, starts=None, goals=None, horizon: int | None = None) -> Plan:
@@ -95,11 +117,50 @@ def plan_windowed(env: BatchedMapfEnv, window: int, starts=None, goals=None) -> 
     return _plan_native(env, starts, goals, int(window), "mapf_plan_windowed")
 
 
-def _plan_native(env: BatchedMapfEnv, starts, goals, H: int, entry: str) -> Plan:
+def plan_cbs(env: BatchedMapfEnv, max_nodes: int = 1024, starts=None, goals=None,
+             horizon: int | None = None) -> CbsPlan:
+    """Conflict-based search of every env of ``env`` on the device (``mapf_plan_cbs``; DESIGN.md §7 N4d): plans with
+    the least sum of arrivals within H under the env's own move rule, or the reason there is none.  ``outcome`` 1 =
+    optimal plan (``status`` 1; it replays like a status-1 :func:`plan_prioritized` plan), 0 = no plan exists within
+    H (an unreachable goal, a start or goal off the map, on an obstacle or repeated, or every split exhausted), 2 =
+    ``max_nodes`` high-level expansions without an answer.  Envs with outcome 0 or 2 get NO_OPs and arrival -1.
+    ``starts`` / ``goals`` / ``horizon`` as in :func:`plan_prioritized`; lifelong envs are refused.  CBS is for small
+    agent counts (2-8): its search grows with the number of conflicts, so :func:`plan_prioritized` stays the
+    large-N baseline."""
+    if not isinstance(env, BatchedMapfEnv):
+        raise TypeError(f"plan_cbs plans a BatchedMapfEnv; use cbs_reference on the CPU (got {type(env).__name__})")
+    if env.lifelong:
+        raise ValueError("a lifelong env assigns new goals during the episode: a plan to the first goals is not a plan")
+    H = int(env.cfg.steps_per_episode if horizon is None else horizon)
+    s, g = _layouts(env, starts, goals)
+    B, N = int(s.shape[0]), int(s.shape[1])
+    L = nat.lib()
+    R, Cc = (int(x) for x in env.grid.shape[-2:])
+    nbytes = nat.check(L.mapf_cbs_workspace_bytes(R, Cc, B, N, max(H, 1), int(max_nodes))) if B > 0 and N > 0 else 0
+    dev = env.device
+    ws = torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=dev)
+    actions = torch.empty((H, B, N), dtype=torch.int8, device=dev)
+    arrival = torch.empty((B, N), dtype=torch.int16, device=dev)
+    outcome = torch.empty(B, dtype=torch.uint8, device=dev)
+    expanded = torch.empty(B, dtype=torch.int32, device=dev)
+    p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
+    args = nat.MapfCbsArgs(num_envs=B, num_agents=N, horizon=H, max_nodes=int(max_nodes), starts=p(s), goals=p(g),
+                           distance_table=p(env.distance_table()), workspace=p(ws), workspace_bytes=ws.numel(),
+                           actions=p(actions), arrival=p(arrival), status=p(outcome), expanded=p(expanded))
+    nat.check(L.mapf_plan_cbs(env._h, C.byref(args), env._stream()))
+    return _finish_cbs(actions, arrival, outcome, expanded)
+
+
+def _layouts(env: BatchedMapfEnv, starts, goals):
     s = (env.state["positions"] if starts is None else torch.as_tensor(starts)).to(env.device, torch.int16).contiguous()
     g = (env.state["goals"] if goals is None else torch.as_tensor(goals)).to(env.device, torch.int16).contiguous()
     if s.ndim != 3 or s.shape[2] != 2 or s.shape != g.shape:
         raise ValueError(f"starts and goals must both be [B,N,2], got {tuple(s.shape)} and {tuple(g.shape)}")
+    return s, g
+
+
+def _plan_native(env: BatchedMapfEnv, starts, goals, H: int, entry: str) -> Plan:
+    s, g = _layouts(env, starts, goals)
     B, N = int(s.shape[0]), int(s.shape[1])
     L = nat.lib()
     R, Cc = (int(x) for x in env.grid.shape[-2:])
@@ -268,13 +329,138 @@ def plan_reference(grid, starts, goals, horizon: int, device=None, window: bool 
     return _finish(actions, arrival, status)
 
 
+_MOVES = ((0, 0), (-1, 0), (0, 1), (1, 0), (0, -1))     # (dr, dc) of NO_OP, UP, RIGHT, DOWN, LEFT
+
+
+def _cbs_low_level(free, W, R, Cc, s, g, cons, H):
+    """One agent's earliest arrival under its constraints ``cons`` ({t: forbidden cell bits}; cell (r, c) is bit
+    r * W + c, W = C + 1 so that shifts never wrap into the next row): the path as the cells at t = 0..arrival, or
+    None."""
+    gb = 1 << (g[0] * W + g[1])
+    L = 1 + max((t for t, m in cons.items() if m & gb), default=-1)
+    f = 1 << (s[0] * W + s[1])
+    if cons.get(0, 0) & f:
+        return None
+    F = [f]
+    ta = 0 if s == g and L == 0 else -1
+    if ta < 0:
+        for t in range(1, H + 1):
+            f = (f | (f << 1) | (f >> 1) | (f << W) | (f >> W)) & free & ~cons.get(t, 0)
+            F.append(f)
+            if t >= L and f & gb:
+                ta = t
+                break
+            if not f:
+                break
+    if ta < 0:
+        return None
+    path = [g]
+    r, c = g
+    for t in range(ta, 0, -1):
+        prev = F[t - 1]
+        for dr, dc in _MOVES:                          # the first predecessor in action order
+            pr, pc = r - dr, c - dc
+            if 0 <= pr < R and 0 <= pc < Cc and prev >> (pr * W + pc) & 1:
+                break
+        r, c = pr, pc
+        path.append((r, c))
+    return path[::-1]
+
+
+def _cbs_first_conflict(paths):
+    """The first conflict of a joint plan in scan order, as its two vertex constraints (a, cell, t), (b, cell, t')."""
+    N = len(paths)
+    at = lambda p, t: p[t] if t < len(p) else p[-1]  # noqa: E731
+    for t in range(max(len(p) for p in paths) - 1):
+        cur = [at(p, t) for p in paths]
+        nxt = [at(p, t + 1) for p in paths]
+        for a in range(N):                             # vertex: lowest a, then lowest b
+            for b in range(a + 1, N):
+                if nxt[a] == nxt[b]:
+                    return (a, nxt[a], t + 1), (b, nxt[a], t + 1)
+        owner = {c: i for i, c in enumerate(cur)}
+        for a in range(N):                             # following: a moves into the cell a higher index holds at t
+            b = owner.get(nxt[a], -1)
+            if nxt[a] != cur[a] and b > a:
+                return (a, nxt[a], t + 1), (b, nxt[a], t)
+    return None
+
+
+def _cbs_one(grid, starts, goals, H, max_nodes):
+    """CBS of one env: (paths or None, outcome, expanded)."""
+    import heapq
+
+    R, Cc = grid.shape
+    W = Cc + 1
+    free = sum(1 << (int(r) * W + int(c)) for r, c in np.argwhere(grid == 0))
+    st = [(int(r), int(c)) for r, c in starts]
+    gl = [(int(r), int(c)) for r, c in goals]
+    inside = lambda p: 0 <= p[0] < R and 0 <= p[1] < Cc and grid[p] == 0  # noqa: E731
+    if not all(inside(p) for p in st + gl) or len(set(st)) < len(st) or len(set(gl)) < len(gl):
+        return None, 0, 0
+    paths = [_cbs_low_level(free, W, R, Cc, s, g, {}, H) for s, g in zip(st, gl)]
+    if any(p is None for p in paths):
+        return None, 0, 0
+    # a node: (SOC, id, per-agent constraint dicts, paths); a child shares its parent's lists but the replanned entry
+    heap = [(sum(len(p) - 1 for p in paths), 0, [{} for _ in st], paths)]
+    expanded, next_id = 0, 1
+    while heap and expanded < max_nodes:
+        soc, _, cons, paths = heapq.heappop(heap)
+        expanded += 1
+        conflict = _cbs_first_conflict(paths)
+        if conflict is None:
+            return paths, 1, expanded
+        for agent, cell, t in conflict:
+            c = dict(cons[agent])
+            c[t] = c.get(t, 0) | 1 << (cell[0] * W + cell[1])
+            p = _cbs_low_level(free, W, R, Cc, st[agent], gl[agent], c, H)
+            if p is None:
+                continue
+            ncons, npaths = list(cons), list(paths)
+            ncons[agent], npaths[agent] = c, p
+            heapq.heappush(heap, (soc - (len(paths[agent]) - 1) + len(p) - 1, next_id, ncons, npaths))
+            next_id += 1
+    return None, (2 if heap else 0), expanded
+
+
+def cbs_reference(grid, starts, goals, horizon: int, max_nodes: int = 1024) -> CbsPlan:
+    """Conflict-based search in pure Python, env by env with integer bitboards (the CPU path, and what the
+    ``mapf_plan_cbs`` kernel is tested against bit for bit: the same actions, arrivals, outcomes and expansion
+    counts).  ``starts`` / ``goals``: [B,N,2] (row, col).  See DESIGN.md §7 N4d for the search it runs."""
+    grid = np.ascontiguousarray(np.asarray(grid), dtype=np.uint8)
+    if grid.ndim != 2 or grid.shape[0] > 32 or grid.shape[1] > 32:
+        raise ValueError(f"the planner needs one map of at most 32x32 cells, got shape {grid.shape}")
+    H, K = int(horizon), int(max_nodes)
+    if H < 1 or not 1 <= K <= 65536:
+        raise ValueError(f"horizon must be >= 1 and max_nodes in 1..65536, got {H} and {K}")
+    st = np.asarray(torch.as_tensor(starts).cpu(), dtype=np.int64)
+    gl = np.asarray(torch.as_tensor(goals).cpu(), dtype=np.int64)
+    B, N = st.shape[:2]
+    actions = np.zeros((H, B, N), np.int8)
+    arrival = np.full((B, N), -1, np.int16)
+    outcome = np.zeros(B, np.uint8)
+    expanded = np.zeros(B, np.int32)
+    for b in range(B):
+        paths, outcome[b], expanded[b] = _cbs_one(grid, st[b], gl[b], H, K)
+        for i, p in enumerate(paths or ()):
+            arrival[b, i] = len(p) - 1
+            for t in range(len(p) - 1):
+                actions[t, b, i] = _MOVES.index((p[t + 1][0] - p[t][0], p[t + 1][1] - p[t][1]))
+    return _finish_cbs(torch.from_numpy(actions), torch.from_numpy(arrival), torch.from_numpy(outcome),
+                       torch.from_numpy(expanded))
+
+
 class PlannedPolicy:
     """A callable policy for :func:`evaluate.evaluate`: on its first call with an env (right after the evaluator's
-    reset) it plans every env's layout once with :func:`plan_prioritized`, then returns action row t at the t-th call
-    (NO_OP past the horizon).  The planner so gets the evaluator's CSV rows, heat-map and success rate on the very
-    layouts a trained policy sees with the same ``env_config``.  Handed a different env it plans again."""
+    reset) it plans every env's layout once with :func:`plan_prioritized` (``method="prioritized"``, the default) or
+    :func:`plan_cbs` with ``max_nodes`` (``method="cbs"``), then returns action row t at the t-th call (NO_OP past the
+    horizon).  The planner so gets the evaluator's CSV rows, heat-map and success rate on the very layouts a trained
+    policy sees with the same ``env_config``.  Handed a different env it plans again."""
 
-    def __init__(self):
+    def __init__(self, method: str = "prioritized", max_nodes: int = 1024):
+        if method not in ("prioritized", "cbs"):
+            raise ValueError(f"method must be 'prioritized' or 'cbs', got {method!r}")
+        self.method, self.max_nodes = method, int(max_nodes)
         self.plan: Plan | None = None
         self._env = None
         self._t = 0
@@ -283,7 +469,8 @@ class PlannedPolicy:
         if not isinstance(env, BatchedMapfEnv):
             raise ValueError("PlannedPolicy plays the multi-agent view (BatchedMapfEnv), not the CTE view")
         if env is not self._env:
-            self.plan, self._env, self._t = plan_prioritized(env), env, 0
+            plan = plan_cbs(env, self.max_nodes) if self.method == "cbs" else plan_prioritized(env)
+            self.plan, self._env, self._t = plan, env, 0
         t, self._t = self._t, self._t + 1
         if t < self.plan.actions.shape[0]:
             return self.plan.actions[t]
@@ -440,8 +627,61 @@ def benchmark_windowed(num_envs: int = 65536, num_agents: int = 16, windows=(8, 
     return res
 
 
+def benchmark_cbs(num_envs: int = 65536, rounds: int = 5, device: str = "cuda:0") -> dict:
+    """:func:`plan_cbs` per shape: ``num_envs`` Philox layouts x 4 agents on maps 2-2 and 3-1 at H = 100 and x 8 agents on
+    the 32x32 benchmark map at H = 256, at K = 1024 and (32x32) K = 256, and the seven deterministic tables as single
+    envs at H = 254.  Per shape: best of ``rounds`` calls after one warm-up, CUDA events around the call (workspace
+    included), plans/s, the outcome split, expansions p50 / p99 / max, and the mean sum of arrivals of CBS and of
+    :func:`plan_prioritized` over the envs both solve.  The GPU's name, power limit and SM clocks are read in the same
+    call."""
+    from . import maps
+
+    rand32 = maps.random_obstacle_grid(32, 32, 0.30, 2026, min_free=32)
+    shapes = [("2-2", maps.get_grid("ReferenceModel-2-2"), 4, 100, 1024, num_envs),
+              ("3-1", maps.get_grid("ReferenceModel-3-1"), 4, 100, 1024, num_envs),
+              ("rand32", rand32, 8, 256, 1024, num_envs), ("rand32", rand32, 8, 256, 256, num_envs)]
+    shapes += [(f"{m}-det", maps.get_grid(f"ReferenceModel-{m}"), 2 if m.startswith("1") else 4, 254, 1024, 1)
+               for m in ("1-1", "1-2", "1-3", "1-4", "2-1", "2-2", "3-1")]
+    res = {"shapes": []}
+    for name, grid, N, H, K, B in shapes:
+        cfg = {"num_agents": N, "sensor_range": 2, "steps_per_episode": H, "lifelong_mapf": False, "seed": 999,
+               "grid": grid, "deterministic": name.endswith("-det"), "env_name": f"ReferenceModel-{name[:-4]}"}
+        env = BatchedMapfEnv(cfg, B, device)
+        env.reset()
+        plan = plan_cbs(env, K)   # warm-up: module load, distance table, allocator
+        times = []
+        for _ in range(rounds):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize(env.device)
+            e0.record()
+            plan = plan_cbs(env, K)
+            e1.record()
+            e1.synchronize()
+            times.append(e0.elapsed_time(e1) / 1e3)
+        pr = plan_prioritized(env)
+        both = (plan.status.bool() & pr.status.bool()).cpu()
+        ex = plan.expanded.cpu().numpy()
+        oc = plan.outcome.cpu().numpy()
+        t = min(times)
+        row = {"map": name, "envs": B, "agents": N, "horizon": H, "max_nodes": K, "call_s": t, "rounds_s": times,
+               "plans_per_s": B / t, "outcome": {str(k): int((oc == k).sum()) for k in (0, 1, 2)},
+               "expanded_p50_p99_max": [float(np.percentile(ex, 50)), float(np.percentile(ex, 99)), int(ex.max())],
+               "prioritized_status1": int(pr.status.sum()), "both_solved": int(both.sum()),
+               "mean_soc_cbs": float(plan.sum_of_costs.cpu()[both].float().mean()) if bool(both.any()) else None,
+               "mean_soc_prioritized": float(pr.sum_of_costs.cpu()[both].float().mean()) if bool(both.any()) else None}
+        if B == 1:
+            row["arrival"] = plan.arrival[0].tolist()
+            row["prioritized_arrival"] = pr.arrival[0].tolist()
+        res["shapes"].append(row)
+        env.close()
+    res["gpu"] = _gpu_name(device)
+    return res
+
+
 if __name__ == "__main__":
     import json
     import sys
 
-    print(json.dumps(benchmark_windowed() if "--windowed" in sys.argv[1:] else benchmark()))
+    flags = sys.argv[1:]
+    print(json.dumps(benchmark_windowed() if "--windowed" in flags else benchmark_cbs() if "--cbs" in flags
+                     else benchmark()))

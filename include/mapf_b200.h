@@ -845,6 +845,53 @@ int mapf_plan_prioritized(mapf_handle *h, const mapf_plan_args *args, void *stre
  * device work; mapf_plan_workspace_bytes(rows, cols, B, W) sizes the workspace.  DESIGN.md §7 N4c. */
 int mapf_plan_windowed(mapf_handle *h, const mapf_plan_args *args, void *stream);
 
+/* Conflict-based search (CBS) on the handle's shared map under mapf_step's move rule: per env, a plan with the least
+ * sum of arrivals within the horizon, or the reason there is none.  A joint plan (every agent on its goal from its
+ * arrival on) replays without a failed move iff no two agents share a cell at t + 1 (vertex) and no agent a moves at t
+ * into the cell a higher index b holds at t (following); each conflict splits into two vertex constraints, (a, c, t+1)
+ * / (b, c, t+1) and (a, c, t+1) / (b, c, t).  The low level is the wavefront of mapf_plan_prioritized with the agent's
+ * constraints as the only obstacles besides the map: earliest arrival t <= H with t > every constrained t of the goal,
+ * the same backtrack tie rule.  The high level pops the open node of least (sum of arrivals, creation id), takes its
+ * first conflict (smallest t; vertex before following; lowest a, then lowest b) and creates the child constraining a,
+ * then the one constraining b, replanning only that agent; a child without a path is not created.  Deterministic: the
+ * same layouts give the same plan and expansion count.  DESIGN.md §7 N4d.
+ *
+ * status[b] (the outcome): 1 = the popped node has no conflict: an optimal plan, whose actions replay through mapf_step
+ * without a failed move and end the episode (terminated) at step max(1, max arrival) with every agent on its goal;
+ * 0 = no plan exists within the horizon (an agent with no path, a start or goal off the map, on an obstacle or repeated
+ * -- these without a search, expanded = 0 -- or the open list exhausted); 2 = max_nodes expansions without an answer.
+ * Outcomes 0 and 2 give NO_OP actions and arrival -1.  expanded[b] = the nodes popped.
+ *
+ * Refused before any device work: those of mapf_plan_prioritized (with mapf_cbs_workspace_bytes for the size), and
+ * max_nodes outside 1..65536 or horizon > 32767 (MAPF_ERR_INVALID_ARG).  The launch first zeroes the workspace's env
+ * counter with cudaMemsetAsync on `stream`; envs are taken from it by one warp each.  CBS is for small agent counts
+ * (2-8): its search grows with the number of conflicts; mapf_plan_prioritized stays the large-N baseline. */
+typedef struct mapf_cbs_args {
+    int32_t num_envs, num_agents;   /* B, N */
+    int32_t horizon;                /* H */
+    int32_t max_nodes;              /* K: the expansion budget, 1..65536 */
+    const int16_t *starts;          /* [B,N,2] (row, col) device */
+    const int16_t *goals;           /* [B,N,2] */
+    const uint8_t *distance_table;  /* [R*C, R*C] written by mapf_distance_table for this handle */
+    void *workspace;                /* device scratch of workspace_bytes, contents need not be initialised */
+    int64_t workspace_bytes;
+    int8_t *actions;                /* [H,B,N] out */
+    int16_t *arrival;               /* [B,N] out: arrival step for outcome 1, else -1 */
+    uint8_t *status;                /* [B] out: the outcome 0 / 1 / 2 */
+    int32_t *expanded;              /* [B] out: high-level nodes popped */
+    int32_t reserved;               /* must be 0 */
+} mapf_cbs_args;
+
+/* Workspace bytes of mapf_plan_cbs, or a MAPF_ERR_* code (MAPF_ERR_INVALID_ARG for non-positive arguments, max_nodes
+ * over 65536 or horizon over 32767, MAPF_ERR_UNSUPPORTED for maps over 32x32 or num_agents over MAPF_MAX_AGENTS):
+ *   16 + num_envs * ceil16(24 (2K + 1) + 64 + 8 (H + 1) rows + (N + 2K) ceil16(H))
+ * (a 16-byte env counter; per env the node records and open-list keys, the root's arrivals, the constraint and
+ * wavefront planes, and one int8 action path per root agent and per child).  65 536 envs at N = 8, H = 256, K = 1024
+ * take 42 GB; the path slots dominate, so size K to the search the layouts need. */
+int64_t mapf_cbs_workspace_bytes(int32_t rows, int32_t cols, int32_t num_envs, int32_t num_agents, int32_t horizon,
+                                 int32_t max_nodes);
+int mapf_plan_cbs(mapf_handle *h, const mapf_cbs_args *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
